@@ -4,6 +4,9 @@ with the other BASELINE configs beside them in the same JSON line.
 
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA, one process per GPU; torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...  the reference's CPU path (oracle port; rank 0 only)
+  python bench.py ... --dump-outputs DIR                   also write the headline's last timed step (obs, reward, done) as
+                                                           DIR/<name>.npy in float32 (DIR/<name>_rank<r>.npy for N > 1), so
+                                                           that two builds can be compared output for output on identical inputs
 
 Headline workload (config.workload): 4096 lockstep walkers per GPU, Wood floor (Carpet walker), i.i.d. U(-1,1) actions per joint
 per env-step (seeded, generated once), dt = 0x1.111134p-6, Iterations = 50, auto-reset on terminal.  One "step" = one fused
@@ -15,7 +18,9 @@ after construction all walkers are identical, which flatters a SIMT kernel: no d
 (the reference's body list changes order exactly once, at the first Walker.Reset -- Walker.cs:212-223).
 
 Timing: every timed step is bracketed by CUDA events on the launching stream; between timed steps an L2 flush (256 MiB memset)
-runs OUTSIDE the event pairs; ms_per_step = sum of the K event intervals / K, max over ranks.
+runs OUTSIDE the event pairs; ms_per_step = sum of the K event intervals / K, max over ranks.  --steps K is the number of timed
+steps of every leg that reports "steps" (headline, e2e, at_scale, contact_stress, secondary); ppo_loop and cfg1 time the fixed
+samples they describe.
 "e2e" = the same step through the public host-buffer call (EnvBatch.step -> wb_env_step) with pinned host actions in and host
 obs/reward/done out every step, wall clock around the call.
 
@@ -337,6 +342,8 @@ def bench_headline(cx, K, W):
 
     total_ms = cx.timed_steps(one, K)
     ndone = int(done_d.sum().item())
+    # what a caller of step_dev receives from the last timed step (the buffers are reused by the e2e leg below)
+    outputs = {"obs": obs_d.cpu().numpy(), "reward": rew_d.cpu().numpy(), "done": done_d.cpu().numpy().astype(np.float32)}
     cx.barrier()
     launches = env.launch_count() - l0
     dev_ms = cx.max_over_ranks(total_ms) / K
@@ -381,7 +388,7 @@ def bench_headline(cx, K, W):
                              "The 50 substeps are fused on chip, so the kernel is issue/latency-bound, not HBM-bound",
                      "substep_granular": {"achieved": achieved_sub, "frac": achieved_sub / hbm,
                                           "note": "752 B/substep x 50 substeps, as if the state round-tripped HBM every substep"}},
-        "clocks": clocks, "episodes_finished_in_last_timed_step": ndone,
+        "clocks": clocks, "episodes_finished_in_last_timed_step": ndone, "outputs": outputs,
     }
 
 
@@ -397,13 +404,12 @@ def bench_at_scale(cx, K):
     for w in range(PREROLL + 3):
         env3.step_dev(acts3[w % 8], obs3, rew3, done3)
     cx.barrier()
-    ka = max(3, min(K, 10))
-    tot3 = cx.timed_steps(lambda k: env3.step_dev(acts3[k % 8], obs3, rew3, done3), ka)
+    tot3 = cx.timed_steps(lambda k: env3.step_dev(acts3[k % 8], obs3, rew3, done3), K)
     cx.barrier()
-    ms3 = cx.max_over_ranks(tot3) / ka
+    ms3 = cx.max_over_ranks(tot3) / K
     hbm_peak = measured_peaks()[0]
     traffic, traffic_src = ncu_traffic("physics_kernel_262144")
-    at_scale = {"value": cx.world * na / (ms3 * 1e-3), "unit": "env-steps/s", "walkers_per_gpu": na, "ms_per_step": ms3, "steps": ka,
+    at_scale = {"value": cx.world * na / (ms3 * 1e-3), "unit": "env-steps/s", "walkers_per_gpu": na, "ms_per_step": ms3, "steps": K,
                 "kernel_variant": env3.get_variant(),
                 "roofline": {"bound": "hbm", "achieved": na * BYTES_PER_ENV_STEP / (ms3 * 1e-3) / 1e9, "peak": hbm_peak, "unit": "GB/s",
                              "frac": na * BYTES_PER_ENV_STEP / (ms3 * 1e-3) / 1e9 / hbm_peak,
@@ -419,12 +425,12 @@ def bench_at_scale(cx, K):
     for w in range(3):
         env4.step_dev(acts3[w % 8], obs3, rew3, done3)
     cx.barrier()
-    tot4 = cx.timed_steps(lambda k: env4.step_dev(acts3[k % 8], obs3, rew3, done3), ka)
+    tot4 = cx.timed_steps(lambda k: env4.step_dev(acts3[k % 8], obs3, rew3, done3), K)
     cx.barrier()
-    ms4 = cx.max_over_ranks(tot4) / ka
+    ms4 = cx.max_over_ranks(tot4) / K
     at_scale["iterations_1"] = {
         "value": cx.world * na / (ms4 * 1e-3), "unit": "substeps/s (Hyperparameters.Iterations = 1: one substep per env-step and per launch)",
-        "ms_per_step": ms4, "steps": ka, "kernel_variant": env4.get_variant(),
+        "ms_per_step": ms4, "steps": K, "kernel_variant": env4.get_variant(),
         "roofline": {"bound": "hbm", "achieved": na * BYTES_PER_ENV_STEP / (ms4 * 1e-3) / 1e9, "peak": hbm_peak, "unit": "GB/s",
                      "frac": na * BYTES_PER_ENV_STEP / (ms4 * 1e-3) / 1e9 / hbm_peak,
                      "note": "824 B per walker per launch (state in + out, actions, obs/reward/done)"}}
@@ -451,11 +457,10 @@ def bench_contact_stress(cx, K):
     for i in range(16):
         env.step_dev(acts[i % 8], obs, rew, done)
     cx.barrier()
-    k = max(5, min(K, 20))
-    tot = cx.timed_steps(lambda i: env.step_dev(acts[i % 8], obs, rew, done), k)
+    tot = cx.timed_steps(lambda i: env.step_dev(acts[i % 8], obs, rew, done), K)
     cx.barrier()
-    ms = cx.max_over_ranks(tot) / k
-    return {"value": cx.world * n / (ms * 1e-3), "unit": "env-steps/s", "walkers_per_gpu": n, "ms_per_step": ms, "steps": k,
+    ms = cx.max_over_ranks(tot) / K
+    return {"value": cx.world * n / (ms * 1e-3), "unit": "env-steps/s", "walkers_per_gpu": n, "ms_per_step": ms, "steps": K,
             "kernel_variant": env.get_variant(),
             "config": {"workload": "contact-stress sweep: 16384 walkers per GPU, 2048 per floor material (Ice..SuperRubber), initial spin "
                                    "U(-5,5) per body, random actions, timed from env-step 16 (BASELINE.json configs[4])"}}
@@ -571,10 +576,18 @@ def bench_ppo_loop(cx, fused):
     return out
 
 
+def dump_outputs(out_dir, arrays, suffix):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), np.ascontiguousarray(a, np.float32))
+
+
 def run_ours(args):
     cx = Ctx()
     K, W = args.steps, args.warmup
     head = bench_headline(cx, K, W)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, head["outputs"], f"_rank{cx.rank}" if cx.world > 1 else "")
     at_scale = bench_at_scale(cx, K)
     stress = bench_contact_stress(cx, K)
     loops = []
@@ -596,7 +609,7 @@ def run_ours(args):
             line["ppo_loop"] = {"config": {"workload": f"full PPO loop, {N_ENVS_LOOP} walkers sharded over {cx.world} GPU(s), horizon 64, global "
                                                        "minibatch 65536, 1 epoch (BASELINE.json configs[3])"}, "runs": loops}
         if not args.no_ppo:
-            line["secondary"], ppo_ctx = bench_ppo(cx, max(5, K), max(3, W))
+            line["secondary"], ppo_ctx = bench_ppo(cx, K, W)
             if cx.world == 1:
                 line["cfg1"] = {"config": {"workload": "single BipedalWalker env, physics step + PPO rollout/update (BASELINE.json configs[0])"},
                                 "gpu": bench_cfg1_gpu(cx)}
@@ -627,7 +640,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-ppo", action="store_true")
     ap.add_argument("--no-loop", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline's last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
