@@ -198,6 +198,45 @@ int32_t wb_scene_set_torques(wb_scene* scene, const float* torques_host);
 /* Environment.StepObjects(deltaTime) */
 int32_t wb_scene_step_objects(wb_scene* scene, float delta_time);
 
+/* ---- the walker on arbitrary terrain: Environment.Update with any IObject list in place of Environment.CreateFloor ----
+ * Hyperparameters.RoughFloor (Hyperparameters.cs:88) -> Environment.CreateRoughFloor (Environment.cs:230-261), or any 1..11 bodies
+ * (static floor hulls, obstacles, loose dynamic bodies).  Scene per copy: the walker's bodies [LLL, LLU, Body, RLL, RLU] and joints
+ * exactly as Walker.CreateCreature builds them (Walker.cs:40-46,155-209), then the terrain bodies; the association masks of the
+ * terrain descriptions index the terrain list.  List order: walker first as constructed (Environment.cs:46-48), terrain first
+ * after a Reset, which re-creates the walker and appends it (Environment.cs:167-173).  Same phases and results contract as
+ * wb_env_step: Terminal latches when Body, LLU or RLU touches any is_floor body (Walker.cs:49-54).  A Reset re-creates the
+ * walker only: terrain bodies keep their state.  Static terrain bodies are never written by an impulse, like the wb_env_* floor:
+ * finite impulses leave them unchanged anyway, and a NaN one (NaN actions) cannot corrupt terrain that outlives the walker's
+ * resets.  More than 11 terrain bodies: WB_ERR_UNSUPPORTED. */
+typedef struct wb_terrain_env wb_terrain_env;
+/* new Environment(...) x N (Environment.cs:39-51) over the terrain: vertices_xy = all terrain vertices, body by body, (x, y) */
+int32_t wb_terrain_env_create(int32_t n_envs, const wb_body_desc* terrain, int32_t n_terrain, const float* vertices_xy,
+                              int32_t walker_material, const wb_hyperparams* hp, wb_terrain_env** out);
+int32_t wb_terrain_env_destroy(wb_terrain_env* env);
+int32_t wb_terrain_env_set_stream(wb_terrain_env* env, void* cuda_stream);
+int32_t wb_terrain_env_state_floats(const wb_terrain_env* env, int32_t* per_copy_out);
+/* per-copy terrain: vertices [N][2 * terrain vertices] (same vertex counts as at create); cached centroids recomputed like
+ * Skeleton.FindCentroid (Skeleton.cs:100-113); terrain velocities / omega / angle and Collided cleared; the walker is not touched */
+int32_t wb_terrain_env_set_terrain(wb_terrain_env* env, const float* vertices_host);
+/* Environment.Reset + Walker.Reset + InitialState (Environment.cs:167-180, Walker.cs:212-236) for copies whose mask byte != 0
+ * (NULL: all); first_episode != 0 restores the constructor's list order (walker first) */
+int32_t wb_terrain_env_reset(wb_terrain_env* env, const uint8_t* mask_host, int32_t first_episode);
+/* floats [rows][N]: the wb_scene_* record, bodies in INDEX order [LLL, LLU, Body, RLL, RLU, terrain...], then the 4 joint torques;
+ * ints [3][N]: Collided bit per body index, flags (WB_FLAG_TERMINAL, WB_FLAG_FLOOR_FIRST = terrain before walker), Environment._steps */
+int32_t wb_terrain_env_get_state(wb_terrain_env* env, float* state_f_host, int32_t* state_i_host);
+int32_t wb_terrain_env_set_state(wb_terrain_env* env, const float* state_f_host, const int32_t* state_i_host);
+/* Walker.GetState (Walker.cs:132-152): obs [N][12] */
+int32_t wb_terrain_env_get_obs(wb_terrain_env* env, float* obs_host);
+/* Environment.Update minus the policy (Environment.cs:64-92), one launch: as wb_env_step; host buffers are staged (copy, launch,
+ * copy back, sync) */
+int32_t wb_terrain_env_step(wb_terrain_env* env, const float* actions_host, float delta_time, int32_t auto_reset, float* obs_host,
+                            float* reward_host, uint8_t* done_host);
+/* device-pointer variant: enqueue only (no copies, no sync) */
+int32_t wb_terrain_env_step_dev(wb_terrain_env* env, const float* actions_dev, float delta_time, int32_t auto_reset, float* obs_dev,
+                                float* reward_dev, uint8_t* done_dev);
+/* number of kernel launches this handle has issued */
+int32_t wb_terrain_env_launch_count(const wb_terrain_env* env, int64_t* count_out);
+
 /* ---- policy: Walker/PPO/PPOAgent.cs, Network/, Matrix.cs ---- */
 /* layer kinds of the network DSL (PPOAgent.ParseLayers, PPOAgent.cs:96-143) */
 enum { WB_DENSE = 0, WB_RELU = 1, WB_LEAKYRELU = 2, WB_TANH = 3 };

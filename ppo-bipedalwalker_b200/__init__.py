@@ -10,5 +10,5 @@ from . import dist  # noqa: F401
 from .ppo import *  # noqa: F401,F403
 from .loop import VectorPPO  # noqa: F401
 from .scene import (CreateCreature, CreateFloor, CreateRoughFloor, Hexagon, Hull, IObject, Joint, Pole, Scene, Square,  # noqa: F401
-                    Triangle)
+                    TerrainEnvBatch, Triangle)
 from .settings import DeserializeJson, SerializeJson, Settings  # noqa: F401

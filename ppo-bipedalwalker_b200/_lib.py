@@ -100,6 +100,18 @@ def lib() -> C.CDLL:
         "wb_scene_get_state": (C.c_int32, [vp, vp, vp]),
         "wb_scene_set_torques": (C.c_int32, [vp, vp]),
         "wb_scene_step_objects": (C.c_int32, [vp, C.c_float]),
+        "wb_terrain_env_create": (C.c_int32, [C.c_int32, C.POINTER(BodyDesc), C.c_int32, vp, C.c_int32, hpp, C.POINTER(vp)]),
+        "wb_terrain_env_destroy": (C.c_int32, [vp]),
+        "wb_terrain_env_set_stream": (C.c_int32, [vp, vp]),
+        "wb_terrain_env_state_floats": (C.c_int32, [vp, ip]),
+        "wb_terrain_env_set_terrain": (C.c_int32, [vp, vp]),
+        "wb_terrain_env_reset": (C.c_int32, [vp, vp, C.c_int32]),
+        "wb_terrain_env_get_state": (C.c_int32, [vp, vp, vp]),
+        "wb_terrain_env_set_state": (C.c_int32, [vp, vp, vp]),
+        "wb_terrain_env_get_obs": (C.c_int32, [vp, vp]),
+        "wb_terrain_env_step": (C.c_int32, [vp, vp, C.c_float, C.c_int32, vp, vp, vp]),
+        "wb_terrain_env_step_dev": (C.c_int32, [vp, vp, C.c_float, C.c_int32, vp, vp, vp]),
+        "wb_terrain_env_launch_count": (C.c_int32, [vp, i64p]),
         "wb_debug_rcp_sqrt_check": (C.c_int32, [C.c_uint32, C.c_uint64, C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
         "wb_policy_create": (C.c_int32, [C.c_int32, C.c_int32, vp, vp, C.c_int32, vp, vp, C.c_int32, hpp, C.POINTER(vp)]),
         "wb_policy_destroy": (C.c_int32, [vp]),

@@ -146,6 +146,11 @@ static void build_floor_constants(const float* floor10, FloorConst* fc) {
   }
 }
 
+void walker_initial_record(float* init92) {
+  float floor10[10];
+  build_scene_constants(init92, floor10);
+}
+
 }  // namespace wb
 
 using namespace wb;

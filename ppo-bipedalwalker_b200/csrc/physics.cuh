@@ -102,4 +102,28 @@ struct SceneParams {
 size_t scene_smem_bytes(const SceneConst& s);
 cudaError_t launch_scene(const SceneParams& p, const SceneConst& s, cudaStream_t stream);
 
+// ---- the walker on arbitrary terrain (physics_scene.cu: terrain_step_kernel): bodies [LLL, LLU, Body, RLL, RLU, terrain...]
+constexpr int kWalkerRecordInit = 68;  // the fresh walker's 29 vertices + 5 cached centroids (floats 0..67 of the 92-float record)
+struct TerrainConst {
+  SceneConst topo;
+  float walker_init[kWalkerRecordInit];
+};
+struct TerrainParams {
+  float* state;               // [rows][n_pad]: the SceneParams record over all bodies, then the 4 joint torques
+  int32_t* ints;              // [3][n_pad]: Collided bit per body index, flags (WB_FLAG_TERMINAL, WB_FLAG_FLOOR_FIRST), steps
+  const float* actions;       // [n][4]
+  const uint8_t* reset_mask;  // [n] or null
+  float* obs;                 // [n][12]
+  float* reward;              // [n]
+  uint8_t* done;              // [n]
+  int32_t n, n_pad;
+  float dt;
+  int32_t iterations, max_timesteps;
+  int32_t phases;             // kPhase* as PhysicsParams
+};
+cudaError_t terrain_kernel_setup();
+cudaError_t launch_terrain(const TerrainConst& tc, const TerrainParams& p, cudaStream_t stream);
+// Walker ctor + CreateCreature (api_env.cu): the 92-float record wb_env_create starts every walker from
+void walker_initial_record(float* init92);
+
 }  // namespace wb

@@ -5,7 +5,8 @@ TakeActions(Clip(a)), Step, record action / log-probability / reward, and at the
 values, returns, advantages, Epochs x shuffled mini-batches of Train(Batch) -- runs here for N walkers at once:
 
   rollout   `horizon` env-steps; per env-step TWO kernel launches: wb_policy_act_dev (actor + critic + Philox Box-Muller sampling +
-            log-probabilities) and wb_env_step_dev (the fused physics step with auto-reset).  The trajectory (states, UNCLIPPED
+            log-probabilities) and wb_env_step_dev (the fused physics step with auto-reset; wb_terrain_env_step_dev when the
+            walkers train on a terrain other than the flat floor).  The trajectory (states, UNCLIPPED
             actions and their log-probabilities -- Environment.cs:87-88 --, rewards, dones, values) stays in HBM, time-major.
   update    wb_segment_returns_dev (MC return / the reference's GAE per episode fragment; a fragment that is still running at the
             end of the horizon is bootstrapped with the critic's value of the next observation -- the reference never meets this
@@ -33,12 +34,16 @@ from . import dist as _dist
 from ._lib import ACT, OBS, Hyperparams, check, lib, ptr
 from .env import DT_FRAME, EnvBatch, default_hyperparams
 from .ppo import PPOAgent
+from .scene import IObject, TerrainEnvBatch
 
 
 class VectorPPO:
     def __init__(self, n_envs_global: int, horizon: int = 64, minibatch_global: int = 65536, epochs: int = 1,
                  floor="Metal", walker="Carpet", hp: Hyperparams | None = None, seed: int = 0, policy_variant: int | None = None,
-                 fused_allreduce: bool = True, bootstrap: bool = True):
+                 fused_allreduce: bool = True, bootstrap: bool = True, terrain=None):
+        """terrain: None (the reference's flat floor of material `floor`, wb_env_*), or an IObject list in its place (e.g.
+        CreateRoughFloor(heights)) shared by every walker, or a list of n_envs_global such lists, indexed by the GLOBAL walker
+        index (wb_terrain_env_*; `floor` is then unused: the terrain bodies carry their materials)."""
         import torch
         self.torch = torch
         self.rank, self.local_rank, self.world = _dist.world()
@@ -61,7 +66,16 @@ class VectorPPO:
         self.hp = hp if hp is not None else default_hyperparams()
         self.hp.batch_size = minibatch_global  # the divisor B of every per-sample gradient (PPOAgent.cs:326,333)
         self.stream = torch.cuda.current_stream().cuda_stream
-        self.env = EnvBatch(self.n, floor_materials=floor, walker_materials=walker, hp=self.hp, stream=self.stream)
+        if terrain is None:
+            self.env = EnvBatch(self.n, floor_materials=floor, walker_materials=walker, hp=self.hp, stream=self.stream)
+            self._env_step_dev = lib().wb_env_step_dev
+        else:
+            terrain = list(terrain)
+            if terrain and not isinstance(terrain[0], IObject):  # one list per walker: this rank's block of the global index
+                assert len(terrain) == n_envs_global, "a per-walker terrain needs one IObject list per walker"
+                terrain = terrain[lo:hi]
+            self.env = TerrainEnvBatch(self.n, terrain, walker_material=walker, hp=self.hp, stream=self.stream)
+            self._env_step_dev = lib().wb_terrain_env_step_dev
         self.agent = PPOAgent(hp=self.hp, seed=seed, stream=self.stream)  # same seed -> identical Xavier weights on every rank
         if policy_variant is not None:
             self.agent.set_variant(policy_variant)
@@ -99,8 +113,8 @@ class VectorPPO:
             # distinct Philox streams per rank: the counter is (local sample index, action dim, step)
             check(L.wb_policy_act_dev(h_agent, self.n, ptr(self.obs), self.seed * 7919 + self.rank, self.step_counter, ptr(self.actions[t]),
                                       ptr(self.logp[t]), None, ptr(self.values[t])))
-            check(L.wb_env_step_dev(h_env, ptr(self.actions[t]), C.c_float(DT_FRAME), 1, ptr(self.obs), ptr(self.rewards[t]),
-                                    ptr(self.dones[t])))
+            check(self._env_step_dev(h_env, ptr(self.actions[t]), C.c_float(DT_FRAME), 1, ptr(self.obs), ptr(self.rewards[t]),
+                                     ptr(self.dones[t])))
             self.step_counter += 1
 
     # -- update: returns/advantages, epochs x mini-batches with one all-reduce each

@@ -3,7 +3,8 @@
 Host-side mirror of the shape factories -- `Square.FromSize` (Square.cs:18-32), `Triangle.FromSize` (Triangle.cs:18-31),
 `Hexagon.FromSize` (Hexagon.cs:18-34), `Pole.FromSize` (Pole.cs:18-34), `Hull.FromPositions` (Hull.cs:18-29),
 `Skeleton.SmoothCorners` (Skeleton.cs:33-53) -- and of `Joint` (Joint.cs), plus `Scene`, which hands the lists to
-libwalker_b200 (`wb_scene_*`) and runs `Environment.StepObjects` (Environment.cs:126-143) on the GPU.  Vertex templates are
+libwalker_b200 (`wb_scene_*`) and runs `Environment.StepObjects` (Environment.cs:126-143) on the GPU, and `TerrainEnvBatch`, the
+walker environment on any such list in place of the flat floor (`wb_terrain_env_*`).  Vertex templates are
 computed here in float32 with the reference's formulas; all stepping happens in csrc/physics_scene.cu (no CPU path).
 """
 from __future__ import annotations
@@ -13,8 +14,8 @@ from dataclasses import dataclass, field
 
 import numpy as np
 
-from ._lib import BodyDesc, JointDesc, check, lib, ptr
-from .env import DT_FRAME, IMaterial, MATERIALS
+from ._lib import ACT, OBS, BodyDesc, Hyperparams, JointDesc, check, lib, ptr
+from .env import DT_FRAME, IMaterial, MATERIALS, default_hyperparams
 
 f32 = np.float32
 
@@ -106,6 +107,24 @@ class Joint:
     indexB: int
 
 
+def _body_desc(o: IObject, index: dict) -> BodyDesc:
+    mask = 0
+    for a in o.associated:
+        mask |= 1 << index[id(a)]
+    return BodyDesc(len(o.vertices), int(o.isStatic), int(o.isFloor), _material_id(o.material), mask, float(o.acceleration[0]),
+                    float(o.acceleration[1]), float(o.inverseInertia))
+
+
+def _describe(objects):
+    """IObject list -> (wb_body_desc array, all vertices concatenated (x, y) float32); associations index the list."""
+    index = {id(o): i for i, o in enumerate(objects)}
+    descs = (BodyDesc * len(objects))()
+    for i, o in enumerate(objects):
+        descs[i] = _body_desc(o, index)
+    vflat = np.ascontiguousarray(np.concatenate([np.asarray(o.vertices, f32).reshape(-1) for o in objects]), f32)
+    return descs, vflat
+
+
 class Scene:
     """N lockstep copies of `objects` (+ `joints`): Environment._rigidBodies in list order."""
 
@@ -115,18 +134,8 @@ class Scene:
         self.joints = list(joints)
         B, J = len(self.objects), len(self.joints)
         index = {id(o): i for i, o in enumerate(self.objects)}
-        descs = (BodyDesc * B)()
-        verts = []
-        for i, o in enumerate(self.objects):
-            v = np.ascontiguousarray(o.vertices, f32).reshape(-1, 2)
-            mask = 0
-            for a in o.associated:
-                mask |= 1 << index[id(a)]
-            descs[i] = BodyDesc(len(v), int(o.isStatic), int(o.isFloor), _material_id(o.material), mask, float(o.acceleration[0]),
-                                float(o.acceleration[1]), float(o.inverseInertia))
-            verts.append(v.reshape(-1))
+        descs, vflat = _describe(self.objects)
         self.vertex_counts = [len(o.vertices) for o in self.objects]
-        vflat = np.ascontiguousarray(np.concatenate(verts), f32)
         jd = (JointDesc * max(J, 1))()
         for k, j in enumerate(self.joints):
             jd[k] = JointDesc(index[id(j.bodyA)], j.indexA, index[id(j.bodyB)], j.indexB)
@@ -163,6 +172,121 @@ class Scene:
 
     def StepObjects(self, deltaTime: float = DT_FRAME):  # Environment.cs:126-143
         check(lib().wb_scene_step_objects(self._h, C.c_float(deltaTime)))
+
+
+def _signature(objects) -> list:
+    index = {id(o): i for i, o in enumerate(objects)}
+    return [tuple(getattr(_body_desc(o, index), k) for k, _ in BodyDesc._fields_) for o in objects]
+
+
+class TerrainEnvBatch:
+    """N walkers, each on its own copy of a terrain (wb_terrain_env handle): Environment.Update (Environment.cs:64-92) with the
+    IObject list `terrain` in place of Environment.CreateFloor -- e.g. CreateRoughFloor(heights) for Hyperparameters.RoughFloor.
+
+    `terrain` is one IObject list shared by every walker, or a list of n such lists with the same topology (vertex counts, flags,
+    materials, associations); their vertices are loaded per copy with set_terrain.  The methods follow EnvBatch; get_state
+    returns the full record ([n, state_floats] floats over [LLL, LLU, Body, RLL, RLU, terrain...] in index order + 4 joint
+    torques, [n, 3] ints: Collided bits per body index, flags, steps) and walker_state() the walker's part as EnvBatch.get_state
+    has it."""
+
+    def __init__(self, n: int, terrain, walker_material="Carpet", hp: Hyperparams | None = None, stream: int | None = None):
+        self.n = int(n)
+        self.hp = hp if hp is not None else default_hyperparams()
+        terrain = list(terrain)
+        per_copy = len(terrain) > 0 and not isinstance(terrain[0], IObject)
+        if per_copy:
+            if len(terrain) != self.n:
+                raise ValueError(f"a per-copy terrain needs {self.n} IObject lists, got {len(terrain)}")
+            first = list(terrain[0])
+            sig = _signature(first)
+            for t in terrain[1:]:
+                if _signature(list(t)) != sig:
+                    raise ValueError("every copy's terrain must have the same topology as the first")
+        else:
+            first = terrain
+        self.objects = first
+        descs, vflat = _describe(first) if first else ((BodyDesc * 0)(), np.zeros(0, f32))
+        self.vertex_counts = [len(o.vertices) for o in first]
+        h = C.c_void_p()
+        check(lib().wb_terrain_env_create(self.n, descs, len(first), ptr(vflat), _material_id(walker_material), C.byref(self.hp),
+                                          C.byref(h)))
+        self._h = h
+        if stream is not None:
+            self.set_stream(stream)
+        k = C.c_int32(0)
+        check(lib().wb_terrain_env_state_floats(self._h, C.byref(k)))
+        self.state_floats = k.value
+        self.n_bodies = 5 + len(first)
+        self.total_verts = 29 + sum(self.vertex_counts)
+        if per_copy:
+            self.set_terrain(np.stack([np.concatenate([np.asarray(o.vertices, f32).reshape(-1) for o in t]) for t in terrain]))
+
+    def close(self):
+        if getattr(self, "_h", None) and lib is not None:
+            lib().wb_terrain_env_destroy(self._h)
+            self._h = None
+
+    __del__ = close
+
+    def set_stream(self, cuda_stream: int):
+        check(lib().wb_terrain_env_set_stream(self._h, C.c_void_p(cuda_stream)))
+
+    def launch_count(self) -> int:
+        out = C.c_int64(0)
+        check(lib().wb_terrain_env_launch_count(self._h, C.byref(out)))
+        return out.value
+
+    def set_terrain(self, vertices):
+        """Per-copy terrain vertices [n, 2 * terrain vertices] (x, y interleaved, body by body); the walkers are not touched."""
+        v = np.asarray(vertices, f32)
+        want = 2 * sum(self.vertex_counts)
+        if v.ndim != 2 or v.shape != (self.n, want):
+            raise ValueError(f"terrain vertices must have shape ({self.n}, {want}), got {v.shape}")
+        check(lib().wb_terrain_env_set_terrain(self._h, ptr(np.ascontiguousarray(v))))
+
+    def get_state(self):
+        f = np.empty((self.state_floats, self.n), np.float32)
+        iv = np.empty((3, self.n), np.int32)
+        check(lib().wb_terrain_env_get_state(self._h, ptr(f), ptr(iv)))
+        return np.ascontiguousarray(f.T), np.ascontiguousarray(iv.T)
+
+    def set_state(self, f, iv):
+        f = np.ascontiguousarray(np.asarray(f, np.float32).reshape(self.n, self.state_floats).T)
+        iv = np.ascontiguousarray(np.asarray(iv, np.int32).reshape(self.n, 3).T)
+        check(lib().wb_terrain_env_set_state(self._h, ptr(f), ptr(iv)))
+
+    def walker_state(self):
+        """The walker's part of the record as EnvBatch.get_state returns it: ([n, 92] floats, [n, 2] ints: flags, steps)."""
+        g, iv = self.get_state()
+        tv, B = self.total_verts, self.n_bodies
+        f = np.concatenate([g[:, 0:58], g[:, 2 * tv:2 * tv + 10], g[:, 2 * tv + 2 * B:2 * tv + 2 * B + 10],
+                            g[:, 2 * tv + 4 * B:2 * tv + 4 * B + 5], g[:, 2 * tv + 5 * B:2 * tv + 5 * B + 5],
+                            g[:, 2 * tv + 6 * B:2 * tv + 6 * B + 4]], axis=1)
+        ints = np.stack([(iv[:, 0] & 0x1F) | iv[:, 1], iv[:, 2]], axis=1).astype(np.int32)
+        return np.ascontiguousarray(f), ints
+
+    def reset(self, mask=None, first_episode: bool = False):
+        m = None if mask is None else np.ascontiguousarray(mask, np.uint8)
+        check(lib().wb_terrain_env_reset(self._h, ptr(m), int(first_episode)))
+
+    def get_obs(self):
+        obs = np.empty((self.n, OBS), np.float32)
+        check(lib().wb_terrain_env_get_obs(self._h, ptr(obs)))
+        return obs
+
+    def step(self, actions, delta_time: float = DT_FRAME, auto_reset: bool = True, out=None):
+        """actions [n, 4] -> (obs [n, 12], reward [n], done [n]) host arrays; one kernel launch."""
+        a = np.ascontiguousarray(actions, np.float32).reshape(self.n, ACT)
+        if out is None:
+            out = (np.empty((self.n, OBS), np.float32), np.empty(self.n, np.float32), np.empty(self.n, np.uint8))
+        obs, rew, done = out
+        check(lib().wb_terrain_env_step(self._h, ptr(a), delta_time, int(auto_reset), ptr(obs), ptr(rew), ptr(done)))
+        return obs, rew, done
+
+    def step_dev(self, actions_dev, obs_dev, reward_dev, done_dev, delta_time: float = DT_FRAME, auto_reset: bool = True):
+        """Device pointers (ints or torch CUDA tensors); enqueues on the handle's stream, no sync."""
+        check(lib().wb_terrain_env_step_dev(self._h, ptr(actions_dev), delta_time, int(auto_reset), ptr(obs_dev), ptr(reward_dev),
+                                            ptr(done_dev)))
 
 
 # ---------------------------------------------------------------- the reference's own scene pieces as IObject lists
@@ -218,4 +342,4 @@ def CreateCreature(position=(125, 800), material="Carpet"):
     return objs, joints
 
 
-__all__ = ["IObject", "Square", "Triangle", "Hexagon", "Pole", "Hull", "Joint", "Scene", "CreateFloor", "CreateRoughFloor", "CreateCreature"]
+__all__ = ["IObject", "Square", "Triangle", "Hexagon", "Pole", "Hull", "Joint", "Scene", "TerrainEnvBatch", "CreateFloor", "CreateRoughFloor", "CreateCreature"]
