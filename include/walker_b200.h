@@ -343,6 +343,32 @@ int32_t wb_ppo_train_indexed_dev(wb_policy* p, int32_t n, const int32_t* index_d
  * pageable buffers are staged.  losses / skipped as wb_ppo_grad. */
 int32_t wb_ppo_train(wb_policy* p, int32_t n, const float* states_host, const float* actions_host, const float* old_logp_host,
                      const float* advantages_host, const float* returns_host, float* losses_host, int32_t* skipped_host);
+/* PPOAgent.Train(Trajectory) (PPOAgent.cs:147-172) for n_traj complete episodes, in list order: trajectory e is trained with the
+ * weights trajectory e-1 left, exactly as n_traj calls of Train.  offsets_host[n_traj+1] (HOST, in both entries; non-decreasing,
+ * offsets[0] >= 0) delimits trajectory e = rows [offsets[e], offsets[e+1]) of states [.][state], actions / old_logp [.][act]
+ * (UNclipped, Environment.cs:87-88) and rewards [.].  Per trajectory: CalculateValues (critic forward), MC return or GAE and the
+ * optional Normalize (PPOAgent.cs:175-189,414-498), then epochs x floor(T_e / B) mini-batches of B = hp.batch_size samples, each
+ * Train(Batch) + Adam.  batch_index: per trajectory, epochs x floor(T_e / B) x B LOCAL row numbers (PPOAgent.CreateBatches,
+ * :501-540; the caller draws them, like the injected Box-Muller uniforms), blocks concatenated in trajectory order.
+ * values / returns / advantages [.] (Trajectory.Values / Returns / Advantages) may be NULL.  losses [n_traj][2] = the last
+ * mini-batch's {sum g_V, sum mean_k g_mu} (0 if T_e < B), skipped [n_traj] = skipped samples over all of the trajectory's
+ * mini-batches; either may be NULL.  A trajectory with T_e < B gets its values / returns / advantages but trains nothing and
+ * consumes no Adam step.  The Adam bias corrections are computed on the host exactly as for wb_adam_step; the gradient buffer
+ * then holds the last trained mini-batch's gradient, losses and skipped count, as after wb_ppo_train.  The default networks
+ * (kernel variants 0 and 1) train in ONE launch: one persistent CTA runs the whole chain of Adam steps without a host round
+ * trip; other networks and variant 2 enqueue the per-trajectory and per-mini-batch kernels with no host sync.  The host entry
+ * range-checks every index and refuses bad offsets, epochs < 0, n_traj < 1 and hp.batch_size < 1 with WB_ERR_INVALID before
+ * anything on the device changes.  A policy connected for data-parallel exchange (world > 1) gets WB_ERR_UNSUPPORTED. */
+int32_t wb_ppo_train_trajectories(wb_policy* p, int32_t n_traj, const int32_t* offsets_host, int32_t epochs, const float* states_host,
+                                  const float* actions_host, const float* old_logp_host, const float* rewards_host,
+                                  const int32_t* batch_index_host, float* values_host, float* returns_host, float* advantages_host,
+                                  float* losses_host, int32_t* skipped_host);
+/* The same with every pointer except offsets_host on the device; enqueue only.  Every index must be a valid local row of its
+ * trajectory: the kernels do not range-check device indices. */
+int32_t wb_ppo_train_trajectories_dev(wb_policy* p, int32_t n_traj, const int32_t* offsets_host, int32_t epochs, const float* states_dev,
+                                      const float* actions_dev, const float* old_logp_dev, const float* rewards_dev,
+                                      const int32_t* batch_index_dev, float* values_dev, float* returns_dev, float* advantages_dev,
+                                      float* losses_dev, int32_t* skipped_dev);
 /* NeuralNetwork.Optimise -> DenseLayer.Adam on both networks (NeuralNetwork.cs:85-91, DenseLayer.cs:125-159) */
 int32_t wb_adam_step(wb_policy* p);
 /* device address + length of the contiguous gradient buffer [actor | critic | 2 loss sums | skipped] for the

@@ -138,6 +138,8 @@ def lib() -> C.CDLL:
         "wb_ppo_train_dev": (C.c_int32, [vp, C.c_int32, vp, vp, vp, vp, vp]),
         "wb_ppo_train_indexed_dev": (C.c_int32, [vp, C.c_int32, vp, vp, vp, vp, vp, vp]),
         "wb_ppo_train": (C.c_int32, [vp, C.c_int32, vp, vp, vp, vp, vp, vp, vp]),
+        "wb_ppo_train_trajectories": (C.c_int32, [vp, C.c_int32, vp, C.c_int32] + [vp] * 10),
+        "wb_ppo_train_trajectories_dev": (C.c_int32, [vp, C.c_int32, vp, C.c_int32] + [vp] * 10),
         "wb_segment_returns_dev": (C.c_int32, [vp, C.c_int32, C.c_int32, vp, vp, vp, vp, vp, vp]),
         "wb_normalize_advantages_dev": (C.c_int32, [vp, C.c_int32, C.c_int64, C.c_int64, vp]),
         "wb_normalize_stats_buffer": (C.c_int32, [vp, C.POINTER(vp), ip]),

@@ -170,6 +170,62 @@ public sealed class GpuPPOAgent : IDisposable
         if (Hyperparameters.SaveWeights) Save();
     }
 
+    // Train(Trajectory, Renderer) for every finished episode of the list, in list order, as ONE native call
+    // (wb_ppo_train_trajectories: one kernel launch on the default networks).  CreateBatches is drawn from _random in the order
+    // the single-trajectory overload draws it, so the mini-batches are the same.  Deviation: the per-mini-batch
+    // renderer.UpdateConsole becomes one update per trajectory (its last mini-batch), since the mini-batches run on the device.
+    public void Train(IReadOnlyList<Trajectory> trajectories, Renderer renderer)
+    {
+        var hp = WbHyperparams.FromStatics();
+        Wb.Ok(Wb.wb_policy_set_hyperparams(_policy, ref hp), "wb_policy_set_hyperparams");
+        int n = trajectories.Count, B = Hyperparameters.BatchSize, epochs = Hyperparameters.Epochs;
+        if (n == 0) return;
+        var offsets = new int[n + 1];
+        for (int e = 0; e < n; e++) offsets[e + 1] = offsets[e] + trajectories[e].States.Count;
+        int rows = offsets[n];
+        float[] states = new float[rows * _stateSize], actions = new float[rows * _actionSize], logp = new float[rows * _actionSize];
+        float[] rewards = new float[rows];
+        var index = new List<int>();
+        for (int e = 0; e < n; e++)
+        {
+            var t = trajectories[e];
+            int T = t.States.Count, o = offsets[e];
+            Array.Copy(Flatten(t.States, _stateSize), 0, states, o * _stateSize, T * _stateSize);
+            Array.Copy(Flatten(t.Actions, _actionSize), 0, actions, o * _actionSize, T * _actionSize);
+            Array.Copy(Flatten(t.LogProbabilities, _actionSize), 0, logp, o * _actionSize, T * _actionSize);
+            t.Rewards.CopyTo(rewards, o);
+            for (int epoch = 0; epoch < epochs; epoch++)  // CreateBatches (:501-540), as in Train(Trajectory, Renderer)
+            {
+                var pool = Enumerable.Range(0, T).ToList();
+                for (int j = 0; j < T / B; j++)
+                    for (int b = 0; b < B; b++)
+                    {
+                        int pick = _random.Next(0, pool.Count);
+                        index.Add(pool[pick]);
+                        pool.RemoveAt(pick);
+                    }
+            }
+        }
+        float[] values = new float[rows], returns = new float[rows], advantages = new float[rows], losses = new float[2 * n];
+        var skipped = new int[n];
+        Wb.Ok(Wb.wb_ppo_train_trajectories(_policy, n, offsets, epochs, states, actions, logp, rewards, index.ToArray(), values, returns,
+                                           advantages, losses, skipped), "wb_ppo_train_trajectories");
+        for (int e = 0; e < n; e++)
+        {
+            var t = trajectories[e];
+            int T = t.States.Count, o = offsets[e];
+            if (T == 0) continue;  // Train returns before anything is recorded
+            t.Values.Clear(); t.Values.AddRange(new ArraySegment<float>(values, o, T));
+            t.Returns.Clear(); t.Returns.AddRange(new ArraySegment<float>(returns, o, T));
+            t.Advantages.Clear(); t.Advantages.AddRange(new ArraySegment<float>(advantages, o, T));
+            renderer.AddTotalEpisodeReward(t.Rewards.Sum());
+            if (T >= B) renderer.UpdateConsole(epochs - 1, T / B - 1, T / B, losses[2 * e]);
+            renderer.AddCriticLoss(losses[2 * e]);
+            renderer.AddActorLoss(losses[2 * e + 1]);
+        }
+        if (Hyperparameters.SaveWeights) Save();
+    }
+
     private static float[] Flatten(List<Matrix> rows, int width)
     {
         var flat = new float[rows.Count * width];

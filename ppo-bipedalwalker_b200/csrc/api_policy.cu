@@ -1,6 +1,7 @@
 // api_policy.cu -- C ABI for the PPO policy/value networks (include/walker_b200.h).  Compute is in mlp.cu.
 #include <cmath>
 #include <cstdlib>
+#include <cstring>
 #include <new>
 #include <vector>
 
@@ -42,6 +43,13 @@ struct wb_policy {
   void* opened[kExchMaxWorld] = {};  // IPC mappings to close
   int comm_rank = -1, comm_world = 0;
   uint32_t comm_epoch = 0;
+  // wb_ppo_train_trajectories: device offsets + Adam correction table (uploaded from a pinned host copy), scratch rows
+  char* h_episode_tab = nullptr;
+  char* d_episode_tab = nullptr;
+  size_t episode_tab_bytes = 0;
+  cudaEvent_t episode_tab_copied = nullptr;  // the previous upload has left the pinned copy
+  float* d_episode_scratch = nullptr;
+  size_t episode_scratch_floats = 0;
 };
 
 static int32_t ensure_stage(wb_policy* p, size_t floats) {
@@ -246,6 +254,10 @@ int32_t wb_policy_destroy(wb_policy* p) {
   cudaFree(p->d_comm_dead);
   cudaFree(p->d_partials);
   cudaFree(p->d_stage);
+  if (p->h_episode_tab) cudaFreeHost(p->h_episode_tab);
+  cudaFree(p->d_episode_tab);
+  if (p->episode_tab_copied) cudaEventDestroy(p->episode_tab_copied);
+  cudaFree(p->d_episode_scratch);
   delete p;
   return WB_OK;
 }
@@ -822,6 +834,217 @@ int32_t wb_returns_advantages(wb_policy* p, int32_t n, const float* rewards_host
   p->launches++;
   WB_CUDA(cudaMemcpyAsync(returns_host, d_G, sizeof(float) * N, cudaMemcpyDeviceToHost, p->stream));
   WB_CUDA(cudaMemcpyAsync(advantages_host, d_A, sizeof(float) * N, cudaMemcpyDeviceToHost, p->stream));
+  WB_CUDA(cudaStreamSynchronize(p->stream));
+  return WB_OK;
+}
+
+// ---- PPOAgent.Train(Trajectory) for a list of trajectories
+// offsets: non-decreasing, offsets[0] >= 0; counts the Adam steps (epochs x floor(T_e / B) per trajectory) and index entries
+static int32_t check_trajectories(const wb_policy* p, int32_t n_traj, const int32_t* offsets_host, int32_t epochs, int64_t* steps,
+                                  int64_t* n_index) {
+  WB_REQUIRE(offsets_host, "offsets_host is null");
+  WB_REQUIRE(n_traj >= 1, "n_traj must be at least 1");
+  WB_REQUIRE(epochs >= 0, "epochs must be >= 0");
+  WB_REQUIRE(p->hp.batch_size >= 1, "hp.batch_size must be positive");
+  if (p->comm_world > 1)
+    return fail(WB_ERR_UNSUPPORTED, "the per-episode schedule is single-process (PPOAgent.cs:147-172); this policy is connected for data-parallel exchange");
+  WB_REQUIRE(offsets_host[0] >= 0, "offsets[0] must be >= 0");
+  *steps = 0;
+  *n_index = 0;
+  for (int32_t e = 0; e < n_traj; e++) {
+    if (offsets_host[e + 1] < offsets_host[e]) return fail(WB_ERR_INVALID, "offsets must be non-decreasing (offsets[%d] > offsets[%d])", e, e + 1);
+    const int64_t nb = (int64_t)epochs * ((offsets_host[e + 1] - offsets_host[e]) / p->hp.batch_size);
+    *steps += nb;
+    *n_index += nb * p->hp.batch_size;
+  }
+  WB_REQUIRE(*n_index <= INT32_MAX, "too many mini-batch indices for one call");
+  return WB_OK;
+}
+
+static int32_t grow(float** buf, size_t* have, size_t want) {
+  if (want <= *have) return WB_OK;
+  cudaFree(*buf);
+  *buf = nullptr;
+  *have = 0;
+  WB_CUDA(cudaMalloc(buf, want * sizeof(float)));
+  *have = want;
+  return WB_OK;
+}
+
+int32_t wb_ppo_train_trajectories_dev(wb_policy* p, int32_t n_traj, const int32_t* offsets_host, int32_t epochs, const float* states_dev,
+                                      const float* actions_dev, const float* old_logp_dev, const float* rewards_dev,
+                                      const int32_t* batch_index_dev, float* values_dev, float* returns_dev, float* advantages_dev,
+                                      float* losses_dev, int32_t* skipped_dev) {
+  WB_REQUIRE(p && states_dev && actions_dev && old_logp_dev && rewards_dev, "null argument");
+  int64_t steps = 0, n_index = 0;
+  if (int32_t rc = check_trajectories(p, n_traj, offsets_host, epochs, &steps, &n_index)) return rc;
+  WB_REQUIRE(batch_index_dev || n_index == 0, "batch_index is null");
+  const size_t rows = (size_t)offsets_host[n_traj];
+  const int B = p->hp.batch_size;
+  const size_t IN = (size_t)p->actor.input, ACT = (size_t)p->actor.output;
+  // Trajectory.Values / Returns / Advantages the caller does not want, and the sequenced path's gathered mini-batch
+  const size_t mb_floats = use_generic(p) ? (size_t)B * (IN + 2 * ACT + 2) : 0;
+  const size_t scratch_rows = (values_dev ? 0 : rows) + (returns_dev ? 0 : rows) + (advantages_dev ? 0 : rows);
+  if (int32_t rc = grow(&p->d_episode_scratch, &p->episode_scratch_floats, scratch_rows + mb_floats + 1)) return rc;
+  float* scratch = p->d_episode_scratch;
+  if (!values_dev) { values_dev = scratch; scratch += rows; }
+  if (!returns_dev) { returns_dev = scratch; scratch += rows; }
+  if (!advantages_dev) { advantages_dev = scratch; scratch += rows; }
+
+  if (use_generic(p)) {
+    // networks the one-launch kernel does not cover: the per-trajectory / per-mini-batch kernels, enqueued without a host sync
+    float* g_states = scratch;
+    float* g_actions = g_states + (size_t)B * IN;
+    float* g_logp = g_actions + (size_t)B * ACT;
+    float* g_adv = g_logp + (size_t)B * ACT;
+    float* g_ret = g_adv + B;
+    if (losses_dev) WB_CUDA(cudaMemsetAsync(losses_dev, 0, sizeof(float) * 2 * n_traj, p->stream));
+    if (skipped_dev) WB_CUDA(cudaMemsetAsync(skipped_dev, 0, sizeof(int32_t) * n_traj, p->stream));
+    const int32_t* index = batch_index_dev;
+    for (int32_t e = 0; e < n_traj; e++) {
+      const int r0 = offsets_host[e], T = offsets_host[e + 1] - r0;
+      if (T == 0) continue;
+      MlpParams f;
+      fill_mlp_common(p, f, T, kModeForward);
+      f.states = states_dev + (size_t)r0 * IN;
+      f.value = values_dev + r0;
+      WB_CUDA(run_mlp(p, f));
+      WB_CUDA(launch_returns(rewards_dev + r0, values_dev + r0, T, p->hp.gamma, p->hp.lambda, p->hp.use_gae, p->hp.normalize_advantages,
+                             p->hp.epsilon, returns_dev + r0, advantages_dev + r0, p->stream));
+      p->launches += 2;
+      const int nb = epochs * (T / B);
+      for (int b = 0; b < nb; b++, index += B) {
+        WB_CUDA(launch_gather_rows(index, B, r0, (int)IN, (int)ACT, states_dev, actions_dev, old_logp_dev, advantages_dev, returns_dev, g_states,
+                                   g_actions, g_logp, g_adv, g_ret, p->stream));
+        MlpParams m;
+        fill_mlp_common(p, m, B, kModeGrad);
+        m.states = g_states;
+        m.actions = g_actions;
+        m.old_logp = g_logp;
+        m.advantages = g_adv;
+        m.returns = g_ret;
+        m.partials = p->d_partials;
+        WB_CUDA(run_mlp(p, m));
+        WB_CUDA(reduce_grads(p, grid_of(p, B)));
+        WB_CUDA(adam_any(p));
+        WB_CUDA(launch_episode_losses(p->d_grads + p->n_total, losses_dev ? losses_dev + 2 * e : nullptr, skipped_dev ? skipped_dev + e : nullptr,
+                                      p->stream));
+        p->launches += 5;
+      }
+    }
+    return WB_OK;
+  }
+
+  // default networks: ONE launch.  Table = device offsets [n_traj + 1] then the Adam bias corrections [steps][10] (next_corrections,
+  // the function every other Adam entry uses, so wb_policy_get_adam reports what the per-mini-batch path reports)
+  const size_t off_bytes = ((sizeof(int32_t) * (n_traj + 1)) + 15) / 16 * 16;
+  const size_t tab_bytes = off_bytes + sizeof(float) * 10 * (size_t)steps;
+  if (!p->episode_tab_copied) WB_CUDA(cudaEventCreateWithFlags(&p->episode_tab_copied, cudaEventDisableTiming));
+  WB_CUDA(cudaEventSynchronize(p->episode_tab_copied));  // (the previous call's upload has read the pinned copy)
+  if (tab_bytes > p->episode_tab_bytes) {
+    if (p->h_episode_tab) cudaFreeHost(p->h_episode_tab);
+    cudaFree(p->d_episode_tab);
+    p->h_episode_tab = nullptr;
+    p->d_episode_tab = nullptr;
+    p->episode_tab_bytes = 0;
+    WB_CUDA(cudaHostAlloc(&p->h_episode_tab, tab_bytes, cudaHostAllocDefault));
+    WB_CUDA(cudaMalloc(&p->d_episode_tab, tab_bytes));
+    p->episode_tab_bytes = tab_bytes;
+  }
+  memcpy(p->h_episode_tab, offsets_host, sizeof(int32_t) * (n_traj + 1));
+  float* corr = reinterpret_cast<float*>(p->h_episode_tab + off_bytes);
+  for (int64_t st = 0; st < steps; st++) next_corrections(p, corr + 10 * st, corr + 10 * st + 5);
+  WB_CUDA(cudaMemcpyAsync(p->d_episode_tab, p->h_episode_tab, tab_bytes, cudaMemcpyHostToDevice, p->stream));
+  WB_CUDA(cudaEventRecord(p->episode_tab_copied, p->stream));
+  EpisodeParams e{};
+  e.rewards = rewards_dev;
+  e.values = values_dev;
+  e.returns = returns_dev;
+  e.advantages = advantages_dev;
+  e.offsets = reinterpret_cast<const int32_t*>(p->d_episode_tab);
+  e.batch_index = batch_index_dev;
+  e.corr = reinterpret_cast<const float*>(p->d_episode_tab + off_bytes);
+  e.grads = p->d_grads;
+  e.losses = losses_dev;
+  e.skipped = skipped_dev;
+  e.adam.params = p->d_params;
+  e.adam.grads = p->d_grads;
+  e.adam.m = p->d_m;
+  e.adam.v = p->d_v;
+  e.adam.alpha = p->hp.alpha;
+  e.adam.beta1 = p->hp.beta1;
+  e.adam.beta2 = p->hp.beta2;
+  e.adam.eps = p->hp.adam_epsilon;
+  e.n_traj = n_traj;
+  e.epochs = epochs;
+  e.batch = B;
+  e.use_gae = p->hp.use_gae;
+  e.normalize = p->hp.normalize_advantages;
+  e.gamma = p->hp.gamma;
+  e.lambda = p->hp.lambda;
+  e.norm_eps = p->hp.epsilon;
+  MlpParams m;
+  fill_mlp_common(p, m, (int)rows, kModeGrad);
+  m.states = states_dev;
+  m.actions = actions_dev;
+  m.old_logp = old_logp_dev;
+  m.advantages = advantages_dev;
+  m.returns = returns_dev;
+  WB_CUDA(launch_episodes(e, m, p->stream));
+  p->launches++;
+  return WB_OK;
+}
+
+int32_t wb_ppo_train_trajectories(wb_policy* p, int32_t n_traj, const int32_t* offsets_host, int32_t epochs, const float* states_host,
+                                  const float* actions_host, const float* old_logp_host, const float* rewards_host,
+                                  const int32_t* batch_index_host, float* values_host, float* returns_host, float* advantages_host,
+                                  float* losses_host, int32_t* skipped_host) {
+  WB_REQUIRE(p && states_host && actions_host && old_logp_host && rewards_host, "null argument");
+  int64_t steps = 0, n_index = 0;
+  if (int32_t rc = check_trajectories(p, n_traj, offsets_host, epochs, &steps, &n_index)) return rc;
+  WB_REQUIRE(batch_index_host || n_index == 0, "batch_index is null");
+  // every index must be a local row of its trajectory: checked before anything on the device changes
+  {
+    const int B = p->hp.batch_size;
+    const int32_t* ix = batch_index_host;
+    for (int32_t e = 0; e < n_traj; e++) {
+      const int T = offsets_host[e + 1] - offsets_host[e];
+      const int64_t cnt = (int64_t)epochs * (T / B) * B;
+      for (int64_t i = 0; i < cnt; i++, ix++)
+        if (*ix < 0 || *ix >= T) return fail(WB_ERR_INVALID, "batch_index of trajectory %d holds %d, outside its %d rows", e, *ix, T);
+    }
+  }
+  const size_t rows = (size_t)offsets_host[n_traj];
+  const size_t IN = (size_t)p->actor.input, ACT = (size_t)p->actor.output, N = (size_t)n_traj;
+  const size_t floats = rows * (IN + 2 * ACT + 4) + (size_t)n_index + 3 * N + 8;
+  if (int32_t rc = ensure_stage(p, floats)) return rc;
+  float* d_states = p->d_stage;
+  float* d_actions = d_states + rows * IN;
+  float* d_logp = d_actions + rows * ACT;
+  float* d_rewards = d_logp + rows * ACT;
+  float* d_values = d_rewards + rows;
+  float* d_returns = d_values + rows;
+  float* d_adv = d_returns + rows;
+  float* d_losses = d_adv + rows;
+  int32_t* d_skipped = reinterpret_cast<int32_t*>(d_losses + 2 * N);
+  int32_t* d_index = d_skipped + N;
+  if (rows) {
+    WB_CUDA(cudaMemcpyAsync(d_states, states_host, sizeof(float) * rows * IN, cudaMemcpyHostToDevice, p->stream));
+    WB_CUDA(cudaMemcpyAsync(d_actions, actions_host, sizeof(float) * rows * ACT, cudaMemcpyHostToDevice, p->stream));
+    WB_CUDA(cudaMemcpyAsync(d_logp, old_logp_host, sizeof(float) * rows * ACT, cudaMemcpyHostToDevice, p->stream));
+    WB_CUDA(cudaMemcpyAsync(d_rewards, rewards_host, sizeof(float) * rows, cudaMemcpyHostToDevice, p->stream));
+  }
+  if (n_index) WB_CUDA(cudaMemcpyAsync(d_index, batch_index_host, sizeof(int32_t) * n_index, cudaMemcpyHostToDevice, p->stream));
+  if (int32_t rc = wb_ppo_train_trajectories_dev(p, n_traj, offsets_host, epochs, d_states, d_actions, d_logp, d_rewards, d_index, d_values,
+                                                 d_returns, d_adv, d_losses, d_skipped))
+    return rc;
+  if (rows) {
+    if (values_host) WB_CUDA(cudaMemcpyAsync(values_host, d_values, sizeof(float) * rows, cudaMemcpyDeviceToHost, p->stream));
+    if (returns_host) WB_CUDA(cudaMemcpyAsync(returns_host, d_returns, sizeof(float) * rows, cudaMemcpyDeviceToHost, p->stream));
+    if (advantages_host) WB_CUDA(cudaMemcpyAsync(advantages_host, d_adv, sizeof(float) * rows, cudaMemcpyDeviceToHost, p->stream));
+  }
+  if (losses_host) WB_CUDA(cudaMemcpyAsync(losses_host, d_losses, sizeof(float) * 2 * N, cudaMemcpyDeviceToHost, p->stream));
+  if (skipped_host) WB_CUDA(cudaMemcpyAsync(skipped_host, d_skipped, sizeof(int32_t) * N, cudaMemcpyDeviceToHost, p->stream));
   WB_CUDA(cudaStreamSynchronize(p->stream));
   return WB_OK;
 }

@@ -102,12 +102,12 @@ struct GradConsts {
   float stdv, neg_log_std, log_sqrt_2pi, upper, lower, variance;
 };
 
-__global__ void __launch_bounds__(kMlpThreads, 1) ppo_fused_kernel(const MlpParams p, const GradConsts gc) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
-  const int tid = threadIdx.x;
+// ---- the 64-sample tile pipeline of PPOAgent.Train(Batch), shared by ppo_fused_kernel and ppo_episodes_kernel (one CTA of
+// kMlpThreads threads over MlpSmem; the callers stage the tile's states in S.X and own the weight-gradient accumulators and loss
+// sums, which stay in registers across every tile the CTA processes)
 
-  // ---- weights -> shared memory (padded rows)
+// weights p.params -> shared memory (padded rows)
+__device__ __forceinline__ void stage_weights(MlpSmem& S, const MlpParams& p, int tid) {
   for (int i = tid; i < kHid * kIn; i += kMlpThreads) {
     S.W1[i] = p.params[kOffW1 + i];
     S.Wc1[i] = p.params[kOffWc1 + i];
@@ -122,250 +122,216 @@ __global__ void __launch_bounds__(kMlpThreads, 1) ppo_fused_kernel(const MlpPara
   }
   if (tid < kAct) S.b3[tid] = p.params[kOffB3 + tid];
   if (tid == 0) S.bc2[0] = p.params[kOffBc2];
+}
 
-  const bool grad = p.mode == kModeGrad;
-  // weight-gradient accumulators, resident in registers across every tile this CTA processes
-  float accW2[4][4];
-#pragma unroll
-  for (int j = 0; j < 4; j++)
-#pragma unroll
-    for (int l = 0; l < 4; l++) accW2[j][l] = 0.0f;
-  float accW1[3] = {0.f, 0.f, 0.f}, accWc1[3] = {0.f, 0.f, 0.f};
-  float accW3 = 0.0f, accS = 0.0f, accT = 0.0f;
-  float lossV = 0.0f, lossA = 0.0f, skipped = 0.0f;
-
-  const int ntiles = (p.n + kTile - 1) / kTile;
-  for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const int s0 = tile * kTile;
-    const int nvalid = min(kTile, p.n - s0);
-    __syncthreads();  // previous tile fully consumed (also orders the weight staging on the first pass)
-    for (int i = tid; i < kTile * kIn; i += kMlpThreads) S.X[i] = (i < nvalid * kIn) ? p.states[(size_t)s0 * kIn + i] : 0.0f;
-    __syncthreads();
-
-    // ---- forward: actor L1, critic L1, actor L2 (NeuralNetwork.FeedForward, DenseLayer.FeedForward)
-    dense64_forward<kIn, kIn, kIn>(S.X, S.W1, S.b1, S.A1);
-    dense64_forward<kIn, kIn, kIn>(S.X, S.Wc1, S.bc1, S.C1);
-    __syncthreads();
-    dense64_forward<kHid, kPad, kPad>(S.A1, S.W2, S.b2, S.A2);
-    __syncthreads();
-    {  // actor L3 + TanH: thread = (sample, action dim); critic L2: threads 0..63
-      const int s = tid >> 2, k = tid & 3;
-      float sum = 0.0f;
+// S.X -> S.A1, S.C1, S.A2, S.MU, S.V; ends with a barrier
+__device__ __forceinline__ void tile_forward(MlpSmem& S, int tid) {
+  // ---- forward: actor L1, critic L1, actor L2 (NeuralNetwork.FeedForward, DenseLayer.FeedForward)
+  dense64_forward<kIn, kIn, kIn>(S.X, S.W1, S.b1, S.A1);
+  dense64_forward<kIn, kIn, kIn>(S.X, S.Wc1, S.bc1, S.C1);
+  __syncthreads();
+  dense64_forward<kHid, kPad, kPad>(S.A1, S.W2, S.b2, S.A2);
+  __syncthreads();
+  {  // actor L3 + TanH: thread = (sample, action dim); critic L2: threads 0..63
+    const int s = tid >> 2, k = tid & 3;
+    int i = 0;
+    float sum = 0.0f;
+#pragma unroll 4
+    for (; i < kHid; i += 4) {
+      const float4 a = ld4(S.A2 + s * kPad + i), w = ld4(S.W3 + k * kPad + i);
+      sum = fmaf(a.x, w.x, sum);
+      sum = fmaf(a.y, w.y, sum);
+      sum = fmaf(a.z, w.z, sum);
+      sum = fmaf(a.w, w.w, sum);
+    }
+    S.MU[s * kAct + k] = tanhf(sum + S.b3[k]);
+    if (tid < kTile) {
+      float v = 0.0f;
 #pragma unroll 4
       for (int i = 0; i < kHid; i += 4) {
-        const float4 a = ld4(S.A2 + s * kPad + i), w = ld4(S.W3 + k * kPad + i);
-        sum = fmaf(a.x, w.x, sum);
-        sum = fmaf(a.y, w.y, sum);
-        sum = fmaf(a.z, w.z, sum);
-        sum = fmaf(a.w, w.w, sum);
+        const float4 a = ld4(S.C1 + tid * kPad + i), w = ld4(S.Wc2 + i);
+        v = fmaf(a.x, w.x, v);
+        v = fmaf(a.y, w.y, v);
+        v = fmaf(a.z, w.z, v);
+        v = fmaf(a.w, w.w, v);
       }
-      S.MU[s * kAct + k] = tanhf(sum + S.b3[k]);
-      if (tid < kTile) {
-        float v = 0.0f;
-#pragma unroll 4
-        for (int i = 0; i < kHid; i += 4) {
-          const float4 a = ld4(S.C1 + tid * kPad + i), w = ld4(S.Wc2 + i);
-          v = fmaf(a.x, w.x, v);
-          v = fmaf(a.y, w.y, v);
-          v = fmaf(a.z, w.z, v);
-          v = fmaf(a.w, w.w, v);
-        }
-        S.V[tid] = v + S.bc2[0];
-      }
+      S.V[tid] = v + S.bc2[0];
     }
-    __syncthreads();
+  }
+  __syncthreads();
+}
 
-    if (!grad) {
-      const int s = tid >> 2, k = tid & 3;
-      const int gs = s0 + s;
-      if (s < nvalid) {
-        const float mu = S.MU[s * kAct + k];
-        if (p.mean) p.mean[(size_t)gs * kAct + k] = mu;
-        if (p.value && k == 0) p.value[gs] = S.V[s];
-        if (p.mode == kModeSample || p.mode == kModeSamplePhilox) {
-          float u1, u2;
-          if (p.mode == kModeSample) {
-            u1 = p.uniforms[((size_t)gs * kAct + k) * 2];
-            u2 = p.uniforms[((size_t)gs * kAct + k) * 2 + 1];
-          } else {
-            const uint4 r = philox4x32(make_uint4((uint32_t)gs, (uint32_t)k, (uint32_t)p.step, (uint32_t)(p.step >> 32)),
-                                       make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32)));
-            u1 = (float)(r.x >> 8) * (1.0f / 16777216.0f);  // [0,1) like (float)Random.NextDouble()
-            u2 = (float)(r.y >> 8) * (1.0f / 16777216.0f);
-          }
-          // NormalDistribution.BoxMullerTransform, NormalDistribution.cs:12-19
-          if (u1 == 0.0f) u1 = 1.0f;
-          const float z = sqrtf(-2.0f * logf(u1)) * sinf(2.0f * 3.14159274f * u2);
-          const float a = mu + (gc.stdv * z);
-          p.out_actions[(size_t)gs * kAct + k] = a;
-          p.out_logp[(size_t)gs * kAct + k] = log_prob(mu, gc.stdv, a, gc.neg_log_std, gc.log_sqrt_2pi);
-        }
-      }
-      continue;
-    }
-
-    // ---- per-sample clipped-surrogate gradient, PPOAgent.cs:232-326 (thread = sample)
-    if (tid < kTile) {
-      const int s = tid, gs = s0 + s;
-      float g[kAct] = {0.f, 0.f, 0.f, 0.f};
-      float gv = 0.0f;
-      if (s < nvalid) {
-        const float adv = p.advantages[gs];
-        bool skip = false;
-#pragma unroll
-        for (int k = 0; k < kAct; k++) {
-          const float mu = S.MU[s * kAct + k];
-          const float a = p.actions[(size_t)gs * kAct + k];
-          const float lp_old = p.old_logp[(size_t)gs * kAct + k];
-          const float lp = log_prob(mu, gc.stdv, a, gc.neg_log_std, gc.log_sqrt_2pi);
-          const float ratio = expf(lp - lp_old);
-          const float clipped = ratio >= gc.upper ? gc.upper : (ratio <= gc.lower ? gc.lower : ratio);  // Matrix.Clip
-          const float cra = clipped * adv, ra = ratio * adv;
-          const float partA = (ra <= cra ? 1.0f : 0.0f) * adv;                              // Matrix.LessThan
-          const float partB = (cra < ra ? 1.0f : 0.0f) * adv;                               // Matrix.LessThanNotEquals
-          const float partC = (ratio >= gc.lower && ratio <= gc.upper) ? 1.0f : 0.0f;       // Matrix.InRange
-          float dclip = (partA + partB * partC) * -1.0f;
-          const float pold = expf(lp_old);
-          if (pold == 0.0f) skip = true;  // HadamardDivision throws -> the sample is skipped (PPOAgent.cs:286-290)
-          dclip = dclip / pold;
-          const float prob = expf(lp);
-          const float dmean = prob * ((a - mu) / gc.variance);
-          g[k] = (dmean * dclip) / p.batch_size;
-        }
-        gv = (2.0f * (S.V[s] - p.returns[gs])) / p.batch_size;
-        if (skip) {
-#pragma unroll
-          for (int k = 0; k < kAct; k++) g[k] = 0.0f;
-          gv = 0.0f;
-          skipped += 1.0f;
-        } else {
-          lossV += gv;
-          lossA += (((g[0] + g[1]) + g[2]) + g[3]) / (float)kAct;  // Matrix.Average
-        }
-      }
-      // TanhLayer.FeedBack: g * (1 - tanh(z)^2), ActivationLayer.cs:18-21,69-72
+// row_of(s): the row of p's actions / old_logp / advantages / returns that sample s < nvalid of the tile is;
+// S.G3 / S.GV <- dL/dmu * tanh', dL/dV; ends with a barrier
+template <class RowOf>
+__device__ __forceinline__ void tile_surrogate(MlpSmem& S, const MlpParams p, const GradConsts gc, int nvalid, RowOf row_of, float& lossV,
+                                               float& lossA, float& skipped, int tid) {
+  // ---- per-sample clipped-surrogate gradient, PPOAgent.cs:232-326 (thread = sample)
+  if (tid < kTile) {
+    const int s = tid, gs = row_of(s);
+    float g[kAct] = {0.f, 0.f, 0.f, 0.f};
+    float gv = 0.0f;
+    if (s < nvalid) {
+      const float adv = p.advantages[gs];
+      bool skip = false;
 #pragma unroll
       for (int k = 0; k < kAct; k++) {
         const float mu = S.MU[s * kAct + k];
-        S.G3[s * kAct + k] = g[k] * (1.0f - (mu * mu));
+        const float a = p.actions[(size_t)gs * kAct + k];
+        const float lp_old = p.old_logp[(size_t)gs * kAct + k];
+        const float lp = log_prob(mu, gc.stdv, a, gc.neg_log_std, gc.log_sqrt_2pi);
+        const float ratio = expf(lp - lp_old);
+        const float clipped = ratio >= gc.upper ? gc.upper : (ratio <= gc.lower ? gc.lower : ratio);  // Matrix.Clip
+        const float cra = clipped * adv, ra = ratio * adv;
+        const float partA = (ra <= cra ? 1.0f : 0.0f) * adv;                              // Matrix.LessThan
+        const float partB = (cra < ra ? 1.0f : 0.0f) * adv;                               // Matrix.LessThanNotEquals
+        const float partC = (ratio >= gc.lower && ratio <= gc.upper) ? 1.0f : 0.0f;       // Matrix.InRange
+        float dclip = (partA + partB * partC) * -1.0f;
+        const float pold = expf(lp_old);
+        if (pold == 0.0f) skip = true;  // HadamardDivision throws -> the sample is skipped (PPOAgent.cs:286-290)
+        dclip = dclip / pold;
+        const float prob = expf(lp);
+        const float dmean = prob * ((a - mu) / gc.variance);
+        g[k] = (dmean * dclip) / p.batch_size;
       }
-      S.GV[s] = gv;
-    }
-    __syncthreads();
-
-    // ---- dL/dz2 = (W3^T g3) * leaky'(z2); dL/dzc1 = (Wc2^T gv) * leaky'(zc1)
-    {
-      const int s = tid >> 2, i0 = (tid & 3) * 16;
-      const float4 g3 = ld4(S.G3 + s * kAct);
-      const float gv = S.GV[s];
+      gv = (2.0f * (S.V[s] - p.returns[gs])) / p.batch_size;
+      if (skip) {
 #pragma unroll
-      for (int i = i0; i < i0 + 16; i++) {
-        float sum = 0.0f;
-        sum = fmaf(S.W3[0 * kPad + i], g3.x, sum);
-        sum = fmaf(S.W3[1 * kPad + i], g3.y, sum);
-        sum = fmaf(S.W3[2 * kPad + i], g3.z, sum);
-        sum = fmaf(S.W3[3 * kPad + i], g3.w, sum);
-        S.G2[s * kPad + i] = sum * leaky_grad_from_output(S.A2[s * kPad + i]);
-        S.Gc1[s * kPad + i] = (0.0f + S.Wc2[i] * gv) * leaky_grad_from_output(S.C1[s * kPad + i]);
+        for (int k = 0; k < kAct; k++) g[k] = 0.0f;
+        gv = 0.0f;
+        skipped += 1.0f;
+      } else {
+        lossV += gv;
+        lossA += (((g[0] + g[1]) + g[2]) + g[3]) / (float)kAct;  // Matrix.Average
       }
     }
-    __syncthreads();
-
-    // ---- dW3 += g3^T A2 ; dW2 += G2^T A1 ; dL/dz1 = (W2^T G2) * leaky'(z1)
-    {
-      const int k = tid >> 6, i = tid & 63;
-#pragma unroll 8
-      for (int s = 0; s < kTile; s++) accW3 = fmaf(S.G3[s * kAct + k], S.A2[s * kPad + i], accW3);
+    // TanhLayer.FeedBack: g * (1 - tanh(z)^2), ActivationLayer.cs:18-21,69-72
+#pragma unroll
+    for (int k = 0; k < kAct; k++) {
+      const float mu = S.MU[s * kAct + k];
+      S.G3[s * kAct + k] = g[k] * (1.0f - (mu * mu));
     }
-    {
-      const int og = tid >> 4, ig = tid & 15;
+    S.GV[s] = gv;
+  }
+  __syncthreads();
+}
+
+// backward pass of the tile into the accumulators; ends WITHOUT a barrier (the next tile's staging starts with one)
+__device__ __forceinline__ void tile_backward(MlpSmem& S, float (&accW2)[4][4], float (&accW1)[3], float (&accWc1)[3], float& accW3, float& accS,
+                                              float& accT, int tid) {
+  // ---- dL/dz2 = (W3^T g3) * leaky'(z2); dL/dzc1 = (Wc2^T gv) * leaky'(zc1)
+  {
+    const int s = tid >> 2, i0 = (tid & 3) * 16;
+    const float4 g3 = ld4(S.G3 + s * kAct);
+    const float gv = S.GV[s];
+#pragma unroll
+    for (int i = i0; i < i0 + 16; i++) {
+      float sum = 0.0f;
+      sum = fmaf(S.W3[0 * kPad + i], g3.x, sum);
+      sum = fmaf(S.W3[1 * kPad + i], g3.y, sum);
+      sum = fmaf(S.W3[2 * kPad + i], g3.z, sum);
+      sum = fmaf(S.W3[3 * kPad + i], g3.w, sum);
+      S.G2[s * kPad + i] = sum * leaky_grad_from_output(S.A2[s * kPad + i]);
+      S.Gc1[s * kPad + i] = (0.0f + S.Wc2[i] * gv) * leaky_grad_from_output(S.C1[s * kPad + i]);
+    }
+  }
+  __syncthreads();
+
+  // ---- dW3 += g3^T A2 ; dW2 += G2^T A1 ; dL/dz1 = (W2^T G2) * leaky'(z1)
+  {
+    const int k = tid >> 6, i = tid & 63;
+#pragma unroll 8
+    for (int s = 0; s < kTile; s++) accW3 = fmaf(S.G3[s * kAct + k], S.A2[s * kPad + i], accW3);
+  }
+  {
+    const int og = tid >> 4, ig = tid & 15;
 #pragma unroll 4
-      for (int s = 0; s < kTile; s++) {
-        const float4 g4 = ld4(S.G2 + s * kPad + og * 4);
-        const float4 a4 = ld4(S.A1 + s * kPad + ig * 4);
-        const float gg[4] = {g4.x, g4.y, g4.z, g4.w};
+    for (int s = 0; s < kTile; s++) {
+      const float4 g4 = ld4(S.G2 + s * kPad + og * 4);
+      const float4 a4 = ld4(S.A1 + s * kPad + ig * 4);
+      const float gg[4] = {g4.x, g4.y, g4.z, g4.w};
 #pragma unroll
-        for (int j = 0; j < 4; j++) {
-          accW2[j][0] = fmaf(gg[j], a4.x, accW2[j][0]);
-          accW2[j][1] = fmaf(gg[j], a4.y, accW2[j][1]);
-          accW2[j][2] = fmaf(gg[j], a4.z, accW2[j][2]);
-          accW2[j][3] = fmaf(gg[j], a4.w, accW2[j][3]);
-        }
-      }
-    }
-    {
-      const int ts = tid >> 4, ig = tid & 15;
-      float acc[4][4];
-#pragma unroll
-      for (int k = 0; k < 4; k++)
-#pragma unroll
-        for (int l = 0; l < 4; l++) acc[k][l] = 0.0f;
-#pragma unroll 2
-      for (int o = 0; o < kHid; o += 4) {
-        float4 g4[4], w4[4];
-#pragma unroll
-        for (int k = 0; k < 4; k++) g4[k] = ld4(S.G2 + (ts * 4 + k) * kPad + o);
-#pragma unroll
-        for (int q = 0; q < 4; q++) w4[q] = ld4(S.W2 + (o + q) * kPad + ig * 4);
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-          const float gq[4] = {g4[k].x, g4[k].y, g4[k].z, g4[k].w};
-#pragma unroll
-          for (int q = 0; q < 4; q++) {
-            acc[k][0] = fmaf(w4[q].x, gq[q], acc[k][0]);
-            acc[k][1] = fmaf(w4[q].y, gq[q], acc[k][1]);
-            acc[k][2] = fmaf(w4[q].z, gq[q], acc[k][2]);
-            acc[k][3] = fmaf(w4[q].w, gq[q], acc[k][3]);
-          }
-        }
-      }
-#pragma unroll
-      for (int k = 0; k < 4; k++) {
-        const int s = ts * 4 + k;
-        const float4 a = ld4(S.A1 + s * kPad + ig * 4);
-        float4 r;
-        r.x = acc[k][0] * leaky_grad_from_output(a.x);
-        r.y = acc[k][1] * leaky_grad_from_output(a.y);
-        r.z = acc[k][2] * leaky_grad_from_output(a.z);
-        r.w = acc[k][3] * leaky_grad_from_output(a.w);
-        *reinterpret_cast<float4*>(S.G1 + s * kPad + ig * 4) = r;
-      }
-    }
-    __syncthreads();
-
-    // ---- dW1 += G1^T X ; dWc1 += Gc1^T X ; biases and the critic head
-    {
-      const int o = tid >> 2, ib = (tid & 3) * 3;
-#pragma unroll 4
-      for (int s = 0; s < kTile; s++) {
-        const float ga = S.G1[s * kPad + o], gcr = S.Gc1[s * kPad + o];
-        const float x0 = S.X[s * kIn + ib], x1 = S.X[s * kIn + ib + 1], x2 = S.X[s * kIn + ib + 2];
-        accW1[0] = fmaf(ga, x0, accW1[0]);
-        accW1[1] = fmaf(ga, x1, accW1[1]);
-        accW1[2] = fmaf(ga, x2, accW1[2]);
-        accWc1[0] = fmaf(gcr, x0, accWc1[0]);
-        accWc1[1] = fmaf(gcr, x1, accWc1[1]);
-        accWc1[2] = fmaf(gcr, x2, accWc1[2]);
-      }
-    }
-    {
-      const int q = tid >> 6, o = tid & 63;  // q: 0 db1, 1 db2, 2 dbc1, 3 dWc2
-      const float* src = (q == 0) ? S.G1 : (q == 1) ? S.G2 : (q == 2) ? S.Gc1 : S.C1;
-#pragma unroll 8
-      for (int s = 0; s < kTile; s++) {
-        const float v = src[s * kPad + o];
-        accS = (q == 3) ? fmaf(S.GV[s], v, accS) : accS + v;
-      }
-      if (tid < kAct + 1) {
-#pragma unroll 8
-        for (int s = 0; s < kTile; s++) accT += (tid < kAct) ? S.G3[s * kAct + tid] : S.GV[s];
+      for (int j = 0; j < 4; j++) {
+        accW2[j][0] = fmaf(gg[j], a4.x, accW2[j][0]);
+        accW2[j][1] = fmaf(gg[j], a4.y, accW2[j][1]);
+        accW2[j][2] = fmaf(gg[j], a4.z, accW2[j][2]);
+        accW2[j][3] = fmaf(gg[j], a4.w, accW2[j][3]);
       }
     }
   }
+  {
+    const int ts = tid >> 4, ig = tid & 15;
+    float acc[4][4];
+#pragma unroll
+    for (int k = 0; k < 4; k++)
+#pragma unroll
+      for (int l = 0; l < 4; l++) acc[k][l] = 0.0f;
+#pragma unroll 2
+    for (int o = 0; o < kHid; o += 4) {
+      float4 g4[4], w4[4];
+#pragma unroll
+      for (int k = 0; k < 4; k++) g4[k] = ld4(S.G2 + (ts * 4 + k) * kPad + o);
+#pragma unroll
+      for (int q = 0; q < 4; q++) w4[q] = ld4(S.W2 + (o + q) * kPad + ig * 4);
+#pragma unroll
+      for (int k = 0; k < 4; k++) {
+        const float gq[4] = {g4[k].x, g4[k].y, g4[k].z, g4[k].w};
+#pragma unroll
+        for (int q = 0; q < 4; q++) {
+          acc[k][0] = fmaf(w4[q].x, gq[q], acc[k][0]);
+          acc[k][1] = fmaf(w4[q].y, gq[q], acc[k][1]);
+          acc[k][2] = fmaf(w4[q].z, gq[q], acc[k][2]);
+          acc[k][3] = fmaf(w4[q].w, gq[q], acc[k][3]);
+        }
+      }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+      const int s = ts * 4 + k;
+      const float4 a = ld4(S.A1 + s * kPad + ig * 4);
+      float4 r;
+      r.x = acc[k][0] * leaky_grad_from_output(a.x);
+      r.y = acc[k][1] * leaky_grad_from_output(a.y);
+      r.z = acc[k][2] * leaky_grad_from_output(a.z);
+      r.w = acc[k][3] * leaky_grad_from_output(a.w);
+      *reinterpret_cast<float4*>(S.G1 + s * kPad + ig * 4) = r;
+    }
+  }
+  __syncthreads();
 
-  if (!grad) return;
-  // ---- per-CTA partial gradient (flat parameter layout) + loss sums
-  float* out = p.partials + (size_t)blockIdx.x * kGradFloats;
+  // ---- dW1 += G1^T X ; dWc1 += Gc1^T X ; biases and the critic head
+  {
+    const int o = tid >> 2, ib = (tid & 3) * 3;
+#pragma unroll 4
+    for (int s = 0; s < kTile; s++) {
+      const float ga = S.G1[s * kPad + o], gcr = S.Gc1[s * kPad + o];
+      const float x0 = S.X[s * kIn + ib], x1 = S.X[s * kIn + ib + 1], x2 = S.X[s * kIn + ib + 2];
+      accW1[0] = fmaf(ga, x0, accW1[0]);
+      accW1[1] = fmaf(ga, x1, accW1[1]);
+      accW1[2] = fmaf(ga, x2, accW1[2]);
+      accWc1[0] = fmaf(gcr, x0, accWc1[0]);
+      accWc1[1] = fmaf(gcr, x1, accWc1[1]);
+      accWc1[2] = fmaf(gcr, x2, accWc1[2]);
+    }
+  }
+  {
+    const int q = tid >> 6, o = tid & 63;  // q: 0 db1, 1 db2, 2 dbc1, 3 dWc2
+    const float* src = (q == 0) ? S.G1 : (q == 1) ? S.G2 : (q == 2) ? S.Gc1 : S.C1;
+#pragma unroll 8
+    for (int s = 0; s < kTile; s++) {
+      const float v = src[s * kPad + o];
+      accS = (q == 3) ? fmaf(S.GV[s], v, accS) : accS + v;
+    }
+    if (tid < kAct + 1) {
+#pragma unroll 8
+      for (int s = 0; s < kTile; s++) accT += (tid < kAct) ? S.G3[s * kAct + tid] : S.GV[s];
+    }
+  }
+}
+
+// the CTA's gradient (flat parameter layout) + loss sums -> out[0 .. kTotalParams + 3); ends with a barrier
+__device__ __forceinline__ void write_grad(MlpSmem& S, const float (&accW2)[4][4], const float (&accW1)[3], const float (&accWc1)[3], float accW3,
+                                           float accS, float accT, float lossV, float lossA, float skipped, float* out, int tid) {
   {
     const int og = tid >> 4, ig = tid & 15;
 #pragma unroll
@@ -404,6 +370,69 @@ __global__ void __launch_bounds__(kMlpThreads, 1) ppo_fused_kernel(const MlpPara
   }
 }
 
+__global__ void __launch_bounds__(kMlpThreads, 1) ppo_fused_kernel(const MlpParams p, const GradConsts gc) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
+  const int tid = threadIdx.x;
+
+  stage_weights(S, p, tid);
+  const bool grad = p.mode == kModeGrad;
+  // weight-gradient accumulators, resident in registers across every tile this CTA processes
+  float accW2[4][4];
+#pragma unroll
+  for (int j = 0; j < 4; j++)
+#pragma unroll
+    for (int l = 0; l < 4; l++) accW2[j][l] = 0.0f;
+  float accW1[3] = {0.f, 0.f, 0.f}, accWc1[3] = {0.f, 0.f, 0.f};
+  float accW3 = 0.0f, accS = 0.0f, accT = 0.0f;
+  float lossV = 0.0f, lossA = 0.0f, skipped = 0.0f;
+
+  const int ntiles = (p.n + kTile - 1) / kTile;
+  for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+    const int s0 = tile * kTile;
+    const int nvalid = min(kTile, p.n - s0);
+    __syncthreads();  // previous tile fully consumed (also orders the weight staging on the first pass)
+    for (int i = tid; i < kTile * kIn; i += kMlpThreads) S.X[i] = (i < nvalid * kIn) ? p.states[(size_t)s0 * kIn + i] : 0.0f;
+    __syncthreads();
+    tile_forward(S, tid);
+    if (!grad) {
+      const int s = tid >> 2, k = tid & 3;
+      const int gs = s0 + s;
+      if (s < nvalid) {
+        const float mu = S.MU[s * kAct + k];
+        if (p.mean) p.mean[(size_t)gs * kAct + k] = mu;
+        if (p.value && k == 0) p.value[gs] = S.V[s];
+        if (p.mode == kModeSample || p.mode == kModeSamplePhilox) {
+          float u1, u2;
+          if (p.mode == kModeSample) {
+            u1 = p.uniforms[((size_t)gs * kAct + k) * 2];
+            u2 = p.uniforms[((size_t)gs * kAct + k) * 2 + 1];
+          } else {
+            const uint4 r = philox4x32(make_uint4((uint32_t)gs, (uint32_t)k, (uint32_t)p.step, (uint32_t)(p.step >> 32)),
+                                       make_uint2((uint32_t)p.seed, (uint32_t)(p.seed >> 32)));
+            u1 = (float)(r.x >> 8) * (1.0f / 16777216.0f);  // [0,1) like (float)Random.NextDouble()
+            u2 = (float)(r.y >> 8) * (1.0f / 16777216.0f);
+          }
+          // NormalDistribution.BoxMullerTransform, NormalDistribution.cs:12-19
+          if (u1 == 0.0f) u1 = 1.0f;
+          const float z = sqrtf(-2.0f * logf(u1)) * sinf(2.0f * 3.14159274f * u2);
+          const float a = mu + (gc.stdv * z);
+          p.out_actions[(size_t)gs * kAct + k] = a;
+          p.out_logp[(size_t)gs * kAct + k] = log_prob(mu, gc.stdv, a, gc.neg_log_std, gc.log_sqrt_2pi);
+        }
+      }
+      continue;
+    }
+
+    tile_surrogate(S, p, gc, nvalid, [&](int s) { return s0 + s; }, lossV, lossA, skipped, tid);
+    tile_backward(S, accW2, accW1, accWc1, accW3, accS, accT, tid);
+  }
+
+  if (!grad) return;
+  // per-CTA partial gradient + loss sums
+  write_grad(S, accW2, accW1, accWc1, accW3, accS, accT, lossV, lossA, skipped, p.partials + (size_t)blockIdx.x * kGradFloats, tid);
+}
+
 // grads[i] = sum over CTAs (fixed order) -- this is also NeuralNetwork.Zero(): the buffer is overwritten
 __global__ void reduce_partials_kernel(const float* __restrict__ partials, int nparts, float* __restrict__ grads) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -421,9 +450,9 @@ __global__ void adam_kernel(const AdamParams a) {
 
 // PPOAgent.MonteCarloReturn/MonteCarloAdvantages (:475-498), GeneralizedAdvantageEstimate (:414-444, whose nextGae is
 // never updated in the reference), Normalize (:461-472).  One trajectory: an inherently sequential fp32 recurrence.
-__global__ void returns_kernel(const float* rewards, const float* values, int n, float gamma, float lambda, int use_gae,
-                               int normalize, float norm_eps, float* returns, float* advantages) {
-  if (blockIdx.x != 0 || threadIdx.x != 0) return;
+__device__ __forceinline__ void trajectory_returns(const float* __restrict__ rewards, const float* __restrict__ values, int n, float gamma,
+                                                   float lambda, int use_gae, int normalize, float norm_eps, float* __restrict__ returns,
+                                                   float* __restrict__ advantages) {
   if (use_gae) {
     const float next_gae = 0.0f;
     float next_value = 0.0f;
@@ -455,6 +484,102 @@ __global__ void returns_kernel(const float* rewards, const float* values, int n,
     const float sd = (float)sqrt(ss / (double)n);
     const float div = __fadd_rn(sd, norm_eps);
     for (int i = 0; i < n; i++) advantages[i] = __fdiv_rn(__fsub_rn(advantages[i], mean), div);
+  }
+}
+__global__ void returns_kernel(const float* rewards, const float* values, int n, float gamma, float lambda, int use_gae,
+                               int normalize, float norm_eps, float* returns, float* advantages) {
+  if (blockIdx.x != 0 || threadIdx.x != 0) return;
+  trajectory_returns(rewards, values, n, gamma, lambda, use_gae, normalize, norm_eps, returns, advantages);
+}
+
+// PPOAgent.Train(Trajectory) (PPOAgent.cs:147-172) for a list of trajectories, in list order, as ONE persistent CTA: the Adam
+// steps form a serial chain (each mini-batch is trained with the weights the previous one left), so one SM without host round
+// trips is the shape of the work.  Per trajectory: critic forward over its rows (tile_forward, as the forward mode of
+// ppo_fused_kernel), returns / advantages (trajectory_returns, as returns_kernel), then epochs x floor(T / B) mini-batches:
+// the indexed rows are gathered into the tile, ceil(B / 64) tiles accumulate in registers (the tile pipeline of
+// ppo_fused_kernel), the gradient goes to the gradient buffer, and DenseLayer.Adam runs over every parameter with that step's
+// bias corrections from the host's table before the shared-memory weights are refreshed.
+struct __align__(16) EpisodeSmem {
+  MlpSmem m;
+  int32_t rows[kTile];  // pool row of every sample of the current mini-batch tile
+};
+
+__global__ void __launch_bounds__(kMlpThreads, 1) ppo_episodes_kernel(const EpisodeParams e, const MlpParams p, const GradConsts gc) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  EpisodeSmem& E = *reinterpret_cast<EpisodeSmem*>(smem_raw);
+  MlpSmem& S = E.m;
+  const int tid = threadIdx.x;
+  const int B = e.batch;
+  stage_weights(S, p, tid);
+  int step = 0;
+  const int32_t* index = e.batch_index;
+  for (int t = 0; t < e.n_traj; t++) {
+    const int r0 = e.offsets[t], T = e.offsets[t + 1] - r0;
+    // ---- CalculateValues (PPOAgent.cs:175-189): the critic over the trajectory's rows with the current weights
+    for (int s0 = 0; s0 < T; s0 += kTile) {
+      const int nvalid = min(kTile, T - s0);
+      __syncthreads();
+      for (int i = tid; i < kTile * kIn; i += kMlpThreads) S.X[i] = (i < nvalid * kIn) ? p.states[(size_t)(r0 + s0) * kIn + i] : 0.0f;
+      __syncthreads();
+      tile_forward(S, tid);
+      if (tid < nvalid) e.values[r0 + s0 + tid] = S.V[tid];
+    }
+    __syncthreads();
+    if (tid == 0 && T > 0)
+      trajectory_returns(e.rewards + r0, e.values + r0, T, e.gamma, e.lambda, e.use_gae, e.normalize, e.norm_eps, e.returns + r0,
+                         e.advantages + r0);
+    __syncthreads();
+    // ---- epochs x floor(T / B) mini-batches, each Train(Batch) + NeuralNetwork.Optimise
+    const int nb = e.epochs * (T / B);
+    float skipped_total = 0.0f;
+    for (int b = 0; b < nb; b++, step++, index += B) {
+      float accW2[4][4];
+#pragma unroll
+      for (int j = 0; j < 4; j++)
+#pragma unroll
+        for (int l = 0; l < 4; l++) accW2[j][l] = 0.0f;
+      float accW1[3] = {0.f, 0.f, 0.f}, accWc1[3] = {0.f, 0.f, 0.f};
+      float accW3 = 0.0f, accS = 0.0f, accT = 0.0f;
+      float lossV = 0.0f, lossA = 0.0f, skipped = 0.0f;
+      for (int b0 = 0; b0 < B; b0 += kTile) {
+        const int nvalid = min(kTile, B - b0);
+        __syncthreads();
+        if (tid < kTile) E.rows[tid] = r0 + (tid < nvalid ? index[b0 + tid] : 0);
+        __syncthreads();
+        for (int i = tid; i < kTile * kIn; i += kMlpThreads) {
+          const int s = i / kIn;
+          S.X[i] = (s < nvalid) ? p.states[(size_t)E.rows[s] * kIn + (i - s * kIn)] : 0.0f;
+        }
+        __syncthreads();
+        tile_forward(S, tid);
+        tile_surrogate(S, p, gc, nvalid, [&](int s) { return E.rows[s]; }, lossV, lossA, skipped, tid);
+        tile_backward(S, accW2, accW1, accWc1, accW3, accS, accT, tid);
+      }
+      __syncthreads();
+      write_grad(S, accW2, accW1, accWc1, accW3, accS, accT, lossV, lossA, skipped, e.grads, tid);
+      // the per-mini-batch path reduces ONE partial (0 + partial + 0 ...): the same values, with -0 stored as +0
+      AdamParams a = e.adam;
+#pragma unroll
+      for (int l = 0; l < 5; l++) {
+        a.corr1[l] = e.corr[step * 10 + l];
+        a.corr2[l] = e.corr[step * 10 + 5 + l];
+      }
+      for (int i = tid; i < kTotalParams + 3; i += kMlpThreads) {
+        const float g = __fadd_rn(e.grads[i], 0.0f);
+        e.grads[i] = g;
+        if (i < kTotalParams) adam_update(a, i, g);
+      }
+      __syncthreads();
+      if (tid == 0) skipped_total += e.grads[kGradSkipped];
+      stage_weights(S, p, tid);  // (ordered before the next use by the next tile's first barrier)
+    }
+    if (tid == 0) {
+      if (e.losses) {
+        e.losses[2 * t] = nb > 0 ? e.grads[kGradLossV] : 0.0f;
+        e.losses[2 * t + 1] = nb > 0 ? e.grads[kGradLossA] : 0.0f;
+      }
+      if (e.skipped) e.skipped[t] = (int32_t)skipped_total;
+    }
   }
 }
 
@@ -564,6 +689,17 @@ __global__ void gather_minibatch_kernel(const int32_t* __restrict__ index, int B
 }
 
 // ---------------------------------------------------------------- host side
+static GradConsts grad_consts(float log_std, float epsilon) {
+  GradConsts gc;
+  gc.stdv = expf(log_std);                         // PPOAgent.GetStandardDeviations, PPOAgent.cs:367-378
+  gc.neg_log_std = -logf(gc.stdv);                 // NormalDistribution.cs:31
+  gc.log_sqrt_2pi = logf(sqrtf(2.0f * 3.14159274f));
+  gc.upper = 1.0f + epsilon;
+  gc.lower = 1.0f - epsilon;
+  gc.variance = gc.stdv * gc.stdv;
+  return gc;
+}
+
 cudaError_t launch_segment_returns(const float* rewards, const float* values, const uint8_t* dones, const float* last_values, int n_envs,
                                    int T, float gamma, float lambda, int use_gae, float* returns, float* advantages, cudaStream_t stream) {
   segment_returns_kernel<<<(n_envs + 127) / 128, 128, 0, stream>>>(rewards, values, dones, last_values, n_envs, T, gamma, lambda, use_gae,
@@ -603,14 +739,7 @@ cudaError_t launch_mlp(const MlpParams& p, int grid, cudaStream_t stream) {
     if (e != cudaSuccess) return e;
     if (dev >= 0 && dev < 64) configured[dev] = true;
   }
-  GradConsts gc;
-  gc.stdv = expf(p.log_std);                       // PPOAgent.GetStandardDeviations, PPOAgent.cs:367-378
-  gc.neg_log_std = -logf(gc.stdv);                 // NormalDistribution.cs:31
-  gc.log_sqrt_2pi = logf(sqrtf(2.0f * 3.14159274f));
-  gc.upper = 1.0f + p.epsilon;
-  gc.lower = 1.0f - p.epsilon;
-  gc.variance = gc.stdv * gc.stdv;
-  ppo_fused_kernel<<<grid, kMlpThreads, sizeof(MlpSmem), stream>>>(p, gc);
+  ppo_fused_kernel<<<grid, kMlpThreads, sizeof(MlpSmem), stream>>>(p, grad_consts(p.log_std, p.epsilon));
   return cudaGetLastError();
 }
 
@@ -727,6 +856,60 @@ cudaError_t launch_reduce_partials(const float* partials, int nparts, float* gra
 
 cudaError_t launch_adam(const AdamParams& p, cudaStream_t stream) {
   adam_kernel<<<(kTotalParams + 127) / 128, 128, 0, stream>>>(p);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_episodes(const EpisodeParams& e, const MlpParams& p, cudaStream_t stream) {
+  static bool configured[64] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 0 || dev >= 64 || !configured[dev]) {
+    cudaError_t err = cudaFuncSetAttribute(ppo_episodes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(EpisodeSmem));
+    if (err != cudaSuccess) return err;
+    if (dev >= 0 && dev < 64) configured[dev] = true;
+  }
+  ppo_episodes_kernel<<<1, kMlpThreads, sizeof(EpisodeSmem), stream>>>(e, p, grad_consts(p.log_std, p.epsilon));
+  return cudaGetLastError();
+}
+
+// rows row_base + index[b] of the row arrays -> a contiguous mini-batch, any state / action width (one thread per (sample, float))
+__global__ void gather_rows_kernel(const int32_t* __restrict__ index, int B, int row_base, int sdim, int adim, const float* __restrict__ states,
+                                   const float* __restrict__ actions, const float* __restrict__ logp, const float* __restrict__ adv,
+                                   const float* __restrict__ ret, float* __restrict__ o_states, float* __restrict__ o_actions,
+                                   float* __restrict__ o_logp, float* __restrict__ o_adv, float* __restrict__ o_ret) {
+  const int per = sdim + 2 * adim + 2;
+  const long gid = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int b = (int)(gid / per), f = (int)(gid % per);
+  if (b >= B) return;
+  const size_t src = (size_t)row_base + index[b];
+  if (f < sdim) o_states[(size_t)b * sdim + f] = states[src * sdim + f];
+  else if (f < sdim + adim) o_actions[(size_t)b * adim + (f - sdim)] = actions[src * adim + (f - sdim)];
+  else if (f < sdim + 2 * adim) o_logp[(size_t)b * adim + (f - sdim - adim)] = logp[src * adim + (f - sdim - adim)];
+  else if (f == sdim + 2 * adim) o_adv[b] = adv[src];
+  else o_ret[b] = ret[src];
+}
+
+// losses[2] <- the gradient buffer's loss sums, skipped += its skipped count (one trajectory's mini-batches, in order)
+__global__ void episode_losses_kernel(const float* __restrict__ tail, float* losses, int32_t* skipped) {
+  if (threadIdx.x != 0) return;
+  if (losses) {
+    losses[0] = tail[0];
+    losses[1] = tail[1];
+  }
+  if (skipped) *skipped += (int32_t)tail[2];
+}
+
+cudaError_t launch_gather_rows(const int32_t* index, int B, int row_base, int sdim, int adim, const float* states, const float* actions,
+                               const float* logp, const float* adv, const float* ret, float* o_states, float* o_actions, float* o_logp,
+                               float* o_adv, float* o_ret, cudaStream_t stream) {
+  const long total = (long)B * (sdim + 2 * adim + 2);
+  gather_rows_kernel<<<(unsigned)((total + 255) / 256), 256, 0, stream>>>(index, B, row_base, sdim, adim, states, actions, logp, adv, ret,
+                                                                          o_states, o_actions, o_logp, o_adv, o_ret);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_episode_losses(const float* grads_tail, float* losses, int32_t* skipped, cudaStream_t stream) {
+  episode_losses_kernel<<<1, 32, 0, stream>>>(grads_tail, losses, skipped);
   return cudaGetLastError();
 }
 

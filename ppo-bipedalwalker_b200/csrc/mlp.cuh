@@ -86,6 +86,31 @@ __device__ __forceinline__ void adam_update(const AdamParams& a, int i, float g)
 }
 #endif
 
+// PPOAgent.Train(Trajectory) over a list of trajectories in one launch (ppo_episodes_kernel, default networks).  The row arrays
+// (states / actions / old_logp of the MlpParams, rewards, values, returns, advantages) hold the trajectories back to back.
+struct EpisodeParams {
+  const float* rewards;
+  float* values;
+  float* returns;
+  float* advantages;
+  const int32_t* offsets;      // [n_traj + 1] (device copy of the host's offsets)
+  const int32_t* batch_index;  // per mini-batch B local row numbers, in call order
+  const float* corr;           // [Adam steps][10]: corr1 of the 5 dense layers, then corr2
+  float* grads;                // the gradient buffer (last mini-batch's gradient, loss sums, skipped)
+  float* losses;               // [n_traj][2] or null
+  int32_t* skipped;            // [n_traj] or null
+  AdamParams adam;             // params / m / v and the hyper-parameters (the corrections come from the table)
+  int32_t n_traj, epochs, batch;
+  int32_t use_gae, normalize;
+  float gamma, lambda, norm_eps;
+};
+cudaError_t launch_episodes(const EpisodeParams& e, const MlpParams& p, cudaStream_t stream);
+cudaError_t launch_gather_rows(const int32_t* index, int B, int row_base, int sdim, int adim, const float* states, const float* actions,
+                               const float* logp, const float* adv, const float* ret, float* o_states, float* o_actions, float* o_logp,
+                               float* o_adv, float* o_ret, cudaStream_t stream);
+// losses[2] <- grads_tail[0..1], *skipped += grads_tail[2] (either may be null)
+cudaError_t launch_episode_losses(const float* grads_tail, float* losses, int32_t* skipped, cudaStream_t stream);
+
 int mlp_grid_for(int n, int sm_count);
 cudaError_t launch_mlp(const MlpParams& p, int grid, cudaStream_t stream);
 cudaError_t launch_reduce_partials(const float* partials, int nparts, float* grads, cudaStream_t stream);

@@ -327,6 +327,45 @@ class PPOAgent:
                 vloss, aloss, _ = self.TrainBatch(S[idx], Acts[idx], LP[idx], Adv[idx], G[idx])
         return vloss, aloss
 
+    def TrainTrajectories(self, trajectories, epochs: int = 5):
+        """PPOAgent.Train(Trajectory) for every trajectory of the list, in list order, as ONE call (wb_ppo_train_trajectories: one
+        launch on the default networks). The mini-batch permutations are drawn from self.rng in the same order and number as
+        `for t in trajectories: self.Train(t, epochs)` draws them, so an agent in the same RNG state trains on the same mini-batches.
+        Fills every trajectory's Values / Returns / Advantages. Returns [(criticLoss, actorLoss)] per trajectory."""
+        trajectories = list(trajectories)
+        if not trajectories:
+            return []
+        B = self.hp.batch_size
+        lengths = [len(t.States) for t in trajectories]
+        offsets = np.zeros(len(trajectories) + 1, np.int32)
+        offsets[1:] = np.cumsum(lengths)
+        blocks = []
+        for T in lengths:
+            if T == 0:  # Train returns before drawing
+                continue
+            for _ in range(epochs):
+                perm = self.rng.permutation(T)
+                blocks.extend(perm[j * B:(j + 1) * B] for j in range(T // B))
+        index = np.ascontiguousarray(np.concatenate(blocks) if blocks else np.zeros(0), np.int32)
+        rows = int(offsets[-1])
+
+        def rows_of(attr, width):
+            parts = [np.asarray(getattr(t, attr), np.float32).reshape(-1, width) for t in trajectories if len(t.States)]
+            return np.ascontiguousarray(np.concatenate(parts) if parts else np.zeros((0, width), np.float32))
+        S = rows_of("States", self.stateSize)
+        Acts = rows_of("Actions", self.actionSize)
+        LP = rows_of("LogProbabilities", self.actionSize)
+        R = rows_of("Rewards", 1).reshape(rows)
+        V, G, A = (np.empty(rows, np.float32) for _ in range(3))
+        losses = np.zeros((len(trajectories), 2), np.float32)
+        skipped = np.zeros(len(trajectories), np.int32)
+        check(lib().wb_ppo_train_trajectories(self._h, len(trajectories), ptr(offsets), epochs, ptr(S), ptr(Acts), ptr(LP), ptr(R),
+                                              ptr(index), ptr(V), ptr(G), ptr(A), ptr(losses), ptr(skipped)))
+        for t, o, T in zip(trajectories, offsets, lengths):
+            if T:
+                t.Values, t.Returns, t.Advantages = list(V[o:o + T]), list(G[o:o + T]), list(A[o:o + T])
+        return [(float(c), float(a)) for c, a in losses]
+
     def Save(self):  # PPOAgent.Save (PPOAgent.cs:192-213) -> the two .weights files' lines
         return self.critic.Save(), self.actor.Save()
 
