@@ -376,6 +376,68 @@ int32_t wb_adam_step(wb_policy* p);
 int32_t wb_policy_grad_buffer(wb_policy* p, void** dev_ptr_out, int32_t* n_floats_out);
 int32_t wb_policy_launch_count(const wb_policy* p, int64_t* count_out);
 
+/* ---- populations: one PPO brain per walker ----
+ * In the reference every walker owns its agent (new Walker() builds its own PPOAgent(12, 4), Walker.cs:25-34) and trains it on each
+ * of its own episodes as soon as the episode ends (Environment.cs:91,157-164 -> PPOAgent.Train(Trajectory), PPOAgent.cs:147-172).
+ * A population holds P such agents with the reference's default networks (Hyperparameters.cs:91-92; 6 149 parameters): each has
+ * its own weights, Adam m / v, per-dense-layer step counters and wb_hyperparams (alpha, beta1, beta2, Adam epsilon, gamma, lambda,
+ * clip epsilon, log_std, use_gae, normalize_advantages, batch_size).  Agent a behaves exactly as one wb_policy on kernel variant 1
+ * with the same weights and hyper-parameters: acting and training give the same bits.  Agents that a call does not name are not
+ * touched.  Weights start at zero (load them with wb_population_set_weights).  The longest episode trained is 1 024 steps
+ * (WB_ERR_UNSUPPORTED beyond). */
+typedef struct wb_population wb_population;
+/* new PPOAgent(12, 4) x n_agents (PPOAgent.cs:23-37); hp = [n_agents] hyper-parameters or NULL (the defaults for every agent).
+ * n_agents < 1 or a batch_size < 1: WB_ERR_INVALID */
+int32_t wb_population_create(int32_t n_agents, const wb_hyperparams* hp, wb_population** out);
+int32_t wb_population_destroy(wb_population* pop);
+int32_t wb_population_set_stream(wb_population* pop, void* cuda_stream);
+int32_t wb_population_sync(wb_population* pop);
+/* number of kernel launches this handle has issued */
+int32_t wb_population_launch_count(const wb_population* pop, int64_t* count_out);
+/* agent a's flat parameters [6149] = actor | critic, each in the DenseLayer.Save order (DenseLayer.cs:73-79) */
+int32_t wb_population_set_weights(wb_population* pop, int32_t agent, const float* flat_host);
+int32_t wb_population_get_weights(wb_population* pop, int32_t agent, float* flat_host);
+/* agent a's gradient buffer [6149] (the last mini-batch it trained, as wb_policy_get_grads) */
+int32_t wb_population_get_grads(wb_population* pop, int32_t agent, float* flat_host);
+/* agent a's Adam moments m / v [6149] and the step counters [5] of its dense layers (actor L1-L3, critic L1-L2; DenseLayer.cs:15-20) */
+int32_t wb_population_get_adam(wb_population* pop, int32_t agent, float* m_host, float* v_host, int32_t* steps_host);
+/* PPOAgent.SampleActions (PPOAgent.cs:381-398) for n == P walkers, walker w with agent w, with the two System.Random uniforms of
+ * each Box-Muller draw injected (NormalDistribution.cs:12-32): states [n][12], uniforms [n][4][2] -> actions, logp [n][4], mean
+ * [n][4] or NULL.  Row w equals wb_policy_sample of agent w. */
+int32_t wb_population_sample(wb_population* pop, int32_t n, const float* states_host, const float* uniforms_host, float* actions_host,
+                             float* logp_host, float* mean_host);
+/* the same from the Philox stream (seed, step) of wb_policy_act_dev (counter (walker, action dim, step)), enqueue only; mean_dev
+ * and the critic's value estimate value_dev [n] (PPOAgent.GetValueEstimate, PPOAgent.cs:350-364) may be NULL.  One launch. */
+int32_t wb_population_act_dev(wb_population* pop, int32_t n, const float* states_dev, uint64_t seed, uint64_t step, float* actions_dev,
+                              float* logp_dev, float* mean_dev, float* value_dev);
+/* PPOAgent.Train(Trajectory) (PPOAgent.cs:147-172) for n_traj finished episodes of several agents in ONE launch: trajectory e
+ * belongs to agent agent_host[e] and is rows [offsets[e], offsets[e+1]) of the packed arrays, as in wb_ppo_train_trajectories.
+ * Every agent trains its own trajectories in list order, so its final state equals wb_ppo_train_trajectories of its sub-list.
+ * batch_index: per trajectory, in list order, epochs x floor(T_e / B_a) x B_a local row numbers (PPOAgent.CreateBatches,
+ * :501-540, drawn by the caller), B_a = that agent's batch_size.  values / returns / advantages [rows], losses [n_traj][2] and
+ * skipped [n_traj] as in wb_ppo_train_trajectories; each may be NULL.  Bad offsets, an agent out of range, epochs < 0,
+ * n_traj < 1 or an index outside its trajectory: WB_ERR_INVALID before anything on the device changes. */
+int32_t wb_population_train_trajectories(wb_population* pop, int32_t n_traj, const int32_t* agent_host, const int32_t* offsets_host,
+                                         int32_t epochs, const float* states_host, const float* actions_host, const float* logp_host,
+                                         const float* rewards_host, const int32_t* batch_index_host, float* values_host,
+                                         float* returns_host, float* advantages_host, float* losses_host, int32_t* skipped_host);
+/* The device form for lockstep walkers (Environment.Update -> TrainNetworks -> Reset, Environment.cs:64-92,157-173): the
+ * rollout arrays are a time-major ring of ring_rows rows x columns (states [R][C][12], actions / logp [R][C][4], rewards /
+ * values / returns / advantages [R][C]).  items_host [n_items][4] = (agent, column, t0, length): the episode's step i is row
+ * ((t0 + i) mod ring_rows) * columns + column.  Every agent trains its items in list order, one CTA per agent with work.
+ * batch_index_dev: caller-drawn indices in the layout of wb_population_train_trajectories, or NULL: the kernel draws them --
+ * epoch k of an episode orders the local rows i < length by (key, i) with key = Philox-4x32-10(counter (i, k, episode, agent),
+ * key (seed & 0xffffffff, seed >> 32)).x, where `episode` is the number of this agent's episodes (items, in both train entries)
+ * trained before this one, and takes floor(length / B) blocks of B (the remainder is dropped).  The episode's values, returns and
+ * advantages are written to its rows of values_dev / returns_dev / advantages_dev (required); losses_dev [n_items][2] and
+ * skipped_dev [n_items] may be NULL.  Host arguments are checked before anything changes (WB_ERR_INVALID): n_items < 1, an
+ * agent or column out of range, length < 0 or > ring_rows, t0 outside the ring, epochs < 0.  Device indices are not
+ * range-checked.  Enqueue only: one launch. */
+int32_t wb_population_train_dev(wb_population* pop, int32_t n_items, const int32_t* items_host, int32_t ring_rows, int32_t columns,
+                                int32_t epochs, uint64_t seed, const float* states_dev, const float* actions_dev, const float* logp_dev,
+                                const float* rewards_dev, const int32_t* batch_index_dev, float* values_dev, float* returns_dev,
+                                float* advantages_dev, float* losses_dev, int32_t* skipped_dev);
+
 /* test hook for the tcgen05 building block: one CTA computes D[M x N] = A[M x K] * B[N x K]^T on the tensor cores
  * (kind::tf32; passes = 1 plain TF32, 3 = 3xTF32 split).  a/b_mn_major choose how the operand tile is read (K-major / MN-major). */
 int32_t wb_debug_tc_gemm(int32_t M, int32_t N, int32_t K, int32_t a_mn_major, int32_t b_mn_major, int32_t passes, const float* A_host,

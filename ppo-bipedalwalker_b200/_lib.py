@@ -151,6 +151,19 @@ def lib() -> C.CDLL:
         "wb_policy_launch_count": (C.c_int32, [vp, i64p]),
         "wb_returns_advantages": (C.c_int32, [vp, C.c_int32, vp, vp, vp, vp]),
         "wb_debug_tc_gemm": (C.c_int32, [C.c_int32] * 6 + [vp, vp, vp]),
+        "wb_population_create": (C.c_int32, [C.c_int32, hpp, C.POINTER(vp)]),
+        "wb_population_destroy": (C.c_int32, [vp]),
+        "wb_population_set_stream": (C.c_int32, [vp, vp]),
+        "wb_population_sync": (C.c_int32, [vp]),
+        "wb_population_launch_count": (C.c_int32, [vp, i64p]),
+        "wb_population_set_weights": (C.c_int32, [vp, C.c_int32, vp]),
+        "wb_population_get_weights": (C.c_int32, [vp, C.c_int32, vp]),
+        "wb_population_get_grads": (C.c_int32, [vp, C.c_int32, vp]),
+        "wb_population_get_adam": (C.c_int32, [vp, C.c_int32, vp, vp, vp]),
+        "wb_population_sample": (C.c_int32, [vp, C.c_int32, vp, vp, vp, vp, vp]),
+        "wb_population_act_dev": (C.c_int32, [vp, C.c_int32, vp, C.c_uint64, C.c_uint64, vp, vp, vp, vp]),
+        "wb_population_train_trajectories": (C.c_int32, [vp, C.c_int32, vp, vp, C.c_int32] + [vp] * 10),
+        "wb_population_train_dev": (C.c_int32, [vp, C.c_int32, vp, C.c_int32, C.c_int32, C.c_int32, C.c_uint64] + [vp] * 10),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)  # AttributeError here = the library does not export what the header declares

@@ -6,7 +6,9 @@
 // receive reward, train on terminal -- for ALL walkers per call: one wb_policy_sample, one fused wb_env_step (which also resets
 // the walkers that terminated and returns their initial observation, Environment.cs:167-180), N trajectories, and
 // PPOAgent.Train on the trajectory of every walker whose episode just ended (one shared brain, like N copies of the
-// reference training the same weights files).
+// reference training the same weights files).  With brainPerWalker every walker owns its agent, as in the reference (Walker.cs:25-34):
+// the actions come from one wb_population_sample and every walker whose episode ended in the step trains its own agent, all in
+// one wb_population_train_trajectories call.
 using System;
 using System.Collections.Generic;
 using System.Linq;
@@ -25,7 +27,8 @@ public class GpuEnvironment : IDisposable
     private readonly IntPtr _env;
     private readonly int _n;
     private readonly Renderer _renderer;
-    private readonly GpuPPOAgent _brain;
+    private readonly GpuPPOAgent _brain;          // one shared brain (brainPerWalker: null)
+    private readonly GpuPopulation _population;   // brainPerWalker: agent i is walker i's brain (otherwise null)
     private readonly GpuWalker[] _walkers;
     private readonly Trajectory[] _trajectories;
     private readonly int[] _steps;
@@ -42,7 +45,8 @@ public class GpuEnvironment : IDisposable
     private int _episodes;
     private float _bestDistance, _previousAverageReward;
 
-    public GpuEnvironment(Renderer renderer, int walkers = 1, Wb.Material floorMaterial = Wb.Material.Metal /* Environment.cs:223 */)
+    public GpuEnvironment(Renderer renderer, int walkers = 1, Wb.Material floorMaterial = Wb.Material.Metal /* Environment.cs:223 */,
+                          bool brainPerWalker = false)
     {
         _n = walkers;
         _renderer = renderer;
@@ -50,8 +54,9 @@ public class GpuEnvironment : IDisposable
         var floors = Enumerable.Repeat((byte)floorMaterial, walkers).ToArray();
         Wb.Ok(Wb.wb_init(0), "wb_init");
         Wb.Ok(Wb.wb_env_create(walkers, floors, null, ref hp, out _env), "wb_env_create");
-        _brain = new GpuPPOAgent(Wb.Obs, Wb.Act);
-        _walkers = Enumerable.Range(0, walkers).Select(i => new GpuWalker(this, i, _brain)).ToArray();
+        if (brainPerWalker) _population = new GpuPopulation(walkers);
+        else _brain = new GpuPPOAgent(Wb.Obs, Wb.Act);
+        _walkers = Enumerable.Range(0, walkers).Select(i => new GpuWalker(this, i, _brain, _population)).ToArray();
         _trajectories = Enumerable.Range(0, walkers).Select(_ => new Trajectory()).ToArray();
         _steps = new int[walkers];
         _obs = new float[walkers * Wb.Obs];
@@ -121,29 +126,40 @@ public class GpuEnvironment : IDisposable
             _trajectories[i].States.Add(_walkers[i].GetState());
         }
         // _walker.GetActions(_state, out logProbabilities) for every walker: one batched forward + Box-Muller
-        _brain.SampleActions(_n, _obs, _actions, _logp, _mean);
+        if (_population != null) _population.SampleActions(_n, _obs, _actions, _logp, _mean);
+        else _brain.SampleActions(_n, _obs, _actions, _logp, _mean);
         var sampled = (float[])_actions.Clone();     // the trajectory stores the UNCLIPPED action (Environment.cs:87)
         // TakeActions(Matrix.Clip(action, 1, -1)) + Step + (on terminal) Reset + InitialState: one fused launch, zero-copy I/O
         Wb.Ok(Wb.wb_env_step_pinned(_env, _hActions.AddrOfPinnedObject(), deltaTime, 1, _hObs.AddrOfPinnedObject(),
                                     _hReward.AddrOfPinnedObject(), _hDone.AddrOfPinnedObject()), "wb_env_step");
         _stateFresh = false;
+        var finished = new List<(int agent, Trajectory trajectory)>();
         for (int i = 0; i < _n; i++)
         {
             _trajectories[i].Actions.Add(Matrix.FromValues(sampled.Skip(i * Wb.Act).Take(Wb.Act).ToArray()));
             _trajectories[i].LogProbabilities.Add(Matrix.FromValues(_logp.Skip(i * Wb.Act).Take(Wb.Act).ToArray()));
             _trajectories[i].Rewards.Add(_reward[i]);
             _previousPosition[i] = _position[i];
-            if (_done[i] != 0) TrainNetworks(i);
+            if (_done[i] == 0) continue;
+            if (_population == null) TrainNetworks(i);
+            else { finished.Add((i, _trajectories[i])); EndEpisode(i); }
         }
+        // brainPerWalker: every walker whose episode ended trains its own agent, all in one native call
+        if (finished.Count > 0) _population.Train(finished, _renderer);
         RefreshPositions();
     }
 
     // Environment.TrainNetworks + Reset (Environment.cs:157-173); the physical reset already happened inside the fused step
     private void TrainNetworks(int i)
     {
+        _walkers[i].Train(_trajectories[i], _renderer);
+        EndEpisode(i);
+    }
+
+    private void EndEpisode(int i)
+    {
         _episodes++;
         if (i == 0) _previousAverageReward = _trajectories[i].Rewards.Average();
-        _walkers[i].Train(_trajectories[i], _renderer);
         _trajectories[i] = new Trajectory();
         _steps[i] = 0;
     }
@@ -174,6 +190,7 @@ public class GpuEnvironment : IDisposable
         if (walker == _n - 1 && joint == Wb.Act - 1) { Wb.Ok(Wb.wb_env_take_actions(_env, _actions), "wb_env_take_actions"); _stateFresh = false; }
     }
     internal float[] Observation(int walker) => _obs.Skip(walker * Wb.Obs).Take(Wb.Obs).ToArray();
+    internal float[] Observations() => (float[])_obs.Clone();
     internal Vector2 Position(int walker) => _position[walker];
     internal Vector2 PreviousPosition(int walker) => _previousPosition[walker];
     internal int Flags(int walker) { FetchState(); return _stateI[walker]; }
@@ -200,6 +217,7 @@ public class GpuEnvironment : IDisposable
         Unpin(ref _hActions);
         Unpin(ref _hDone);
         Wb.wb_env_destroy(_env);
-        _brain.Dispose();
+        _brain?.Dispose();
+        _population?.Dispose();
     }
 }

@@ -82,7 +82,7 @@ public sealed class GpuPPOAgent : IDisposable
 
     // DenseLayer ctor (DenseLayer.cs:22-33): weights Matrix.FromXavier(out, in) (Matrix.cs:59-80), zero biases;
     // flat layout per dense layer W[out][in] row-major then b[out] (DenseLayer.Save order)
-    private static float[] Xavier(List<(int outSize, int inSize)> shapes)
+    internal static float[] Xavier(List<(int outSize, int inSize)> shapes)
     {
         var flat = new List<float>();
         foreach (var (o, i) in shapes)
@@ -226,7 +226,7 @@ public sealed class GpuPPOAgent : IDisposable
         if (Hyperparameters.SaveWeights) Save();
     }
 
-    private static float[] Flatten(List<Matrix> rows, int width)
+    internal static float[] Flatten(List<Matrix> rows, int width)
     {
         var flat = new float[rows.Count * width];
         for (int t = 0; t < rows.Count; t++)
@@ -293,4 +293,106 @@ public sealed class GpuPPOAgent : IDisposable
     }
 
     public void Dispose() => Wb.wb_policy_destroy(_policy);
+}
+
+// One PPO brain per walker: P agents of the reference's default networks (Hyperparameters.cs:91-92) on one native handle
+// (wb_population_*).  In the reference every walker owns its PPOAgent (Walker.cs:25-34) and trains it on each of its own episodes
+// (Environment.cs:91,157-164); agent a here is one GpuPPOAgent with its own weights, Adam state and step counters.  The
+// hyper-parameters are the statics at construction.  Xavier initialisation, the Box-Muller uniforms and CreateBatches are drawn
+// from System.Random in C#, as GpuPPOAgent draws them.
+public sealed class GpuPopulation : IDisposable
+{
+    private readonly IntPtr _population;
+    private readonly int _n;
+    private readonly Random _random = new Random();
+    private static readonly List<(int outSize, int inSize)> ActorDense = new() { (64, Wb.Obs), (64, 64), (Wb.Act, 64) };
+    private static readonly List<(int outSize, int inSize)> CriticDense = new() { (64, Wb.Obs), (1, 64) };
+
+    public GpuPopulation(int agents)
+    {
+        _n = agents;
+        var hp = Enumerable.Repeat(WbHyperparams.FromStatics(), agents).ToArray();
+        Wb.Ok(Wb.wb_init(0), "wb_init");
+        Wb.Ok(Wb.wb_population_create(agents, ref hp[0], out _population), "wb_population_create");
+        for (int a = 0; a < agents; a++)   // PPOAgent ctor: the critic's layers are created first, then the actor's (PPOAgent.cs:41-93)
+        {
+            float[] critic = GpuPPOAgent.Xavier(CriticDense), actor = GpuPPOAgent.Xavier(ActorDense);
+            Wb.Ok(Wb.wb_population_set_weights(_population, a, actor.Concat(critic).ToArray()), "wb_population_set_weights");
+        }
+    }
+
+    public int Count => _n;
+
+    // PPOAgent.SampleActions (PPOAgent.cs:381-398) of every agent on its walker's state: states [n][12] -> actions / logp / mean [n][4]
+    public void SampleActions(int n, float[] states, float[] actions, float[] logp, float[] mean)
+    {
+        var uniforms = new float[n * Wb.Act * 2];
+        for (int i = 0; i < uniforms.Length; i++) uniforms[i] = (float)_random.NextDouble();
+        Wb.Ok(Wb.wb_population_sample(_population, n, states, uniforms, actions, logp, mean), "wb_population_sample");
+    }
+
+    // one agent's action on `state`, the other walkers' states as given (the native call samples every agent)
+    public Matrix SampleAction(int agent, float[] state, float[] states, out Matrix logProbabilities)
+    {
+        var all = (float[])states.Clone();
+        Array.Copy(state, 0, all, agent * Wb.Obs, Wb.Obs);
+        float[] actions = new float[_n * Wb.Act], logp = new float[_n * Wb.Act], mean = new float[_n * Wb.Act];
+        SampleActions(_n, all, actions, logp, mean);
+        logProbabilities = Matrix.FromValues(logp.Skip(agent * Wb.Act).Take(Wb.Act).ToArray());
+        return Matrix.FromValues(actions.Skip(agent * Wb.Act).Take(Wb.Act).ToArray());
+    }
+
+    // PPOAgent.Train(Trajectory, Renderer) (PPOAgent.cs:147-172) of each listed agent on its episodes, in list order, as ONE native
+    // call (wb_population_train_trajectories: one kernel launch).  CreateBatches is drawn in list order, as calling
+    // GpuPPOAgent.Train per episode would draw it; the console is updated once per episode, as in GpuPPOAgent's list overload.
+    public void Train(IReadOnlyList<(int agent, Trajectory trajectory)> episodes, Renderer renderer)
+    {
+        int n = episodes.Count, B = Hyperparameters.BatchSize, epochs = Hyperparameters.Epochs;
+        if (n == 0) return;
+        var agents = new int[n];
+        var offsets = new int[n + 1];
+        for (int e = 0; e < n; e++) { agents[e] = episodes[e].agent; offsets[e + 1] = offsets[e] + episodes[e].trajectory.States.Count; }
+        int rows = offsets[n];
+        float[] states = new float[rows * Wb.Obs], actions = new float[rows * Wb.Act], logp = new float[rows * Wb.Act], rewards = new float[rows];
+        var index = new List<int>();
+        for (int e = 0; e < n; e++)
+        {
+            var t = episodes[e].trajectory;
+            int T = t.States.Count, o = offsets[e];
+            Array.Copy(GpuPPOAgent.Flatten(t.States, Wb.Obs), 0, states, o * Wb.Obs, T * Wb.Obs);
+            Array.Copy(GpuPPOAgent.Flatten(t.Actions, Wb.Act), 0, actions, o * Wb.Act, T * Wb.Act);
+            Array.Copy(GpuPPOAgent.Flatten(t.LogProbabilities, Wb.Act), 0, logp, o * Wb.Act, T * Wb.Act);
+            t.Rewards.CopyTo(rewards, o);
+            for (int epoch = 0; epoch < epochs; epoch++)  // CreateBatches (:501-540): sampling without replacement
+            {
+                var pool = Enumerable.Range(0, T).ToList();
+                for (int j = 0; j < T / B; j++)
+                    for (int b = 0; b < B; b++)
+                    {
+                        int pick = _random.Next(0, pool.Count);
+                        index.Add(pool[pick]);
+                        pool.RemoveAt(pick);
+                    }
+            }
+        }
+        float[] values = new float[rows], returns = new float[rows], advantages = new float[rows], losses = new float[2 * n];
+        var skipped = new int[n];
+        Wb.Ok(Wb.wb_population_train_trajectories(_population, n, agents, offsets, epochs, states, actions, logp, rewards, index.ToArray(),
+                                                   values, returns, advantages, losses, skipped), "wb_population_train_trajectories");
+        for (int e = 0; e < n; e++)
+        {
+            var t = episodes[e].trajectory;
+            int T = t.States.Count, o = offsets[e];
+            if (T == 0) continue;
+            t.Values.Clear(); t.Values.AddRange(new ArraySegment<float>(values, o, T));
+            t.Returns.Clear(); t.Returns.AddRange(new ArraySegment<float>(returns, o, T));
+            t.Advantages.Clear(); t.Advantages.AddRange(new ArraySegment<float>(advantages, o, T));
+            renderer.AddTotalEpisodeReward(t.Rewards.Sum());
+            if (T >= B) renderer.UpdateConsole(epochs - 1, T / B - 1, T / B, losses[2 * e]);
+            renderer.AddCriticLoss(losses[2 * e]);
+            renderer.AddActorLoss(losses[2 * e + 1]);
+        }
+    }
+
+    public void Dispose() => Wb.wb_population_destroy(_population);
 }

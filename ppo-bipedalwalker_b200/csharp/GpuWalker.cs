@@ -17,14 +17,16 @@ public sealed class GpuWalker
 {
     private readonly GpuEnvironment _environment;
     private readonly int _index;
-    private readonly GpuPPOAgent _brain;
+    private readonly GpuPPOAgent _brain;          // the shared brain, or null when every walker owns one
+    private readonly GpuPopulation _population;   // brainPerWalker: this walker's agent is agent _index
     public bool Terminal => (_environment.Flags(_index) & 32) != 0;      // WB_FLAG_TERMINAL: Walker.Terminal (Walker.cs:23)
 
-    internal GpuWalker(GpuEnvironment environment, int index, GpuPPOAgent brain)
+    internal GpuWalker(GpuEnvironment environment, int index, GpuPPOAgent brain, GpuPopulation population = null)
     {
         _environment = environment;
         _index = index;
         _brain = brain;
+        _population = population;
     }
 
     // Walker.CreateCreature (Walker.cs:40-46): the library builds bodies, joints, association lists and gravity at wb_env_create
@@ -35,7 +37,9 @@ public sealed class GpuWalker
 
     // Walker.GetActions (Walker.cs:58-62)
     public PPO.Matrix GetActions(PPO.Matrix state, out PPO.Matrix logProbabilities)
-        => _brain.SampleActions(state, out logProbabilities, out _, out _);
+        => _population == null
+            ? _brain.SampleActions(state, out logProbabilities, out _, out _)
+            : _population.SampleAction(_index, PPO.Matrix.GetRepresentation(state), _environment.Observations(), out logProbabilities);
 
     // Walker.TakeActions (Walker.cs:66-75): this walker's four torques; the library clips like Environment.cs:78
     public void TakeActions(PPO.Matrix actions)
@@ -45,7 +49,11 @@ public sealed class GpuWalker
     }
 
     // Walker.Train (Walker.cs:79-82)
-    public void Train(Trajectory trajectory, Renderer renderer) => _brain.Train(trajectory, renderer);
+    public void Train(Trajectory trajectory, Renderer renderer)
+    {
+        if (_population == null) _brain.Train(trajectory, renderer);
+        else _population.Train(new[] { (_index, trajectory) }, renderer);
+    }
 
     // Walker.GetState (Walker.cs:132-152): the 12-float observation the last step produced
     public PPO.Matrix GetState() => PPO.Matrix.FromValues(_environment.Observation(_index));

@@ -102,6 +102,31 @@ struct GradConsts {
   float stdv, neg_log_std, log_sqrt_2pi, upper, lower, variance;
 };
 
+// The sampling of ppo_fused_kernel's forward modes, restated for population_act_kernel (the same expressions in the same
+// translation unit and flags: the same arithmetic; ppo_fused_kernel keeps its own copy so that its SASS stays as it is).
+// The two uniforms of action dimension k of sample gs: injected (kModeSample) or from the Philox stream (gs, k, step) under seed
+__device__ __forceinline__ void sample_uniforms(int mode, const float* uniforms, uint64_t seed, uint64_t step, int gs, int k, float& u1,
+                                                float& u2) {
+  if (mode == kModeSample) {
+    u1 = uniforms[((size_t)gs * kAct + k) * 2];
+    u2 = uniforms[((size_t)gs * kAct + k) * 2 + 1];
+  } else {
+    const uint4 r = philox4x32(make_uint4((uint32_t)gs, (uint32_t)k, (uint32_t)step, (uint32_t)(step >> 32)),
+                               make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+    u1 = (float)(r.x >> 8) * (1.0f / 16777216.0f);  // [0,1) like (float)Random.NextDouble()
+    u2 = (float)(r.y >> 8) * (1.0f / 16777216.0f);
+  }
+}
+
+// NormalDistribution.BoxMullerTransform (NormalDistribution.cs:12-19) around mu, and the action's log-probability
+__device__ __forceinline__ void sample_action(float mu, float stdv, float neg_log_std, float log_sqrt_2pi, float u1, float u2, float& a,
+                                              float& lp) {
+  if (u1 == 0.0f) u1 = 1.0f;
+  const float z = sqrtf(-2.0f * logf(u1)) * sinf(2.0f * 3.14159274f * u2);
+  a = mu + (stdv * z);
+  lp = log_prob(mu, stdv, a, neg_log_std, log_sqrt_2pi);
+}
+
 // ---- the 64-sample tile pipeline of PPOAgent.Train(Batch), shared by ppo_fused_kernel and ppo_episodes_kernel (one CTA of
 // kMlpThreads threads over MlpSmem; the callers stage the tile's states in S.X and own the weight-gradient accumulators and loss
 // sums, which stay in registers across every tile the CTA processes)
@@ -583,6 +608,282 @@ __global__ void __launch_bounds__(kMlpThreads, 1) ppo_episodes_kernel(const Epis
   }
 }
 
+// ---- populations: P independent agents of the default networks, agent a at a * kAgentStride of the parameter / Adam / gradient
+// arrays (new Walker() builds its own PPOAgent(12, 4), Walker.cs:25-34; N walkers of the reference are N independent learners)
+
+__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
+  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+
+// population_act_kernel: PPOAgent.SampleActions (PPOAgent.cs:381-398) for N walkers, walker w with agent w.  One warp per walker:
+// its 5 252 actor parameters (21 KB, every env-step) are copied into the warp's shared memory with cp.async, W2 into rows padded
+// to kPad floats so that the lanes' float4 row reads are conflict-free.  Lane o computes hidden units o and o + 32, lanes 0..3
+// the four means and the sampling, lane 4 the optional critic value.  Every dot product is the chain of dense64_forward /
+// tile_forward (a left-to-right fmaf chain from 0, then + b, then leaky or tanhf) and the sampling is ppo_fused_kernel's, so
+// each row equals wb_policy_act_dev / wb_policy_sample of that agent on kernel variant 1 bit for bit.  Bandwidth-bound.
+constexpr int kActHead = kHid * kIn + kHid;          // W1, b1
+constexpr int kActTail = kHid + kAct * kHid + kAct;  // b2, W3, b3
+struct __align__(16) ActWarpSmem {
+  float head[kActHead];
+  float W2[kHid * kPad];
+  float tail[kActTail];
+  float x[16];
+  float a1[kHid], a2[kHid], c1[kHid];
+};
+
+__global__ void __launch_bounds__(kActWarps * 32) population_act_kernel(const PopActParams P) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int w = blockIdx.x * kActWarps + warp;
+  if (w >= P.n) return;  // (warp-uniform; the kernel has no CTA-wide barrier)
+  ActWarpSmem& S = reinterpret_cast<ActWarpSmem*>(smem_raw)[warp];
+  const float* prm = P.params + (size_t)w * kAgentStride;
+  for (int c = lane; c < kActHead / 4; c += 32) cp_async16(S.head + 4 * c, prm + 4 * c);
+  for (int c = lane; c < kHid * kHid / 4; c += 32) cp_async16(S.W2 + (c >> 4) * kPad + (c & 15) * 4, prm + kOffW2 + 4 * c);
+  for (int c = lane; c < kActTail / 4; c += 32) cp_async16(S.tail + 4 * c, prm + kOffB2 + 4 * c);
+  if (lane < kIn) S.x[lane] = P.states[(size_t)w * kIn + lane];
+  cp_async_wait_all();
+  __syncwarp();
+  const float *W1 = S.head, *b1 = S.head + kHid * kIn, *b2 = S.tail, *W3 = S.tail + kHid, *b3 = W3 + kAct * kHid;
+#pragma unroll
+  for (int h = 0; h < 2; h++) {  // actor L1
+    const int o = lane + 32 * h;
+    float acc = 0.0f;
+#pragma unroll
+    for (int i = 0; i < kIn; i += 4) {
+      const float4 a = ld4(S.x + i), wv = ld4(W1 + o * kIn + i);
+      acc = fmaf(a.x, wv.x, acc);
+      acc = fmaf(a.y, wv.y, acc);
+      acc = fmaf(a.z, wv.z, acc);
+      acc = fmaf(a.w, wv.w, acc);
+    }
+    S.a1[o] = leaky(acc + b1[o]);
+  }
+  if (P.value) {  // critic L1, straight from global memory (read only when the value is asked for)
+#pragma unroll
+    for (int h = 0; h < 2; h++) {
+      const int o = lane + 32 * h;
+      float acc = 0.0f;
+#pragma unroll
+      for (int i = 0; i < kIn; i += 4) {
+        const float4 a = ld4(S.x + i), wv = __ldg(reinterpret_cast<const float4*>(prm + kOffWc1 + o * kIn + i));
+        acc = fmaf(a.x, wv.x, acc);
+        acc = fmaf(a.y, wv.y, acc);
+        acc = fmaf(a.z, wv.z, acc);
+        acc = fmaf(a.w, wv.w, acc);
+      }
+      S.c1[o] = leaky(acc + __ldg(prm + kOffBc1 + o));
+    }
+  }
+  __syncwarp();
+  {  // actor L2
+    float acc0 = 0.0f, acc1 = 0.0f;
+#pragma unroll 4
+    for (int i = 0; i < kHid; i += 4) {
+      const float4 a = ld4(S.a1 + i), w0 = ld4(S.W2 + lane * kPad + i), w1 = ld4(S.W2 + (lane + 32) * kPad + i);
+      acc0 = fmaf(a.x, w0.x, acc0);
+      acc0 = fmaf(a.y, w0.y, acc0);
+      acc0 = fmaf(a.z, w0.z, acc0);
+      acc0 = fmaf(a.w, w0.w, acc0);
+      acc1 = fmaf(a.x, w1.x, acc1);
+      acc1 = fmaf(a.y, w1.y, acc1);
+      acc1 = fmaf(a.z, w1.z, acc1);
+      acc1 = fmaf(a.w, w1.w, acc1);
+    }
+    S.a2[lane] = leaky(acc0 + b2[lane]);
+    S.a2[lane + 32] = leaky(acc1 + b2[lane + 32]);
+  }
+  __syncwarp();
+  if (lane < kAct) {  // actor L3 + TanH, then Box-Muller and log_prob
+    const int k = lane;
+    float sum = 0.0f;
+#pragma unroll 4
+    for (int i = 0; i < kHid; i += 4) {
+      const float4 a = ld4(S.a2 + i), wv = ld4(W3 + k * kHid + i);
+      sum = fmaf(a.x, wv.x, sum);
+      sum = fmaf(a.y, wv.y, sum);
+      sum = fmaf(a.z, wv.z, sum);
+      sum = fmaf(a.w, wv.w, sum);
+    }
+    const float mu = tanhf(sum + b3[k]);
+    const PopAgent& ag = P.agents[w];
+    float u1, u2, a, lp;
+    sample_uniforms(P.mode, P.uniforms, P.seed, P.step, w, k, u1, u2);
+    sample_action(mu, ag.stdv, ag.neg_log_std, ag.log_sqrt_2pi, u1, u2, a, lp);
+    P.actions[(size_t)w * kAct + k] = a;
+    P.logp[(size_t)w * kAct + k] = lp;
+    if (P.mean) P.mean[(size_t)w * kAct + k] = mu;
+  } else if (lane == kAct && P.value) {  // critic L2
+    float v = 0.0f;
+#pragma unroll 4
+    for (int i = 0; i < kHid; i += 4) {
+      const float4 a = ld4(S.c1 + i), wv = __ldg(reinterpret_cast<const float4*>(prm + kOffWc2 + i));
+      v = fmaf(a.x, wv.x, v);
+      v = fmaf(a.y, wv.y, v);
+      v = fmaf(a.z, wv.z, v);
+      v = fmaf(a.w, wv.w, v);
+    }
+    P.value[w] = v + __ldg(prm + kOffBc2);
+  }
+}
+
+// population_episodes_kernel: ppo_episodes_kernel over many agents -- one CTA per agent with work in the call, training that agent's
+// items (finished episodes) in list order with the agent's own parameters, Adam moments, gradient buffer, constants and slice of
+// the host's Adam correction table.  Independent networks, so the CTAs need no exchange (one SM per agent).  An item's rows live
+// in a time-major ring [R][C]: row i = ((t0 + i) mod R) * C + column.  Its rewards and values are gathered into shared memory for
+// trajectory_returns and the returns / advantages scattered back.  Mini-batch indices come from the caller or, with a null index
+// pointer, from draw_permutation (below).
+struct __align__(16) PopSmem {
+  MlpSmem m;
+  int32_t rows[kTile];
+  float rew[kPopMaxLen], val[kPopMaxLen], ret[kPopMaxLen], adv[kPopMaxLen];
+  uint32_t key[kPopMaxLen];
+  int32_t perm[kPopMaxLen];
+};
+
+// PPOAgent.CreateBatches (PPOAgent.cs:501-540: sampling without replacement) drawn on the device: local row i of the episode gets
+// key(i) = Philox-4x32-10(counter (i, epoch, episode, agent), key (seed lo, seed hi)).x, where `episode` counts the agent's episodes
+// trained before this one; perm = the rows ordered by (key, row).  Each row's rank is counted over the <= 1 024 keys.
+__device__ __forceinline__ void draw_permutation(PopSmem& E, int L, int epoch, int episode, int agent, uint64_t seed, int tid) {
+  for (int i = tid; i < L; i += kMlpThreads)
+    E.key[i] = philox4x32(make_uint4((uint32_t)i, (uint32_t)epoch, (uint32_t)episode, (uint32_t)agent),
+                          make_uint2((uint32_t)seed, (uint32_t)(seed >> 32))).x;
+  __syncthreads();
+  for (int j = tid; j < L; j += kMlpThreads) {
+    const uint32_t kj = E.key[j];
+    int rank = 0;
+    for (int i = 0; i < L; i++) {
+      const uint32_t ki = E.key[i];
+      rank += (ki < kj || (ki == kj && i < j)) ? 1 : 0;
+    }
+    E.perm[rank] = j;
+  }
+  __syncthreads();
+}
+
+__global__ void __launch_bounds__(kMlpThreads, 1) population_episodes_kernel(const PopTrainParams P) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  PopSmem& E = *reinterpret_cast<PopSmem*>(smem_raw);
+  MlpSmem& S = E.m;
+  const int tid = threadIdx.x;
+  const PopCta cta = P.ctas[blockIdx.x];
+  const PopAgent ag = P.agents[cta.agent];
+  const size_t base = (size_t)cta.agent * kAgentStride;
+  MlpParams p{};
+  p.params = P.params + base;
+  p.states = P.states;
+  p.actions = P.actions;
+  p.old_logp = P.old_logp;
+  p.advantages = P.advantages;
+  p.returns = P.returns;
+  p.batch_size = ag.batch_size_f;
+  const GradConsts gc{ag.stdv, ag.neg_log_std, ag.log_sqrt_2pi, ag.upper, ag.lower, ag.variance};
+  float* grads = P.grads + base;
+  AdamParams adam{};
+  adam.params = P.params + base;
+  adam.grads = grads;
+  adam.m = P.m + base;
+  adam.v = P.v + base;
+  adam.alpha = ag.alpha;
+  adam.beta1 = ag.beta1;
+  adam.beta2 = ag.beta2;
+  adam.eps = ag.adam_eps;
+  const int B = ag.batch, R = P.ring_rows, C = P.columns;
+  stage_weights(S, p, tid);
+  for (int it = 0; it < cta.count; it++) {
+    const PopItem item = P.items[cta.first + it];
+    const int L = item.length;
+    auto row_of = [&](int i) {
+      const int t = item.t0 + i;
+      return (t >= R ? t - R : t) * C + item.column;
+    };
+    // ---- CalculateValues (PPOAgent.cs:175-189)
+    for (int s0 = 0; s0 < L; s0 += kTile) {
+      const int nvalid = min(kTile, L - s0);
+      __syncthreads();
+      for (int i = tid; i < kTile * kIn; i += kMlpThreads) {
+        const int s = i / kIn;
+        S.X[i] = (s < nvalid) ? p.states[(size_t)row_of(s0 + s) * kIn + (i - s * kIn)] : 0.0f;
+      }
+      __syncthreads();
+      tile_forward(S, tid);
+      if (tid < nvalid) E.val[s0 + tid] = S.V[tid];
+    }
+    for (int i = tid; i < L; i += kMlpThreads) E.rew[i] = P.rewards[row_of(i)];
+    __syncthreads();
+    if (tid == 0 && L > 0)
+      trajectory_returns(E.rew, E.val, L, ag.gamma, ag.lambda, ag.use_gae, ag.normalize, ag.norm_eps, E.ret, E.adv);
+    __syncthreads();
+    for (int i = tid; i < L; i += kMlpThreads) {
+      const int r = row_of(i);
+      P.values[r] = E.val[i];
+      P.returns[r] = E.ret[i];
+      P.advantages[r] = E.adv[i];
+    }
+    __syncthreads();  // (the surrogate reads the returns / advantages back from global memory)
+    // ---- epochs x floor(L / B) mini-batches, each Train(Batch) + NeuralNetwork.Optimise
+    const int per_epoch = L / B;
+    int step = 0;
+    float skipped_total = 0.0f;
+    for (int epoch = 0; epoch < P.epochs && per_epoch > 0; epoch++) {
+      const int32_t* index = E.perm;
+      if (P.batch_index) index = P.batch_index + item.index_off + (size_t)epoch * per_epoch * B;
+      else draw_permutation(E, L, epoch, item.episode, cta.agent, P.seed, tid);
+      for (int b = 0; b < per_epoch; b++, step++, index += B) {
+        float accW2[4][4];
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+#pragma unroll
+          for (int l = 0; l < 4; l++) accW2[j][l] = 0.0f;
+        float accW1[3] = {0.f, 0.f, 0.f}, accWc1[3] = {0.f, 0.f, 0.f};
+        float accW3 = 0.0f, accS = 0.0f, accT = 0.0f;
+        float lossV = 0.0f, lossA = 0.0f, skipped = 0.0f;
+        for (int b0 = 0; b0 < B; b0 += kTile) {
+          const int nvalid = min(kTile, B - b0);
+          __syncthreads();
+          if (tid < kTile) E.rows[tid] = row_of(tid < nvalid ? index[b0 + tid] : 0);
+          __syncthreads();
+          for (int i = tid; i < kTile * kIn; i += kMlpThreads) {
+            const int s = i / kIn;
+            S.X[i] = (s < nvalid) ? p.states[(size_t)E.rows[s] * kIn + (i - s * kIn)] : 0.0f;
+          }
+          __syncthreads();
+          tile_forward(S, tid);
+          tile_surrogate(S, p, gc, nvalid, [&](int s) { return E.rows[s]; }, lossV, lossA, skipped, tid);
+          tile_backward(S, accW2, accW1, accWc1, accW3, accS, accT, tid);
+        }
+        __syncthreads();
+        write_grad(S, accW2, accW1, accWc1, accW3, accS, accT, lossV, lossA, skipped, grads, tid);
+        AdamParams a = adam;
+        const float* corr = P.corr + (size_t)(item.corr_off + step) * 10;
+#pragma unroll
+        for (int l = 0; l < 5; l++) {
+          a.corr1[l] = corr[l];
+          a.corr2[l] = corr[5 + l];
+        }
+        for (int i = tid; i < kTotalParams + 3; i += kMlpThreads) {
+          const float g = __fadd_rn(grads[i], 0.0f);  // (as ppo_episodes_kernel: what the one-partial reduction stores)
+          grads[i] = g;
+          if (i < kTotalParams) adam_update(a, i, g);
+        }
+        __syncthreads();
+        if (tid == 0) skipped_total += grads[kGradSkipped];
+        stage_weights(S, p, tid);  // (ordered before the next use by the next tile's first barrier)
+      }
+    }
+    if (tid == 0) {
+      const bool trained = P.epochs > 0 && per_epoch > 0;
+      if (P.losses) {
+        P.losses[2 * item.out] = trained ? grads[kGradLossV] : 0.0f;
+        P.losses[2 * item.out + 1] = trained ? grads[kGradLossA] : 0.0f;
+      }
+      if (P.skipped) P.skipped[item.out] = (int32_t)skipped_total;
+    }
+  }
+}
+
 // The same recurrences over a time-major rollout buffer [T][N] of N lockstep environments (the reference trains on one
 // episode of one environment, PPOAgent.cs:147; here every environment contributes the fragments of its episodes that fall
 // inside the T-step segment).  One thread per environment, reverse scan; a step with done != 0 is the LAST step of its
@@ -698,6 +999,55 @@ static GradConsts grad_consts(float log_std, float epsilon) {
   gc.lower = 1.0f - epsilon;
   gc.variance = gc.stdv * gc.stdv;
   return gc;
+}
+
+void population_agent_consts(const wb_hyperparams& hp, PopAgent* o) {
+  const GradConsts gc = grad_consts(hp.log_std, hp.epsilon);
+  *o = PopAgent{};
+  o->stdv = gc.stdv;
+  o->neg_log_std = gc.neg_log_std;
+  o->log_sqrt_2pi = gc.log_sqrt_2pi;
+  o->upper = gc.upper;
+  o->lower = gc.lower;
+  o->variance = gc.variance;
+  o->alpha = hp.alpha;
+  o->beta1 = hp.beta1;
+  o->beta2 = hp.beta2;
+  o->adam_eps = hp.adam_epsilon;
+  o->gamma = hp.gamma;
+  o->lambda = hp.lambda;
+  o->norm_eps = hp.epsilon;  // PPOAgent.Normalize divides by std + the PPO clip epsilon, as trajectory_returns' callers pass it
+  o->batch_size_f = (float)hp.batch_size;
+  o->batch = hp.batch_size;
+  o->use_gae = hp.use_gae;
+  o->normalize = hp.normalize_advantages;
+}
+
+cudaError_t launch_population_act(const PopActParams& a, cudaStream_t stream) {
+  static bool configured[64] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  const int smem = (int)(kActWarps * sizeof(ActWarpSmem));
+  if (dev < 0 || dev >= 64 || !configured[dev]) {
+    cudaError_t err = cudaFuncSetAttribute(population_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+    if (err != cudaSuccess) return err;
+    if (dev >= 0 && dev < 64) configured[dev] = true;
+  }
+  population_act_kernel<<<(a.n + kActWarps - 1) / kActWarps, kActWarps * 32, smem, stream>>>(a);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_population_episodes(const PopTrainParams& t, int n_ctas, cudaStream_t stream) {
+  static bool configured[64] = {};
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev < 0 || dev >= 64 || !configured[dev]) {
+    cudaError_t err = cudaFuncSetAttribute(population_episodes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PopSmem));
+    if (err != cudaSuccess) return err;
+    if (dev >= 0 && dev < 64) configured[dev] = true;
+  }
+  population_episodes_kernel<<<n_ctas, kMlpThreads, sizeof(PopSmem), stream>>>(t);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_segment_returns(const float* rewards, const float* values, const uint8_t* dones, const float* last_values, int n_envs,

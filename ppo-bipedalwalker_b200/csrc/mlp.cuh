@@ -111,6 +111,68 @@ cudaError_t launch_gather_rows(const int32_t* index, int B, int row_base, int sd
 // losses[2] <- grads_tail[0..1], *skipped += grads_tail[2] (either may be null)
 cudaError_t launch_episode_losses(const float* grads_tail, float* losses, int32_t* skipped, cudaStream_t stream);
 
+// ---- populations: P independent agents of the default networks (population_act_kernel / population_episodes_kernel, mlp.cu)
+// Every agent's parameters, Adam moments and gradient buffer sit at agent * kAgentStride floats (16-byte aligned rows).
+constexpr int kAgentStride = kGradFloats;  // 6152 >= kTotalParams + 3
+constexpr int kPopMaxLen = 1024;           // longest episode a population trains (the reference caps one at MaxTimesteps + 1 = 1 001)
+constexpr int kActWarps = 4;               // walkers (one warp each) per CTA of population_act_kernel
+// per-agent constants, built on the host from the agent's wb_hyperparams (population_agent_consts)
+struct PopAgent {
+  float stdv, neg_log_std, log_sqrt_2pi, upper, lower, variance;  // GradConsts
+  float alpha, beta1, beta2, adam_eps;
+  float gamma, lambda, norm_eps, batch_size_f;
+  int32_t batch, use_gae, normalize, pad;
+};
+void population_agent_consts(const wb_hyperparams& hp, PopAgent* out);
+struct PopActParams {
+  const float* params;     // [P][kAgentStride]
+  const PopAgent* agents;  // [P]
+  int32_t n, mode;         // walker w acts with agent w; mode kModeSample (uniforms) or kModeSamplePhilox
+  const float* states;     // [n][12]
+  const float* uniforms;   // [n][4][2] (kModeSample)
+  uint64_t seed, step;     // (kModeSamplePhilox)
+  float* actions;          // [n][4]
+  float* logp;             // [n][4]
+  float* mean;             // [n][4] or null
+  float* value;            // [n] or null
+};
+cudaError_t launch_population_act(const PopActParams& a, cudaStream_t stream);
+// one item = one finished episode: rows ((t0 + i) mod ring_rows) * columns + column, i < length
+struct PopItem {
+  int32_t out;        // position of the item in the caller's list (losses / skipped)
+  int32_t column, t0, length;
+  int32_t index_off;  // first of its caller-drawn mini-batch indices (unused for device draws)
+  int32_t corr_off;   // first of its Adam steps in the correction table
+  int32_t episode;    // episodes of this agent trained before this one (device draws)
+  int32_t pad;
+};
+struct PopCta {
+  int32_t agent, first, count, pad;  // items [first, first + count) of the table, in list order
+};
+struct PopTrainParams {
+  const float* states;      // ring [R][C][12]
+  const float* actions;     // ring [R][C][4]
+  const float* old_logp;    // ring [R][C][4]
+  const float* rewards;     // ring [R][C]
+  float* values;            // ring [R][C]
+  float* returns;           // ring [R][C]
+  float* advantages;        // ring [R][C]
+  const int32_t* batch_index;  // caller-drawn local rows, or null: drawn on the device
+  const PopCta* ctas;
+  const PopItem* items;
+  const float* corr;        // [Adam steps][10]
+  const PopAgent* agents;
+  float* params;            // [P][kAgentStride]
+  float* m;
+  float* v;
+  float* grads;
+  float* losses;            // [n_items][2] or null
+  int32_t* skipped;         // [n_items] or null
+  int32_t ring_rows, columns, epochs;
+  uint64_t seed;
+};
+cudaError_t launch_population_episodes(const PopTrainParams& t, int n_ctas, cudaStream_t stream);
+
 int mlp_grid_for(int n, int sm_count);
 cudaError_t launch_mlp(const MlpParams& p, int grid, cudaStream_t stream);
 cudaError_t launch_reduce_partials(const float* partials, int nparts, float* grads, cudaStream_t stream);

@@ -112,17 +112,8 @@ class _Net:
         check(lib().wb_policy_set_adam(self._a._h, self._which, ptr(np.ascontiguousarray(m, np.float32)),
                                        ptr(np.ascontiguousarray(v, np.float32)), ptr(np.ascontiguousarray(it, np.int32))))
 
-    # NeuralNetwork.Save / DenseLayer.Save (NeuralNetwork.cs:159-176, DenseLayer.cs:73-79, Matrix.cs:133-153)
     def Save(self) -> list[str]:
-        flat = self.get_flat()
-        lines, p = [self.structure], 0
-        for out, inp in self.shapes:
-            w = flat[p:p + out * inp]
-            p += out * inp
-            b = flat[p:p + out]
-            p += out
-            lines.append("W " + " ".join(net_float_str(x) for x in w) + " B " + " ".join(net_float_str(x) for x in b))
-        return lines
+        return weights_lines(self.structure, self.shapes, self.get_flat())
 
     # NeuralNetwork.Load / ValidateWeights / DenseLayer.Load / Matrix.Load (NeuralNetwork.cs:94-150, DenseLayer.cs:55-69, Matrix.cs:109-130)
     def Load(self, contents: list[str]) -> bool:
@@ -155,6 +146,19 @@ class _Net:
             p += out
         self.set_flat(flat)
         return True
+
+
+# NeuralNetwork.Save / DenseLayer.Save (NeuralNetwork.cs:159-176, DenseLayer.cs:73-79, Matrix.cs:133-153)
+def weights_lines(structure: str, shapes, flat) -> list[str]:
+    """The lines of a .weights file: the structure line, then "W <weights> B <biases>" per dense layer."""
+    lines, p = [structure], 0
+    for out, inp in shapes:
+        w = flat[p:p + out * inp]
+        p += out * inp
+        b = flat[p:p + out]
+        p += out
+        lines.append("W " + " ".join(net_float_str(x) for x in w) + " B " + " ".join(net_float_str(x) for x in b))
+    return lines
 
 
 def net_float_str(x) -> str:
