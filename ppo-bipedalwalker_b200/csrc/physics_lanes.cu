@@ -159,7 +159,9 @@ __device__ __forceinline__ void calculate_impulse(const BodyDyn& A, const BodyDy
   const float2 vrel = vsub(vb, va);
   const float vn = vdot(vrel, n);
   const float j = fmul(-force, vn);
-  const float denom = fadd(fadd(fadd(A.im, B.im), fmul(fmul(kA, kA), A.ii)), fmul(fmul(kB, kB), B.ii));
+  const float2 k = mk2(kA, kB);
+  const float2 kki = vmul2_nosum(vmul2_nosum(k, k), mk2(A.ii, B.ii));  // (kA*kA*A.ii, kB*kB*B.ii)
+  const float denom = fadd(fadd(fadd(A.im, B.im), kki.x), kki.y);
   impulse = fdiv(j, denom);
 }
 
@@ -196,14 +198,16 @@ __device__ __forceinline__ void move_bodies(const EV& e, bool on, int A, float2 
 }
 
 // ---------------------------------------------------------------- Joint.Step, Joint.cs:31-41
-template <class EV, bool TRACE>
+// G = EV::L: the env's lanes step one joint; G < EV::L: the working group of G lanes (e.gsub, e.gshift) steps its own joint
+template <class EV, bool TRACE, int G = EV::L>
 __device__ __forceinline__ void joint_step(const EV& e, int A, int ia, int B, int ib, wb_joint_trace* tr) {
+  const bool leader = (G == EV::L) ? e.sub == 0 : e.gsub == 0;
   const float2 pA = V2(e, A * 6 + ia);
   const float2 pB = V2(e, B * 6 + ib);
   float2 ab = vsub(pB, pA);
-  const float depth = fsqrt(fadd(fmul(ab.x, ab.x), fmul(ab.y, ab.y)));  // Vector2.Length
+  const float depth = fsqrt(vdot(ab, ab));  // Vector2.Length
   if (TRACE) {
-    if (tr && e.live && e.sub == 0) {
+    if (tr && e.live && leader) {
       tr->active = !(depth < 0.1f);
       tr->depth = depth;
     }
@@ -216,7 +220,7 @@ __device__ __forceinline__ void joint_step(const EV& e, int A, int ia, int B, in
   BodyDyn X = load_dyn(e, B);  // Manifold(bodyA := joint._bodyB, bodyB := joint._bodyA), Joint.cs:40
   BodyDyn Y = load_dyn(e, A);
   lanes_sync<EV::L>();  // every lane has read the pre-move points, centroids and velocities
-  move_bodies<EV, EV::L>(e, active, A, dA, true, B, dB);
+  move_bodies<EV, G>(e, active, A, dA, true, B, dB);
   X.c = vadd(X.c, dB);  // the impulse sees the POST-move centroids and joint points
   Y.c = vadd(Y.c, dA);
   const float2 contact = vhalf(vadd(vadd(pA, dA), vadd(pB, dB)));  // Vector2.Divide(p0 + p1, 2), Impulses.cs:35
@@ -224,7 +228,7 @@ __device__ __forceinline__ void joint_step(const EV& e, int A, int ia, int B, in
   float j;
   calculate_impulse(X, Y, contact, fadd(1.0f, 1.0f), ab, rX, rY, j);
   apply_impulses(X, Y, ab, j, rX, rY);
-  if (active && e.sub == 0) {
+  if (active && leader) {
     store_dyn(e, B, X);
     store_dyn(e, A, Y);
   }
@@ -302,8 +306,8 @@ __device__ __forceinline__ Face significant_face_floor(const EV& e, float2 nrm) 
 // ClipVectors, ContactPoints.cs:56-76: appends up to 3 points; only the first two are ever used
 __device__ __forceinline__ int clip_vectors(float2 a, float2 b, float2 nrm, float offset, float2& o0, float2& o1) {
   int cnt = 0;
-  const float da = fsub(vdot(a, nrm), offset);
-  const float db = fsub(vdot(b, nrm), offset);
+  const float2 dab = vsub(mk2(vdot(a, nrm), vdot(b, nrm)), mk2(offset, offset));
+  const float da = dab.x, db = dab.y;
   if (da >= 0.0f) {
     o0 = a;
     cnt = 1;
@@ -547,7 +551,8 @@ __device__ __forceinline__ void resolve_pair(EV& e, bool want, int A, int B, wb_
     constexpr bool kVote = VOTE < 0 ? (G != 4) : (VOTE != 0);
     bool my_sep = false;
     auto accumulate = [&](bool use, float2 axis, int axis_idx, float omin, float omax, float tmin, float tmax) {
-      const float temp = fminf(fsub(tmax, omin), fsub(omax, tmin));
+      const float2 dd = vsub(mk2(tmax, omax), mk2(omin, tmin));  // (tmax - omin, omax - tmin)
+      const float temp = fminf(dd.x, dd.y);
       const bool overlapping = (omin < tmax) && (tmin < omax);
       if (use && temp < depth) {
         depth = temp;
@@ -783,7 +788,6 @@ __device__ __forceinline__ void body_step(EV& e, bool on, int b, float dt, wb_pa
   else if (ang < -PI_F) ang = fadd(ang, TAU_F);
   float m11, m12;
   rotz(theta, m11, m12);
-  const float m21 = -m12, m22 = m11;
   const float2 cen = vadd(V2(e, kV2Cen + b), d);
   lanes_sync<EV::L>();  // all reads of the old centroid / velocity / angle are done
 #pragma unroll
@@ -793,9 +797,7 @@ __device__ __forceinline__ void body_step(EV& e, bool on, int b, float dt, wb_pa
       // Move then Rotate (Vector2.Transform(p - centroid, R) + centroid, Skeleton.cs:93)
       float2 p = vadd(V2(e, b * 6 + i), d);
       p = vsub(p, cen);
-      float2 t;
-      t.x = fadd(fadd(fmul(p.x, m11), fmul(p.y, m21)), 0.0f);
-      t.y = fadd(fadd(fmul(p.x, m12), fmul(p.y, m22)), 0.0f);
+      const float2 t = vrotate(p, m11, m12);
       V2(e, b * 6 + i) = vadd(t, cen);
     }
   }
@@ -956,10 +958,26 @@ __global__ void __launch_bounds__(32, (L <= 4) ? 16 : 8) physics_lanes_kernel(co
         if (p.pair_trace) pt = p.pair_trace + ((size_t)envc * p.iterations + it) * WB_PAIR_SLOTS;  // all 9 slots are written every substep
       }
       // joints in creation order (Walker.cs:182-187): (Body v1, LLU v4) (Body v1, RLU v4) (LLU v2, LLL v3) (RLU v2, RLL v3)
+      if (LEGS == 1) {
 #pragma unroll 1
-      for (int k = 0; k < 4; k++) {
-        const int A = (0x4122 >> (4 * k)) & 0xF, B = (0x3041 >> (4 * k)) & 0xF;
-        joint_step<EV, TRACE>(e, A, k < 2 ? 1 : 2, B, k < 2 ? 4 : 3, jt ? jt + k : nullptr);
+        for (int k = 0; k < 4; k++) {
+          const int A = (0x4122 >> (4 * k)) & 0xF, B = (0x3041 >> (4 * k)) & 0xF;
+          joint_step<EV, TRACE>(e, A, k < 2 ? 1 : 2, B, k < 2 ? 4 : 3, jt ? jt + k : nullptr);
+        }
+      } else {
+        // joint 1 (Body, RLU) and joint 2 (LLU, LLL) share no body: each body still sees its joints in creation order
+        // (Body: 0, 1; LLU: 0, 2; RLU: 1, 3), so stepping 1 and 2 side by side on the two halves of the env's lanes gives the
+        // sequential result bit for bit with three joint steps on the walker's chain instead of four
+        constexpr int G = L / LEGS;
+        joint_step<EV, TRACE>(e, BODY, 1, LLU, 4, jt ? jt + 0 : nullptr);
+        const int leg = e.sub / G;
+        e.gsub = e.sub % G;
+        e.gshift = col * L + leg * G;
+        const bool left = leg == 0;  // (one call with per-lane bodies: control flow stays warp-uniform)
+        joint_step<EV, TRACE, G>(e, left ? LLU : BODY, left ? 2 : 1, left ? LLL : RLU, left ? 3 : 4, jt ? jt + (left ? 2 : 1) : nullptr);
+        e.gsub = e.sub;
+        e.gshift = col * L;
+        joint_step<EV, TRACE>(e, RLU, 2, RLL, 3, jt ? jt + 3 : nullptr);
       }
       // bodies in list order; the static floor's Update is a no-op (a = v = 0, returns before rotation/collisions)
       if (LEGS == 1) {
@@ -1282,15 +1300,12 @@ __device__ __forceinline__ void integrate_body_inl(const EV& e, int b, float dt)
   else if (ang < -PI_F) ang = fadd(ang, TAU_F);
   float m11, m12;
   rotz(theta, m11, m12);
-  const float m21 = -m12, m22 = m11;
   const float2 cen = vadd(V2(e, kV2Cen + b), d);
 #pragma unroll
   for (int i = 0; i < 6; i++) {
     float2 p = vadd(V2(e, b * 6 + i), d);
     p = vsub(p, cen);
-    float2 t;
-    t.x = fadd(fadd(fmul(p.x, m11), fmul(p.y, m21)), 0.0f);
-    t.y = fadd(fadd(fmul(p.x, m12), fmul(p.y, m22)), 0.0f);
+    const float2 t = vrotate(p, m11, m12);
     V2(e, b * 6 + i) = vadd(t, cen);
   }
   V2(e, kV2Cen + b) = cen;
@@ -1323,16 +1338,13 @@ __device__ __noinline__ bool integrate_body_floor_test(int col, int b, float dt)
   else if (ang < -PI_F) ang = fadd(ang, TAU_F);
   float m11, m12;
   rotz(theta, m11, m12);
-  const float m21 = -m12, m22 = m11;
   const float2 cen = vadd(V2(e, kV2Cen + b), d);
   float2 P[6];
 #pragma unroll
   for (int i = 0; i < 6; i++) {
     float2 p = vadd(V2(e, b * 6 + i), d);
     p = vsub(p, cen);
-    float2 t;
-    t.x = fadd(fadd(fmul(p.x, m11), fmul(p.y, m21)), 0.0f);
-    t.y = fadd(fadd(fmul(p.x, m12), fmul(p.y, m22)), 0.0f);
+    const float2 t = vrotate(p, m11, m12);
     P[i] = vadd(t, cen);
     V2(e, b * 6 + i) = P[i];
   }

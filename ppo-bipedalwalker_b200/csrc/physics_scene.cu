@@ -324,14 +324,11 @@ __device__ void body_step(Ctx& c, int b, float dt) {
   ANGLE(c, b) = ang;
   float m11, m12;
   rotz(theta, m11, m12);
-  const float m21 = -m12, m22 = m11;
   const float2 cen = CEN(c, b);
   const int n = c.s->n_verts[b];
   for (int i = 0; i < n; i++) {  // Skeleton.Rotate, Skeleton.cs:89-97
     const float2 p = vsub(VX(c, b, i), cen);
-    float2 t;
-    t.x = fadd(fadd(fmul(p.x, m11), fmul(p.y, m21)), 0.0f);
-    t.y = fadd(fadd(fmul(p.x, m12), fmul(p.y, m22)), 0.0f);
+    const float2 t = vrotate(p, m11, m12);
     VX(c, b, i) = vadd(t, cen);
   }
   resolve_collisions(c, b);

@@ -10,7 +10,7 @@ unset CC CXX
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xcompiler -ffp-contract=off -ftz=false -prec-div=true -prec-sqrt=true"
 objs=""
 for f in physics_lanes api_env physics_scene api_scene; do nvcc $FLAGS -fmad=false -c $tmp/ppo-bipedalwalker_b200/csrc/$f.cu -o $tmp/$f.o & done
-for f in mlp mlp_tc mlp_generic api_policy; do nvcc $FLAGS -c $tmp/ppo-bipedalwalker_b200/csrc/$f.cu -o $tmp/$f.o & done
+for f in mlp mlp_tc mlp_generic api_policy api_population; do nvcc $FLAGS -c $tmp/ppo-bipedalwalker_b200/csrc/$f.cu -o $tmp/$f.o & done
 wait
 nvcc -gencode arch=compute_100a,code=sm_100a -shared -o ppo-bipedalwalker_b200/lib/libwalker_b200_$tag.so $tmp/*.o -lcudart_static -lpthread -ldl -lrt
 rm -rf "$tmp"

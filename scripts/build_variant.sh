@@ -10,5 +10,5 @@ L=ppo-bipedalwalker_b200/lib
 FLAGS="-gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xcompiler -ffp-contract=off -ftz=false -prec-div=true -prec-sqrt=true -fmad=false"
 nvcc $FLAGS "$@" -c ppo-bipedalwalker_b200/csrc/physics_lanes.cu -o $L/physics_lanes_$tag.o
 nvcc -gencode arch=compute_100a,code=sm_100a -shared -o $L/libwalker_b200_$tag.so $L/physics_lanes_$tag.o $L/api_env.o $L/physics_scene.o $L/api_scene.o \
-  $L/mlp.o $L/mlp_tc.o $L/mlp_generic.o $L/api_policy.o -lcudart_static -lpthread -ldl -lrt
+  $L/mlp.o $L/mlp_tc.o $L/mlp_generic.o $L/api_policy.o $L/api_population.o -lcudart_static -lpthread -ldl -lrt
 echo built $L/libwalker_b200_$tag.so
