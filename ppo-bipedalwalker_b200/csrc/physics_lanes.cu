@@ -37,6 +37,10 @@
 #ifndef WB_SAT_UNROLL
 #define WB_SAT_UNROLL 6
 #endif
+// 1: the leg-split body sweep gives the Body a slot of its own (three slots per substep instead of two, see legs_sweep)
+#ifndef WB_BODY_SLOT
+#define WB_BODY_SLOT 0
+#endif
 
 namespace wb {
 namespace pl {
@@ -484,6 +488,19 @@ __device__ __noinline__ void contact_stage_shared(int col, bool live, bool colli
   lanes_sync<EV::L>();
 }
 
+// pair-trace record of a candidate whose SAT has not found a collision (yet)
+__device__ __forceinline__ wb_pair_trace pair_trace_no_sat(int other, bool aabb) {
+  wb_pair_trace rec;
+  rec.other = other;
+  rec.aabb = aabb ? 1 : 0;
+  rec.sat = 0;
+  rec.axis = -1;
+  rec.nx = rec.ny = rec.depth = 0.0f;
+  rec.ncontacts = 0;
+  rec.c0x = rec.c0y = rec.c1x = rec.c1y = 0.0f;
+  return rec;
+}
+
 // ---------------------------------------------------------------- one candidate of RigidBody.ResolveCollisions (RigidBody.cs:66-96)
 // FLOORB = false: a leg segment A against the other segment B of its own leg (both dynamic poles)
 // FLOORB = true : a walker body A against the static floor (scene constants)
@@ -515,15 +532,7 @@ __device__ __forceinline__ void resolve_pair(EV& e, bool want, int A, int B, wb_
   }
   if (FLOORB && hit) e.flags |= (1 << A);  // if (body._isFloor) Collided = true  (before SAT: RigidBody.cs:75)
   wb_pair_trace rec;
-  if (TRACE) {
-    rec.other = FLOORB ? FLOOR : B;
-    rec.aabb = hit ? 1 : 0;
-    rec.sat = 0;
-    rec.axis = -1;
-    rec.nx = rec.ny = rec.depth = 0.0f;
-    rec.ncontacts = 0;
-    rec.c0x = rec.c0y = rec.c1x = rec.c1y = 0.0f;
-  }
+  if (TRACE) rec = pair_trace_no_sat(FLOORB ? FLOOR : B, hit);
 #ifdef WB_PHASE_PROFILE
   const long long rp_t0 = prof_clock();
   long long rp_t1 = rp_t0;
@@ -772,9 +781,11 @@ __device__ __forceinline__ void resolve_pair(EV& e, bool want, int A, int B, wb_
 
 
 // ---------------------------------------------------------------- RigidBody.Step, RigidBody.cs:54-61,116-140
-// `on`: this lane group really steps body b (false for the right-leg half while the left-leg half steps the Body)
-template <class EV, int G, bool TRACE>
-__device__ __forceinline__ void body_step(EV& e, bool on, int b, float dt, wb_pair_trace* tr_base) {
+// The integration half: StepLinearVelocity, StepAngularVelocity, Skeleton.Move + Rotate of body b by the nq lanes that step it
+// (this lane is number q of them); round r moves vertex slot r * nq + q and also leaves the new vertex in P[r].
+// `on`: this lane really steps body b (false for the right-leg half while the left-leg half steps the Body)
+template <class EV, int R>
+__device__ __forceinline__ void integrate_step(const EV& e, bool on, int b, int q, int nq, float dt, float2 (&P)[R]) {
   // StepLinearVelocity: v += a * dt (gravity (0, 980), Walker.cs:45); Skeleton.Move(v * dt)
   float2 v = V2(e, kV2Vel + b);
   v = vadd(v, vmul(mk2(0.0f, 980.0f), dt));
@@ -791,22 +802,29 @@ __device__ __forceinline__ void body_step(EV& e, bool on, int b, float dt, wb_pa
   const float2 cen = vadd(V2(e, kV2Cen + b), d);
   lanes_sync<EV::L>();  // all reads of the old centroid / velocity / angle are done
 #pragma unroll
-  for (int i0 = 0; i0 < 6; i0 += G) {
-    const int i = i0 + e.gsub;
+  for (int r = 0; r < R; r++) {
+    const int i = r * nq + q;
+    P[r] = mk2(0.0f, 0.0f);
     if (i < 6 && on) {
       // Move then Rotate (Vector2.Transform(p - centroid, R) + centroid, Skeleton.cs:93)
       float2 p = vadd(V2(e, b * 6 + i), d);
       p = vsub(p, cen);
       const float2 t = vrotate(p, m11, m12);
-      V2(e, b * 6 + i) = vadd(t, cen);
+      P[r] = vadd(t, cen);
+      V2(e, b * 6 + i) = P[r];
     }
   }
-  if (e.gsub == 0 && on) {
+  if (q == 0 && on) {
     V2(e, kV2Cen + b) = cen;
     V2(e, kV2Vel + b) = v;
     F1(e, kFAngle + b) = ang;
   }
   lanes_sync<EV::L>();
+}
+
+// The collision half: RigidBody.ResolveCollisions of body b
+template <class EV, int G, bool TRACE>
+__device__ __forceinline__ void resolve_candidates(EV& e, bool on, int b, wb_pair_trace* tr_base) {
   // ResolveCollisions: candidates in Environment._rigidBodies order, skipping self and associated bodies (Walker.cs:204-208):
   // a leg segment meets the other segment of its own leg and the floor; the Body only the floor.  The floor comes first in the
   // list after the first Reset (Walker.cs:212-223).  Three uniform phases keep a warp whose environments disagree on the list
@@ -825,6 +843,59 @@ __device__ __forceinline__ void body_step(EV& e, bool on, int b, float dt, wb_pa
       if (__any_sync(kFull, want))
         resolve_pair<EV, G, TRACE, true>(e, want, b, FLOOR, (TRACE && tr_base) ? tr_base + slot + ((b == BODY || floor_first) ? 0 : 1) : nullptr);
     }
+  }
+}
+
+template <class EV, int G, bool TRACE>
+__device__ __forceinline__ void body_step(EV& e, bool on, int b, float dt, wb_pair_trace* tr_base) {
+  float2 P[(6 + G - 1) / G];
+  integrate_step(e, on, b, e.gsub, G, dt, P);
+  resolve_candidates<EV, G, TRACE>(e, on, b, tr_base);
+}
+
+// The body sweep of the leg split (LEGS = 2) with G >= 4 lanes per half in TWO slots instead of three: the Body shares no
+// mutable state with either leg during the sweep (it only meets the floor), so it needs no slot of its own.
+//   slot 0  integrate LLL on lanes 0..H-1 of the left half, the Body on lanes H..G-1 and RLL on the right half in ONE pass (one
+//           rotz on the chain); test the Body's bounding box against the floor on its new vertices; resolve the Body-floor
+//           pair only in a warp where that test hits (a Body on the floor ends the episode, so this is rare); then LLL's and
+//           RLL's candidates
+//   slot 1  LLU on the left half, RLU on the right half
+// Every body still meets its candidates in list order with the values the sequential sweep gives it, so the result is the
+// sequential one bit for bit.  -DWB_BODY_SLOT=1 builds the three-slot sweep instead (same-box A/B).  With G = 2 (4 lanes per
+// walker) the left half would move each of LLL and the Body on one lane in six rounds instead of three: measured slower
+// (contact_stress +2 %), so that layout keeps the three-slot sweep.
+template <class EV, int G, bool TRACE>
+__device__ __forceinline__ void legs_sweep(EV& e, bool left, float dt, wb_pair_trace* tr_base) {
+  static_assert(G >= 4, "two or more lanes per body in slot 0");
+  constexpr int H = G / 2;            // lanes per body on the left half in slot 0
+  constexpr int R = (6 + H - 1) / H;  // vertex rounds
+  const int base = e.gshift - (left ? 0 : G);  // the walker's first lane
+#pragma unroll 1
+  for (int k = 0; k < 2; k++) {
+    const bool body_lane = k == 0 && left && e.gsub >= H;
+    const int seg = left ? (k == 0 ? LLL : LLU) : (k == 0 ? RLL : RLU);
+    float2 P[R];
+    integrate_step(e, e.live, body_lane ? BODY : seg, body_lane ? e.gsub - H : e.gsub, (k == 0 && left) ? H : G, dt, P);
+    if (k == 0) {
+      // BoundingBox.IsColliding(Body, floor) (Skeleton.cs:133-140) on the new vertices: slot i is P[i / H] of body lane i mod H
+      float2 Q[6];
+#pragma unroll
+      for (int i = 0; i < 6; i++) {
+        Q[i].x = __shfl_sync(kFull, P[i / H].x, base + H + i % H);
+        Q[i].y = __shfl_sync(kFull, P[i / H].y, base + H + i % H);
+      }
+      float2 mn, mx;
+      aabb6(Q, mn, mx);
+      const unsigned hits = __ballot_sync(kFull, body_lane && e.live && aabb_hit(mn, mx, e.fl->bb_min, e.fl->bb_max));
+      const bool body_hit = ((hits >> base) & ((1u << G) - 1u)) != 0u;  // on every lane of the walker
+      if (body_hit) e.flags |= 1 << BODY;  // if (body._isFloor) Collided = true  (before SAT: RigidBody.cs:75)
+      wb_pair_trace* tr = (TRACE && tr_base) ? tr_base + 4 : nullptr;  // the Body's one candidate, the floor
+      if (TRACE) {
+        if (tr && e.live && left && e.gsub == 0 && !body_hit) *tr = pair_trace_no_sat(FLOOR, false);
+      }
+      if (hits != 0u) resolve_pair<EV, G, TRACE, true, -1, true>(e, left && body_hit, left ? BODY : RLL, FLOOR, tr);
+    }
+    resolve_candidates<EV, G, TRACE>(e, e.live, seg, tr_base);
   }
 }
 
@@ -850,8 +921,11 @@ __device__ __forceinline__ int record_word(int f) {
   return kV2Count * E * 2 + (f - 78) * E;
 }
 
+// 16 resident warps per SM for L = 16 as well (at most 128 registers): a warp's registers come from ONE of the four SM
+// sub-partitions (16 K each), so 129-160 registers leave 3 warps per sub-partition, and 4096 walkers with 16 lanes (2048
+// warps) no longer fit one wave
 template <int L, int LEGS, bool TRACE>
-__global__ void __launch_bounds__(32, (L <= 4) ? 16 : 8) physics_lanes_kernel(const PhysicsParams p) {
+__global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lanes_kernel(const PhysicsParams p) {
   static_assert(LEGS == 1 || (LEGS == 2 && L >= 2), "the leg split needs at least two lanes per environment");
   constexpr int E = 32 / L;
   __shared__ __align__(16) float s_state[(kV2Count * 2 + kFCount) * E];
@@ -990,10 +1064,14 @@ __global__ void __launch_bounds__(32, (L <= 4) ? 16 : 8) physics_lanes_kernel(co
         const int leg = e.sub / G;
         e.gsub = e.sub % G;
         e.gshift = col * L + leg * G;
+        if constexpr (G >= 4 && !WB_BODY_SLOT) {
+          legs_sweep<EV, G, TRACE>(e, leg == 0, dt, pt);
+        } else {  // three slots: (LLL | RLL), (LLU | RLU), (Body | idle)  (G <= 2, or -DWB_BODY_SLOT=1)
 #pragma unroll 1
-        for (int k = 0; k < 3; k++) {
-          const bool on = e.live && (leg == 0 || k < 2);
-          body_step<EV, G, TRACE>(e, on, leg == 0 ? k : (k < 2 ? RLL + k : RLU), dt, pt);
+          for (int k = 0; k < 3; k++) {
+            const bool on = e.live && (leg == 0 || k < 2);
+            body_step<EV, G, TRACE>(e, on, leg == 0 ? k : (k < 2 ? RLL + k : RLU), dt, pt);
+          }
         }
         e.gsub = e.sub;
         e.gshift = col * L;
