@@ -30,6 +30,7 @@
 // as the reference's C# (SURVEY.md Appendix A/C).  Bit-exact against the oracle.  There is no CPU path.
 #include <cstdio>
 #include <cstdlib>
+#include <type_traits>
 #include "physics.cuh"
 #include "physics_math.cuh"
 
@@ -50,6 +51,7 @@ constexpr unsigned kFull = 0xFFFFFFFFu;
 
 #ifdef WB_PHASE_PROFILE
 // experiment builds only (scripts/build_variant.sh prof -DWB_PHASE_PROFILE): cycle accounting of the compacting kernel
+// (scripts/phase_profile.py) and of the lanes kernel (scripts/lanes_profile.py)
 __device__ unsigned long long g_prof[24];
 __device__ __forceinline__ long long prof_clock() {
   long long t;
@@ -57,6 +59,10 @@ __device__ __forceinline__ long long prof_clock() {
   return t;
 }
 __device__ long long g_prof_sat_scratch;  // (unused; keeps the symbol table stable)
+// lanes kernel: clock64 cycles of each CTA (one warp) of the last launch: entry to the first substep, the substep loop,
+// observe + write-back (3 per CTA, CTAs beyond kLanesProfCtas are not recorded); read with wb_lanes_prof_read
+constexpr int kLanesProfCtas = 1 << 16;
+__device__ unsigned long long g_lanes_prof[3 * kLanesProfCtas];
 #endif
 
 
@@ -921,6 +927,53 @@ __device__ __forceinline__ int record_word(int f) {
   return kV2Count * E * 2 + (f - 78) * E;
 }
 
+// a walker's inputs besides its record, staged in shared memory with the record (physics_lanes_kernel)
+struct __align__(16) WalkerInputs {
+  float4 actions;
+  float torque[4];
+  float2 pos;
+  int32_t flags, steps;
+  uint32_t mat_words[2];  // the aligned words of walker_mat / floor_mat that hold this walker's bytes
+};
+
+template <int V> struct FloatVec;
+template <> struct FloatVec<1> { using T = float; };
+template <> struct FloatVec<2> { using T = float2; };
+template <> struct FloatVec<4> { using T = float4; };
+
+// The CTA's E records as whole aligned pieces: each of the 39 float2 slot rows is one run of 2E floats in HBM
+// (state_index) and in s_state (record_word), each of the 10 float rows (78..87) one run of E floats.  Calls
+// fn(HBM float offset, s_state float offset, first column, floats per column, std::integral_constant<int, V>) for the
+// pieces of this lane: V = 4 floats (16 B) where the run allows it.  Every piece of the CTA lies inside the padded rows
+// (kEnvPad is a multiple of E).  The loops have compile-time trip counts, so they unroll and every piece is in flight
+// before any is consumed.
+template <int E, class F>
+__device__ __forceinline__ void for_record_pieces(int lane, int env0, int n_pad, F&& fn) {
+  constexpr int VA = 2 * E < 4 ? 2 * E : 4, PA = 2 * E / VA, NA = kStateSlots2 * PA;
+  constexpr int VB = E < 4 ? E : 4, PB = E / VB, NB = kFCount * PB;
+#pragma unroll
+  for (int j = 0; j < (NA + 31) / 32; j++) {
+    const int i = j * 32 + lane, s2 = i / PA, k = i % PA;
+    if (NA % 32 == 0 || i < NA)
+      fn(((size_t)s2 * n_pad + env0) * 2 + k * VA, (s2 + (s2 >= 17 ? 1 : 0)) * 2 * E + k * VA, k * VA / 2, 2,
+         std::integral_constant<int, VA>());
+  }
+#pragma unroll
+  for (int j = 0; j < (NB + 31) / 32; j++) {
+    const int i = j * 32 + lane, r = i / PB, k = i % PB;
+    if (NB % 32 == 0 || i < NB)
+      fn((size_t)(78 + r) * n_pad + env0 + k * VB, kV2Count * 2 * E + r * E + k * VB, k * VB, 1, std::integral_constant<int, VB>());
+  }
+}
+
+// cp.async of one aligned piece of B = 4, 8 or 16 bytes, global -> shared; complete for this thread after cp_async_wait_all
+template <int B>
+__device__ __forceinline__ void cp_async(float* smem, const float* gmem) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem), "n"(B)
+               : "memory");
+}
+__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
+
 // 16 resident warps per SM for L = 16 as well (at most 128 registers): a warp's registers come from ONE of the four SM
 // sub-partitions (16 K each), so 129-160 registers leave 3 warps per sub-partition, and 4096 walkers with 16 lanes (2048
 // warps) no longer fit one wave
@@ -930,28 +983,12 @@ __global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lane
   constexpr int E = 32 / L;
   __shared__ __align__(16) float s_state[(kV2Count * 2 + kFCount) * E];
   __shared__ FloorConst s_floor;
+  __shared__ WalkerInputs s_in[E];
   const int lane = threadIdx.x;
   const int env0 = blockIdx.x * E;
-
-  // ---- stage the E records (all 32 lanes share the loads: SoA rows are contiguous over envs) and the floor constants
-  for (int w = lane; w < (int)(sizeof(FloorConst) / 4); w += 32)
-    reinterpret_cast<uint32_t*>(&s_floor)[w] = reinterpret_cast<const uint32_t*>(&c_floor)[w];
-  // (x, y) of a point are adjacent in HBM: the E walkers' share of a float2 slot is one run of 2E floats
-  for (int idx = lane; idx < 88 * E; idx += 32) {
-    int f, c;
-    if (idx < 78 * E) {
-      const int slot = idx / (2 * E), r = idx % (2 * E);
-      c = r >> 1;
-      f = 2 * slot + (r & 1);
-    } else {
-      f = 78 + (idx - 78 * E) / E;
-      c = idx % E;
-    }
-    const int env = env0 + c;
-    const float v = (env < p.n) ? p.state[state_index(f, env, p.n_pad)] : c_init_state[f];
-    s_state[record_word<E>(f) + (f < 78 ? 2 * c : c)] = v;
-  }
-  __syncwarp();
+#ifdef WB_PHASE_PROFILE
+  const long long t_entry = prof_clock();
+#endif
 
   using EV = Env<L, E>;
   EV e;
@@ -965,28 +1002,72 @@ __global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lane
   e.gshift = col * L;
   e.live = env < p.n;
   const int envc = e.live ? env : 0;  // dead lanes shadow env 0 read-only (they never store)
-  if (e.sub == 0) V2(e, BODY * 6 + 5) = V2(e, BODY * 6);
   float* torque_rows = p.state + (size_t)88 * p.n_pad + envc;
 
-  e.flags = p.flags[envc];
-  int steps = p.steps[envc];
-  {
-    const Material mw = c_materials[p.walker_mat[envc]];
-    const Material mf = c_materials[p.floor_mat[envc]];
-    set_materials(e, mw, mf);
+  // ---- stage the E records and each walker's inputs with every load in flight at once, so that this prologue costs one
+  // memory round trip before the first substep rather than one per load.  Everything goes to shared memory by cp.async and
+  // is waited for once (plain loads issued here would be scheduled behind the wait).  The record's rows are shared by all
+  // 32 lanes (SoA rows are contiguous over envs); lane 0 of each walker fetches that walker's scalars, and Walker.TakeActions'
+  // four joint torques (they stay in HBM) and actions.
+  for_record_pieces<E>(lane, env0, p.n_pad, [&](size_t g, int s, int, int, auto v) {
+    cp_async<decltype(v)::value * 4>(s_state + s, p.state + g);
+  });
+  WalkerInputs& in = s_in[col];
+  if (e.sub == 0) {
+    cp_async<4>(reinterpret_cast<float*>(&in.flags), reinterpret_cast<const float*>(p.flags + envc));
+    cp_async<4>(reinterpret_cast<float*>(&in.steps), reinterpret_cast<const float*>(p.steps + envc));
+    cp_async<4>(&in.pos.x, p.pos + envc);
+    cp_async<4>(&in.pos.y, p.pos + p.n_pad + envc);
+    // the material bytes arrive as the aligned word that holds them (the rows are padded to kEnvPad walkers)
+    cp_async<4>(reinterpret_cast<float*>(&in.mat_words[0]), reinterpret_cast<const float*>(p.walker_mat + (envc & ~3)));
+    cp_async<4>(reinterpret_cast<float*>(&in.mat_words[1]), reinterpret_cast<const float*>(p.floor_mat + (envc & ~3)));
+    if (p.phases & kPhaseTakeActions) {
+#pragma unroll
+      for (int k = 0; k < 4; k++) cp_async<4>(&in.torque[k], torque_rows + (size_t)k * p.n_pad);
+      if (e.live) cp_async<16>(reinterpret_cast<float*>(&in.actions), p.actions + (size_t)env * 4);
+    }
   }
-  float2 pos = mk2(p.pos[envc], p.pos[p.n_pad + envc]);
+  constexpr int kFloorWords = sizeof(FloorConst) / 4;
+#pragma unroll
+  for (int j = 0; j < (kFloorWords + 31) / 32; j++) {
+    const int w = j * 32 + lane;
+    if (w < kFloorWords) reinterpret_cast<uint32_t*>(&s_floor)[w] = reinterpret_cast<const uint32_t*>(&c_floor)[w];
+  }
+  cp_async_wait_all();
+  __syncwarp();
+  e.flags = in.flags;
+  int steps = in.steps;
+  float2 pos = in.pos;
+  {
+    const int byte = 8 * (envc & 3);
+    set_materials(e, c_materials[(in.mat_words[0] >> byte) & 0xFFu], c_materials[(in.mat_words[1] >> byte) & 0xFFu]);
+  }
+
+  // the fresh walker record into this lane's column, shared by the walker's L lanes (88 / L words per lane instead of 88 on
+  // one lane; the loop stays rolled to keep the register count); the caller syncs the warp before the column is read
+  auto write_initial_column = [&]() {
+#pragma unroll 1
+    for (int j = 0; j < (88 + L - 1) / L; j++) {
+      const int f = j * L + e.sub;
+      if (88 % L == 0 || f < 88) s_state[record_word<E>(f) + (f < 78 ? 2 * col : col)] = c_init_state[f];
+    }
+  };
+  // the columns of walkers past n (the last CTA only) hold the fresh walker record, as a reset would leave it
+  if (!e.live) write_initial_column();
+  __syncwarp();
+  if (e.sub == 0) V2(e, BODY * 6 + 5) = V2(e, BODY * 6);
   __syncwarp();
 
   // Walker.Reset + CreateCreature: fresh walker record (constants computed on the host with the reference's formulas)
   auto write_initial_record = [&](bool on) {
     if (!__any_sync(kFull, on)) return;
     __syncwarp();
+    if (on) write_initial_column();
+    __syncwarp();
     if (on && e.sub == 0) {
-#pragma unroll 1
-      for (int f = 0; f < 88; f++) s_state[record_word<E>(f) + (f < 78 ? 2 * col : col)] = c_init_state[f];
       V2(e, BODY * 6 + 5) = V2(e, BODY * 6);
-      for (int k = 0; k < 4; k++) torque_rows[(size_t)k * p.n_pad] = c_init_state[88 + k];
+#pragma unroll
+      for (int k = 0; k < 4; k++) torque_rows[(size_t)k * p.n_pad] = in.torque[k] = c_init_state[88 + k];
     }
     __syncwarp();
   };
@@ -1005,14 +1086,13 @@ __global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lane
   if (p.phases & kPhaseTakeActions) {
     // Matrix.Clip (Matrix.cs:377-405), Walker.TakeActions (Walker.cs:66-75), Joint.SetTorque (Joint.cs:56-61)
     if (e.live && e.sub == 0) {
-      const float4 a4 = *reinterpret_cast<const float4*>(p.actions + (size_t)env * 4);
-      const float act[4] = {a4.x, a4.y, a4.z, a4.w};
+      const float act[4] = {in.actions.x, in.actions.y, in.actions.z, in.actions.w};
 #pragma unroll
       for (int k = 0; k < 4; k++) {
         float a = act[k];
         if (a >= 1.0f) a = 1.0f;
         else if (a <= -1.0f) a = -1.0f;
-        const float change = fsub(a, torque_rows[(size_t)k * p.n_pad]);
+        const float change = fsub(a, in.torque[k]);
         torque_rows[(size_t)k * p.n_pad] = a;
         const int bodyB = (k == 0) ? LLU : (k == 1) ? RLU : (k == 2) ? LLL : RLL;  // Walker.cs:182-185
         F1(e, kFOmega + bodyB) = fadd(F1(e, kFOmega + bodyB), fmul(change, 5.0f));
@@ -1021,6 +1101,9 @@ __global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lane
     __syncwarp();
   }
 
+#ifdef WB_PHASE_PROFILE
+  const long long t_substeps = prof_clock();
+#endif
   if (p.phases & kPhaseStepObjects) {
     const float dt = fdiv(p.dt, (float)p.iterations);  // deltaTime /= Hyperparameters.Iterations
 #pragma unroll 1
@@ -1079,6 +1162,9 @@ __global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lane
     }
     if (LEGS == 2) e.flags |= __shfl_xor_sync(kFull, e.flags, L / LEGS);  // each half latched its own bodies' Collided bits
   }
+#ifdef WB_PHASE_PROFILE
+  const long long t_observe = prof_clock();
+#endif
 
   if (p.phases & kPhaseObserve) {
     // Walker.Update, Walker.cs:49-54
@@ -1123,19 +1209,27 @@ __global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lane
     p.pos[p.n_pad + env] = pos.y;
   }
   __syncwarp();
-  // ---- write the records back (same coalesced pattern)
-  for (int idx = lane; idx < 88 * E; idx += 32) {
-    int f, c;
-    if (idx < 78 * E) {
-      const int slot = idx / (2 * E), r = idx % (2 * E);
-      c = r >> 1;
-      f = 2 * slot + (r & 1);
+  // ---- write the records back in the same pieces; a piece that reaches past n (the last CTA only) stores float by float
+  const bool all_live = env0 + E <= p.n;
+  for_record_pieces<E>(lane, env0, p.n_pad, [&](size_t g, int s, int c0, int per_col, auto v) {
+    constexpr int V = decltype(v)::value;
+    using T = typename FloatVec<V>::T;
+    if (all_live) {
+      *reinterpret_cast<T*>(p.state + g) = *reinterpret_cast<const T*>(s_state + s);
     } else {
-      f = 78 + (idx - 78 * E) / E;
-      c = idx % E;
+#pragma unroll
+      for (int j = 0; j < V; j++)
+        if (env0 + c0 + j / per_col < p.n) p.state[g + j] = s_state[s + j];
     }
-    if (env0 + c < p.n) p.state[state_index(f, env0 + c, p.n_pad)] = s_state[record_word<E>(f) + (f < 78 ? 2 * c : c)];
+  });
+#ifdef WB_PHASE_PROFILE
+  if (lane == 0 && blockIdx.x < kLanesProfCtas) {
+    const long long t_end = prof_clock();
+    g_lanes_prof[3 * blockIdx.x + 0] = t_substeps - t_entry;
+    g_lanes_prof[3 * blockIdx.x + 1] = t_observe - t_substeps;
+    g_lanes_prof[3 * blockIdx.x + 2] = t_end - t_observe;
   }
+#endif
 }
 
 // test hook: compares rcp_sqrt_rn(s) with __frcp_rn(__fsqrt_rn(s)) for every bit pattern in [first, first + count)
@@ -2008,6 +2102,12 @@ extern "C" int wb_prof_read(unsigned long long* out24, int reset) {
     cudaMemcpyToSymbol(pl::g_prof, z, sizeof(z));
   }
   return 0;
+}
+// the lanes kernel's last launch: 3 cycle counts per CTA for the first `ctas` CTAs (pl::g_lanes_prof)
+extern "C" int wb_lanes_prof_read(unsigned long long* out, int ctas) {
+  if (ctas < 0 || ctas > pl::kLanesProfCtas) return 1;
+  cudaDeviceSynchronize();
+  return cudaMemcpyFromSymbol(out, pl::g_lanes_prof, sizeof(unsigned long long) * 3 * ctas) != cudaSuccess;
 }
 #endif
 
