@@ -379,31 +379,44 @@ int32_t wb_policy_launch_count(const wb_policy* p, int64_t* count_out);
 /* ---- populations: one PPO brain per walker ----
  * In the reference every walker owns its agent (new Walker() builds its own PPOAgent(12, 4), Walker.cs:25-34) and trains it on each
  * of its own episodes as soon as the episode ends (Environment.cs:91,157-164 -> PPOAgent.Train(Trajectory), PPOAgent.cs:147-172).
- * A population holds P such agents with the reference's default networks (Hyperparameters.cs:91-92; 6 149 parameters): each has
- * its own weights, Adam m / v, per-dense-layer step counters and wb_hyperparams (alpha, beta1, beta2, Adam epsilon, gamma, lambda,
- * clip epsilon, log_std, use_gae, normalize_advantages, batch_size).  Agent a behaves exactly as one wb_policy on kernel variant 1
- * with the same weights and hyper-parameters: acting and training give the same bits.  Agents that a call does not name are not
- * touched.  Weights start at zero (load them with wb_population_set_weights).  The longest episode trained is 1 024 steps
- * (WB_ERR_UNSUPPORTED beyond). */
+ * A population holds P such agents, all with the same two networks: the reference's defaults (Hyperparameters.cs:91-92; 6 149
+ * parameters, wb_population_create) or any pair the DSL describes (wb_population_create_net).  Each agent has its own weights,
+ * Adam m / v, per-dense-layer step counters and wb_hyperparams (alpha, beta1, beta2, Adam epsilon, gamma, lambda, clip epsilon,
+ * log_std, use_gae, normalize_advantages, batch_size).  Agent a behaves exactly as one wb_policy with the same networks, weights
+ * and hyper-parameters -- on kernel variant 1 for the default networks, on the any-topology kernel (variant 2) otherwise: acting
+ * and training give the same bits.  Agents that a call does not name are not touched.  Weights start at zero (load them with
+ * wb_population_set_weights).  The longest episode trained is 1 024 steps (WB_ERR_UNSUPPORTED beyond).  Below, n_actor /
+ * n_critic / n_dense are the population's parameter and dense-layer counts (wb_population_num_params; 5 252 / 897 / 3 + 2 for the
+ * defaults), state / act its state and action sizes (12 / 4). */
 typedef struct wb_population wb_population;
 /* new PPOAgent(12, 4) x n_agents (PPOAgent.cs:23-37); hp = [n_agents] hyper-parameters or NULL (the defaults for every agent).
  * n_agents < 1 or a batch_size < 1: WB_ERR_INVALID */
 int32_t wb_population_create(int32_t n_agents, const wb_hyperparams* hp, wb_population** out);
+/* new PPOAgent(state_size, action_size) x n_agents with the networks of the layer lists (as wb_policy_create: the same checks and
+ * statuses for a network outside the limits).  The default lists give the population of wb_population_create; other networks run
+ * the any-topology population kernels.  A network whose layer caches and one episode's arrays exceed a CTA's shared memory:
+ * WB_ERR_UNSUPPORTED. */
+int32_t wb_population_create_net(int32_t n_agents, int32_t state_size, int32_t action_size, const int32_t* actor_kinds,
+                                 const int32_t* actor_sizes, int32_t actor_layers, const int32_t* critic_kinds, const int32_t* critic_sizes,
+                                 int32_t critic_layers, const wb_hyperparams* hp, wb_population** out);
+/* parameters of each agent's actor (which = 0) or critic (which = 1) */
+int32_t wb_population_num_params(const wb_population* pop, int32_t which, int32_t* n_out);
 int32_t wb_population_destroy(wb_population* pop);
 int32_t wb_population_set_stream(wb_population* pop, void* cuda_stream);
 int32_t wb_population_sync(wb_population* pop);
 /* number of kernel launches this handle has issued */
 int32_t wb_population_launch_count(const wb_population* pop, int64_t* count_out);
-/* agent a's flat parameters [6149] = actor | critic, each in the DenseLayer.Save order (DenseLayer.cs:73-79) */
+/* agent a's flat parameters [n_actor + n_critic] = actor | critic, each in the DenseLayer.Save order (DenseLayer.cs:73-79) */
 int32_t wb_population_set_weights(wb_population* pop, int32_t agent, const float* flat_host);
 int32_t wb_population_get_weights(wb_population* pop, int32_t agent, float* flat_host);
-/* agent a's gradient buffer [6149] (the last mini-batch it trained, as wb_policy_get_grads) */
+/* agent a's gradient buffer [n_actor + n_critic] (the last mini-batch it trained, as wb_policy_get_grads) */
 int32_t wb_population_get_grads(wb_population* pop, int32_t agent, float* flat_host);
-/* agent a's Adam moments m / v [6149] and the step counters [5] of its dense layers (actor L1-L3, critic L1-L2; DenseLayer.cs:15-20) */
+/* agent a's Adam moments m / v [n_actor + n_critic] and the step counters [n_dense] of its dense layers (actor layers, then critic
+ * layers; DenseLayer.cs:15-20) */
 int32_t wb_population_get_adam(wb_population* pop, int32_t agent, float* m_host, float* v_host, int32_t* steps_host);
 /* PPOAgent.SampleActions (PPOAgent.cs:381-398) for n == P walkers, walker w with agent w, with the two System.Random uniforms of
- * each Box-Muller draw injected (NormalDistribution.cs:12-32): states [n][12], uniforms [n][4][2] -> actions, logp [n][4], mean
- * [n][4] or NULL.  Row w equals wb_policy_sample of agent w. */
+ * each Box-Muller draw injected (NormalDistribution.cs:12-32): states [n][state], uniforms [n][act][2] -> actions, logp [n][act],
+ * mean [n][act] or NULL.  Row w equals wb_policy_sample of agent w. */
 int32_t wb_population_sample(wb_population* pop, int32_t n, const float* states_host, const float* uniforms_host, float* actions_host,
                              float* logp_host, float* mean_host);
 /* the same from the Philox stream (seed, step) of wb_policy_act_dev (counter (walker, action dim, step)), enqueue only; mean_dev
@@ -422,7 +435,7 @@ int32_t wb_population_train_trajectories(wb_population* pop, int32_t n_traj, con
                                          const float* rewards_host, const int32_t* batch_index_host, float* values_host,
                                          float* returns_host, float* advantages_host, float* losses_host, int32_t* skipped_host);
 /* The device form for lockstep walkers (Environment.Update -> TrainNetworks -> Reset, Environment.cs:64-92,157-173): the
- * rollout arrays are a time-major ring of ring_rows rows x columns (states [R][C][12], actions / logp [R][C][4], rewards /
+ * rollout arrays are a time-major ring of ring_rows rows x columns (states [R][C][state], actions / logp [R][C][act], rewards /
  * values / returns / advantages [R][C]).  items_host [n_items][4] = (agent, column, t0, length): the episode's step i is row
  * ((t0 + i) mod ring_rows) * columns + column.  Every agent trains its items in list order, one CTA per agent with work.
  * batch_index_dev: caller-drawn indices in the layout of wb_population_train_trajectories, or NULL: the kernel draws them --

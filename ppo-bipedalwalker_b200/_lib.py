@@ -152,6 +152,8 @@ def lib() -> C.CDLL:
         "wb_returns_advantages": (C.c_int32, [vp, C.c_int32, vp, vp, vp, vp]),
         "wb_debug_tc_gemm": (C.c_int32, [C.c_int32] * 6 + [vp, vp, vp]),
         "wb_population_create": (C.c_int32, [C.c_int32, hpp, C.POINTER(vp)]),
+        "wb_population_create_net": (C.c_int32, [C.c_int32, C.c_int32, C.c_int32, vp, vp, C.c_int32, vp, vp, C.c_int32, hpp, C.POINTER(vp)]),
+        "wb_population_num_params": (C.c_int32, [vp, C.c_int32, ip]),
         "wb_population_destroy": (C.c_int32, [vp]),
         "wb_population_set_stream": (C.c_int32, [vp, vp]),
         "wb_population_sync": (C.c_int32, [vp]),

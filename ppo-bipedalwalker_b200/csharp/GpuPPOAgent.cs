@@ -29,19 +29,7 @@ public sealed class GpuPPOAgent : IDisposable
     {
         _stateSize = stateSize;
         _actionSize = actionSize;
-        const string defaultCritic = "Input |64| (LeakyReLU) |1| Output", defaultActor = "Input |64| (LeakyReLU) |64| (LeakyReLU) |4| (TanH) Output";
-        if (!TryParse(Hyperparameters.CriticNeuralNetwork, out var ck, out var cs) || cs.Last(s => s > 0) != 1)
-        {
-            ErrorLogger.LogError("Exception occurred while attempting to parse the critic neural network.");
-            Hyperparameters.CriticNeuralNetwork = defaultCritic;
-            TryParse(defaultCritic, out ck, out cs);
-        }
-        if (!TryParse(Hyperparameters.ActorNeuralNetwork, out var ak, out var asz) || asz.Last(s => s > 0) != actionSize)
-        {
-            ErrorLogger.LogError("Exception occurred while attempting to parse the actor neural network.");
-            Hyperparameters.ActorNeuralNetwork = defaultActor;
-            TryParse(defaultActor, out ak, out asz);
-        }
+        ParseNetworks(actionSize, out var ak, out var asz, out var ck, out var cs);
         var hp = WbHyperparams.FromStatics();
         Wb.Ok(Wb.wb_init(0), "wb_init");
         Wb.Ok(Wb.wb_policy_create(stateSize, actionSize, ak, asz, ak.Length, ck, cs, ck.Length, ref hp, out _policy), "wb_policy_create");
@@ -54,6 +42,25 @@ public sealed class GpuPPOAgent : IDisposable
     }
 
     internal IntPtr Handle => _policy;
+
+    // PPOAgent.CreateNetworks (PPOAgent.cs:41-93): parse Hyperparameters.CriticNeuralNetwork / ActorNeuralNetwork; a string that does
+    // not parse, or whose last dense layer is not 1 / actionSize wide, is logged and replaced by the default network
+    internal static void ParseNetworks(int actionSize, out int[] ak, out int[] asz, out int[] ck, out int[] cs)
+    {
+        const string defaultCritic = "Input |64| (LeakyReLU) |1| Output", defaultActor = "Input |64| (LeakyReLU) |64| (LeakyReLU) |4| (TanH) Output";
+        if (!TryParse(Hyperparameters.CriticNeuralNetwork, out ck, out cs) || cs.Last(s => s > 0) != 1)
+        {
+            ErrorLogger.LogError("Exception occurred while attempting to parse the critic neural network.");
+            Hyperparameters.CriticNeuralNetwork = defaultCritic;
+            TryParse(defaultCritic, out ck, out cs);
+        }
+        if (!TryParse(Hyperparameters.ActorNeuralNetwork, out ak, out asz) || asz.Last(s => s > 0) != actionSize)
+        {
+            ErrorLogger.LogError("Exception occurred while attempting to parse the actor neural network.");
+            Hyperparameters.ActorNeuralNetwork = defaultActor;
+            TryParse(defaultActor, out ak, out asz);
+        }
+    }
 
     // PPOAgent.ParseLayers (PPOAgent.cs:96-143) -> kinds / sizes for wb_policy_create
     private static bool TryParse(string structure, out int[] kinds, out int[] sizes)
@@ -73,7 +80,7 @@ public sealed class GpuPPOAgent : IDisposable
         return k.Contains(Wb.Dense);
     }
 
-    private static void DenseShapes(int input, int[] kinds, int[] sizes, List<(int, int)> shapes)
+    internal static void DenseShapes(int input, int[] kinds, int[] sizes, List<(int, int)> shapes)
     {
         int width = input;
         for (int i = 0; i < kinds.Length; i++)
@@ -265,16 +272,23 @@ public sealed class GpuPPOAgent : IDisposable
     // are present replace the leading dense layers
     public void Load(string type)
     {
-        string[] contents = type == "critic" ? Hyperparameters.CriticWeights : Hyperparameters.ActorWeights;
-        string network = type == "critic" ? Hyperparameters.CriticNeuralNetwork : Hyperparameters.ActorNeuralNetwork;
-        var shapes = type == "critic" ? _criticDense : _actorDense;
         int which = type == "critic" ? 1 : 0;
-        if (contents.Length < 2 || contents[0] != network) return;
-        (bool ok, _) = NeuralNetwork.ValidateWeights(contents);
-        if (!ok || contents.Length - 1 > shapes.Count) return;
         Wb.wb_policy_num_params(_policy, which, out int count);
         var flat = new float[count];
         Wb.Ok(Wb.wb_policy_get_weights(_policy, which, flat), "wb_policy_get_weights");
+        if (LoadInto(type, type == "critic" ? _criticDense : _actorDense, flat))
+            Wb.Ok(Wb.wb_policy_set_weights(_policy, which, flat), "wb_policy_set_weights");
+    }
+
+    // the weights file of `type` (Hyperparameters.CriticWeights / ActorWeights) over one network's flat parameters; false: nothing loaded
+    internal static bool LoadInto(string type, List<(int outSize, int inSize)> shapes, float[] flat)
+    {
+        string[] contents = type == "critic" ? Hyperparameters.CriticWeights : Hyperparameters.ActorWeights;
+        string network = type == "critic" ? Hyperparameters.CriticNeuralNetwork : Hyperparameters.ActorNeuralNetwork;
+        if (contents.Length < 2 || contents[0] != network) return false;
+        (bool ok, _) = NeuralNetwork.ValidateWeights(contents);
+        if (!ok || contents.Length - 1 > shapes.Count) return false;
+        var loaded = (float[])flat.Clone();
         int p = 0;
         for (int l = 0; l < contents.Length - 1; l++)
         {
@@ -283,20 +297,21 @@ public sealed class GpuPPOAgent : IDisposable
             int wi = line.IndexOf("W", StringComparison.Ordinal) + 2, bi = line.IndexOf("B", StringComparison.Ordinal) + 2;
             float[] w = Array.ConvertAll(line.Substring(wi, bi - wi - 3).Split(), float.Parse);
             float[] b = Array.ConvertAll(line.Substring(bi).Split(), float.Parse);
-            if (w.Length < o * i || b.Length < o) return;           // Matrix.Load would throw (Matrix.cs:118-127)
-            Array.Copy(w, 0, flat, p, o * i);
+            if (w.Length < o * i || b.Length < o) return false;     // Matrix.Load would throw (Matrix.cs:118-127)
+            Array.Copy(w, 0, loaded, p, o * i);
             p += o * i;
-            Array.Copy(b, 0, flat, p, o);
+            Array.Copy(b, 0, loaded, p, o);
             p += o;
         }
-        Wb.Ok(Wb.wb_policy_set_weights(_policy, which, flat), "wb_policy_set_weights");
+        loaded.CopyTo(flat, 0);
+        return true;
     }
 
     public void Dispose() => Wb.wb_policy_destroy(_policy);
 }
 
-// One PPO brain per walker: P agents of the reference's default networks (Hyperparameters.cs:91-92) on one native handle
-// (wb_population_*).  In the reference every walker owns its PPOAgent (Walker.cs:25-34) and trains it on each of its own episodes
+// One PPO brain per walker: P agents with the networks of Hyperparameters.ActorNeuralNetwork / CriticNeuralNetwork (parsed, with
+// the reference's fallbacks, as GpuPPOAgent parses them) on one native handle (wb_population_*).  In the reference every walker owns its PPOAgent (Walker.cs:25-34) and trains it on each of its own episodes
 // (Environment.cs:91,157-164); agent a here is one GpuPPOAgent with its own weights, Adam state and step counters.  The
 // hyper-parameters are the statics at construction.  Xavier initialisation, the Box-Muller uniforms and CreateBatches are drawn
 // from System.Random in C#, as GpuPPOAgent draws them.
@@ -305,18 +320,25 @@ public sealed class GpuPopulation : IDisposable
     private readonly IntPtr _population;
     private readonly int _n;
     private readonly Random _random = new Random();
-    private static readonly List<(int outSize, int inSize)> ActorDense = new() { (64, Wb.Obs), (64, 64), (Wb.Act, 64) };
-    private static readonly List<(int outSize, int inSize)> CriticDense = new() { (64, Wb.Obs), (1, 64) };
+    private readonly List<(int outSize, int inSize)> _actorDense = new(), _criticDense = new();
 
+    // new PPOAgent(12, 4) per agent (PPOAgent.cs:23-37): the networks of the DSL strings, Xavier initialisation (critic first, then
+    // actor), then Load("critic") / Load("actor") when weights are set
     public GpuPopulation(int agents)
     {
         _n = agents;
+        GpuPPOAgent.ParseNetworks(Wb.Act, out var ak, out var asz, out var ck, out var cs);
         var hp = Enumerable.Repeat(WbHyperparams.FromStatics(), agents).ToArray();
         Wb.Ok(Wb.wb_init(0), "wb_init");
-        Wb.Ok(Wb.wb_population_create(agents, ref hp[0], out _population), "wb_population_create");
-        for (int a = 0; a < agents; a++)   // PPOAgent ctor: the critic's layers are created first, then the actor's (PPOAgent.cs:41-93)
+        Wb.Ok(Wb.wb_population_create_net(agents, Wb.Obs, Wb.Act, ak, asz, ak.Length, ck, cs, ck.Length, ref hp[0], out _population),
+              "wb_population_create_net");
+        GpuPPOAgent.DenseShapes(Wb.Obs, ak, asz, _actorDense);
+        GpuPPOAgent.DenseShapes(Wb.Obs, ck, cs, _criticDense);
+        for (int a = 0; a < agents; a++)
         {
-            float[] critic = GpuPPOAgent.Xavier(CriticDense), actor = GpuPPOAgent.Xavier(ActorDense);
+            float[] critic = GpuPPOAgent.Xavier(_criticDense), actor = GpuPPOAgent.Xavier(_actorDense);
+            GpuPPOAgent.LoadInto("critic", _criticDense, critic);
+            GpuPPOAgent.LoadInto("actor", _actorDense, actor);
             Wb.Ok(Wb.wb_population_set_weights(_population, a, actor.Concat(critic).ToArray()), "wb_population_set_weights");
         }
     }

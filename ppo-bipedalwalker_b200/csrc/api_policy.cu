@@ -62,24 +62,6 @@ static int32_t ensure_stage(wb_policy* p, size_t floats) {
   return WB_OK;
 }
 
-static bool is_default_topology(int32_t state_size, int32_t action_size, const int32_t* ak, const int32_t* as, int32_t al,
-                                const int32_t* ck, const int32_t* cs, int32_t cl) {
-  if (state_size != kIn || action_size != kAct || al != 6 || cl != 3) return false;
-  const int32_t want_ak[6] = {WB_DENSE, WB_LEAKYRELU, WB_DENSE, WB_LEAKYRELU, WB_DENSE, WB_TANH};
-  const int32_t want_as[6] = {kHid, 0, kHid, 0, kAct, 0};
-  for (int i = 0; i < 6; i++) {
-    if (ak[i] != want_ak[i]) return false;
-    if (ak[i] == WB_DENSE && as[i] != want_as[i]) return false;
-  }
-  const int32_t want_ck[3] = {WB_DENSE, WB_LEAKYRELU, WB_DENSE};
-  const int32_t want_cs[3] = {kHid, 0, 1};
-  for (int i = 0; i < 3; i++) {
-    if (ck[i] != want_ck[i]) return false;
-    if (ck[i] == WB_DENSE && cs[i] != want_cs[i]) return false;
-  }
-  return true;
-}
-
 static bool use_generic(const wb_policy* p) { return !p->default_topology || p->variant == 2; }
 
 static cudaError_t run_mlp(wb_policy* p, const MlpParams& m) {
@@ -133,43 +115,6 @@ static void fill_mlp_common(const wb_policy* p, MlpParams& m, int n, int mode) {
   m.batch_size = (float)p->hp.batch_size;
 }
 
-// PPOAgent.ParseLayers output (kinds / sizes) -> layer table; false when the DSL instance is outside what the kernels cover
-static bool build_net(int32_t input, const int32_t* kinds, const int32_t* sizes, int32_t n_layers, GenNet* net, const char** why) {
-  *net = GenNet{};
-  if (n_layers < 1 || n_layers > kGenMaxLayers) { *why = "a network holds 1..16 layers"; return false; }
-  if (input < 1 || input > kGenMaxWidth) { *why = "the state size must be 1..128"; return false; }
-  net->n_layers = n_layers;
-  net->input = input;
-  int width = input, cache = 0, off = 0;
-  for (int l = 0; l < n_layers; l++) {
-    GenLayer& L = net->L[l];
-    L.kind = kinds[l];
-    L.in = width;
-    L.cache_off = cache;
-    cache += width;
-    if (kinds[l] == WB_DENSE) {
-      if (sizes[l] < 1 || sizes[l] > kGenMaxWidth) { *why = "dense layer widths must be 1..128"; return false; }
-      L.out = sizes[l];
-      L.w_off = off;
-      off += L.out * L.in;
-      L.b_off = off;
-      off += L.out;
-      width = L.out;
-      net->n_dense++;
-    } else if (kinds[l] == WB_RELU || kinds[l] == WB_LEAKYRELU || kinds[l] == WB_TANH) {
-      L.out = width;
-    } else {
-      *why = "unknown layer kind";
-      return false;
-    }
-  }
-  if (net->n_dense < 1) { *why = "a network needs at least one dense layer"; return false; }
-  net->output = width;
-  net->n_params = off;
-  net->cache_floats = cache;
-  return true;
-}
-
 // a timed-out exchange leaves the ranks' weights out of step: refuse every later data-parallel update of this handle
 static int32_t comm_healthy(const wb_policy* p) {
   if (*reinterpret_cast<volatile uint32_t*>(p->h_comm_status) != 0u)
@@ -185,29 +130,22 @@ int32_t wb_policy_create(int32_t state_size, int32_t action_size, const int32_t*
                          const wb_hyperparams* hp, wb_policy** out) {
   WB_REQUIRE(out, "out is null");
   *out = nullptr;
-  WB_REQUIRE(actor_kinds && actor_sizes && critic_kinds && critic_sizes, "null layer list");
-  GenNet actor, critic;
-  const char* why = "";
-  if (!build_net(state_size, actor_kinds, actor_sizes, actor_layers, &actor, &why)) return fail(WB_ERR_UNSUPPORTED, "actor network: %s", why);
-  if (!build_net(state_size, critic_kinds, critic_sizes, critic_layers, &critic, &why)) return fail(WB_ERR_UNSUPPORTED, "critic network: %s", why);
-  // PPOAgent.CreateNetworks checks the two output sizes (PPOAgent.cs:78-92); the host shim falls back to the defaults like the reference
-  if (actor.output != action_size) return fail(WB_ERR_INVALID, "the actor's last dense layer must have action_size outputs (PPOAgent.cs:86)");
-  if (critic.output != 1) return fail(WB_ERR_INVALID, "the critic's last dense layer must have one output (PPOAgent.cs:78)");
-  if (action_size > 64) return fail(WB_ERR_UNSUPPORTED, "action_size must be 1..64");
-  if (actor.n_dense + critic.n_dense > kGenMaxDense) return fail(WB_ERR_UNSUPPORTED, "at most 32 dense layers in both networks together");
-  const int gen_ts = generic_tile_samples(actor, critic);
-  if (gen_ts == 0) return fail(WB_ERR_UNSUPPORTED, "the layer caches of one sample exceed shared memory (sum of layer widths too large)");
+  Networks nets;
+  if (int32_t rc = build_networks(state_size, action_size, actor_kinds, actor_sizes, actor_layers, critic_kinds, critic_sizes, critic_layers, &nets))
+    return rc;
+  const GenNet& actor = nets.actor;
+  const GenNet& critic = nets.critic;
   if (int32_t rc = require_device()) return rc;
   wb_policy* p = new (std::nothrow) wb_policy();
   WB_REQUIRE(p, "out of host memory");
-  p->default_topology = is_default_topology(state_size, action_size, actor_kinds, actor_sizes, actor_layers, critic_kinds, critic_sizes, critic_layers);
+  p->default_topology = nets.default_topology;
   p->actor = actor;
   p->critic = critic;
   p->n_actor = actor.n_params;
   p->n_critic = critic.n_params;
   p->n_total = actor.n_params + critic.n_params;
   p->grad_floats = (p->n_total + 3 + 3) / 4 * 4;
-  p->gen_ts = gen_ts;
+  p->gen_ts = nets.gen_ts;
   cudaGetDevice(&p->device);
   cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, p->device);
   if (hp) p->hp = *hp; else wb_hyperparams_default(&p->hp);
@@ -625,12 +563,7 @@ static cudaError_t adam_any(wb_policy* p) {
   g.m = p->d_m;
   g.v = p->d_v;
   g.n_params = p->n_total;
-  g.n_dense = p->actor.n_dense + p->critic.n_dense;
-  int k = 0;
-  for (int l = 0; l < p->actor.n_layers; l++)
-    if (p->actor.L[l].kind == WB_DENSE) g.layer_end[k++] = p->actor.L[l].b_off + p->actor.L[l].out;
-  for (int l = 0; l < p->critic.n_layers; l++)
-    if (p->critic.L[l].kind == WB_DENSE) g.layer_end[k++] = p->n_actor + p->critic.L[l].b_off + p->critic.L[l].out;
+  g.n_dense = generic_layer_ends(p->actor, p->critic, g.layer_end);
   g.alpha = p->hp.alpha;
   g.beta1 = p->hp.beta1;
   g.beta2 = p->hp.beta2;

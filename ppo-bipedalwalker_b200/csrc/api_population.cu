@@ -1,5 +1,6 @@
 // api_population.cu -- C ABI of a population of independent PPO agents (include/walker_b200.h, wb_population_*).  Compute is in
-// mlp.cu (population_act_kernel, population_episodes_kernel).
+// mlp.cu (population_act_kernel, population_episodes_kernel: the reference's default networks) and mlp_generic.cu
+// (population_generic_act_kernel, population_generic_episodes_kernel: any other network the DSL describes).
 #include <cmath>
 #include <cstring>
 #include <new>
@@ -10,19 +11,21 @@
 
 using namespace wb;
 
-namespace {
-constexpr int kDenseLayers = 5;  // actor L1, L2, L3, critic L1, L2
-}
-
 struct wb_population {
   int device = 0;
   cudaStream_t stream = nullptr;
   int n = 0;
   int64_t launches = 0;
+  Networks nets{};                  // default_topology: the default kernels; otherwise the any-topology ones
+  int state = kIn, action = kAct;
+  int n_total = kTotalParams;       // actor | critic parameters of one agent
+  int stride = kAgentStride;        // floats per agent row: n_total + 3 (loss sums, skipped) rounded up to a float4 multiple
+  int n_dense = 5;                  // dense layers of both networks (actor first)
+  int32_t layer_end[kGenMaxDense] = {};
   std::vector<wb_hyperparams> hp;
-  std::vector<int32_t> iterations;  // [n][5] DenseLayer._iteration per dense layer
+  std::vector<int32_t> iterations;  // [n][n_dense] DenseLayer._iteration per dense layer
   std::vector<int32_t> episodes;    // [n] episodes trained so far (counter of the device-drawn mini-batches)
-  float* d_params = nullptr;        // [n][kAgentStride] actor | critic
+  float* d_params = nullptr;        // [n][stride] actor | critic
   float* d_m = nullptr;
   float* d_v = nullptr;
   float* d_grads = nullptr;
@@ -70,7 +73,8 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
     if (L > kPopMaxLen) return fail(WB_ERR_UNSUPPORTED, "item %d: an episode of %d steps (at most %d)", i, L, kPopMaxLen);
     steps += (int64_t)epochs * (L / p->hp[a].batch_size);
   }
-  WB_REQUIRE(steps <= INT32_MAX / 10, "too many Adam steps for one call");
+  // (the correction table holds 2 * n_dense floats per Adam step)
+  WB_REQUIRE(steps <= INT32_MAX / (2 * p->n_dense), "too many Adam steps for one call");
   // CTAs: the agents with work, in order of first appearance; each trains its items in list order
   std::vector<int32_t> first_cta(p->n, -1);
   std::vector<PopCta> ctas;
@@ -85,7 +89,8 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
   for (size_t k = 1; k < ctas.size(); k++) ctas[k].first = ctas[k - 1].first + ctas[k - 1].count;
   const size_t cta_bytes = align16(sizeof(PopCta) * ctas.size());
   const size_t item_bytes = align16(sizeof(PopItem) * n_items);
-  const size_t tab_bytes = cta_bytes + item_bytes + sizeof(float) * 10 * (size_t)steps;
+  const int nd = p->n_dense;
+  const size_t tab_bytes = cta_bytes + item_bytes + sizeof(float) * 2 * nd * (size_t)steps;
   if (!p->tab_copied) WB_CUDA(cudaEventCreateWithFlags(&p->tab_copied, cudaEventDisableTiming));
   WB_CUDA(cudaEventSynchronize(p->tab_copied));  // (the previous call's upload has read the pinned copy)
   if (tab_bytes > p->tab_bytes) {
@@ -111,13 +116,13 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
     PopItem& it = tab_items[ctas[k].first + fill[k]++];
     it = PopItem{i, items[4 * i + 1], items[4 * i + 2], L, (int32_t)index_off, (int32_t)corr_off, p->episodes[a]++, 0};
     // DenseLayer.Adam bias corrections (float)(1 - Math.Pow(beta, t)) (DenseLayer.cs:127,142-145), as next_corrections computes them
-    int32_t* iter = &p->iterations[(size_t)a * kDenseLayers];
+    int32_t* iter = &p->iterations[(size_t)a * nd];
     for (int64_t s = 0; s < nb; s++) {
-      float* c = corr + 10 * (corr_off + s);
-      for (int l = 0; l < kDenseLayers; l++) {
+      float* c = corr + 2 * nd * (corr_off + s);
+      for (int l = 0; l < nd; l++) {
         iter[l] += 1;
         c[l] = (float)(1.0 - pow((double)p->hp[a].beta1, (double)iter[l]));
-        c[5 + l] = (float)(1.0 - pow((double)p->hp[a].beta2, (double)iter[l]));
+        c[nd + l] = (float)(1.0 - pow((double)p->hp[a].beta2, (double)iter[l]));
       }
     }
     index_off += nb * B;
@@ -148,16 +153,29 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
   t.columns = columns;
   t.epochs = epochs;
   t.seed = seed;
-  WB_CUDA(launch_population_episodes(t, (int)ctas.size(), p->stream));
+  if (p->nets.default_topology) {
+    WB_CUDA(launch_population_episodes(t, (int)ctas.size(), p->stream));
+  } else {
+    PopGenTrainParams g{};
+    g.actor = p->nets.actor;
+    g.critic = p->nets.critic;
+    g.stride = p->stride;
+    g.ts = p->nets.gen_ts;
+    g.grad_floats = p->stride;
+    g.n_dense = nd;
+    memcpy(g.layer_end, p->layer_end, sizeof(g.layer_end));
+    g.t = t;
+    WB_CUDA(launch_population_generic_episodes(g, (int)ctas.size(), p->stream));
+  }
   p->launches++;
   return WB_OK;
 }
 
 static int32_t copy_agent(wb_population* p, int32_t agent, float* dev_base, const float* src_host, float* dst_host) {
   WB_REQUIRE(agent >= 0 && agent < p->n, "agent outside the population");
-  float* d = dev_base + (size_t)agent * kAgentStride;
-  if (src_host) WB_CUDA(cudaMemcpyAsync(d, src_host, sizeof(float) * kTotalParams, cudaMemcpyHostToDevice, p->stream));
-  if (dst_host) WB_CUDA(cudaMemcpyAsync(dst_host, d, sizeof(float) * kTotalParams, cudaMemcpyDeviceToHost, p->stream));
+  float* d = dev_base + (size_t)agent * p->stride;
+  if (src_host) WB_CUDA(cudaMemcpyAsync(d, src_host, sizeof(float) * p->n_total, cudaMemcpyHostToDevice, p->stream));
+  if (dst_host) WB_CUDA(cudaMemcpyAsync(dst_host, d, sizeof(float) * p->n_total, cudaMemcpyDeviceToHost, p->stream));
   WB_CUDA(cudaStreamSynchronize(p->stream));
   return WB_OK;
 }
@@ -178,16 +196,33 @@ static int32_t act(wb_population* p, int32_t n, int32_t mode, const float* state
   a.logp = logp;
   a.mean = mean;
   a.value = value;
-  WB_CUDA(launch_population_act(a, p->stream));
+  if (p->nets.default_topology) {
+    WB_CUDA(launch_population_act(a, p->stream));
+  } else {
+    PopGenActParams g{};
+    g.actor = p->nets.actor;
+    g.critic = p->nets.critic;
+    g.stride = p->stride;
+    g.chunk_floats = generic_act_chunk_floats(p->nets.actor, p->nets.critic);
+    g.a = a;
+    WB_CUDA(launch_population_generic_act(g, p->stream));
+  }
   p->launches++;
   return WB_OK;
 }
 
 extern "C" {
 
-int32_t wb_population_create(int32_t n_agents, const wb_hyperparams* hp, wb_population** out) {
+int32_t wb_population_create_net(int32_t n_agents, int32_t state_size, int32_t action_size, const int32_t* actor_kinds,
+                                 const int32_t* actor_sizes, int32_t actor_layers, const int32_t* critic_kinds, const int32_t* critic_sizes,
+                                 int32_t critic_layers, const wb_hyperparams* hp, wb_population** out) {
   WB_REQUIRE(out, "out is null");
   *out = nullptr;
+  Networks nets;
+  if (int32_t rc = build_networks(state_size, action_size, actor_kinds, actor_sizes, actor_layers, critic_kinds, critic_sizes, critic_layers, &nets))
+    return rc;
+  if (!nets.default_topology && generic_episodes_smem_bytes(nets.actor, nets.critic, nets.gen_ts) > kPopGenMaxSmem)
+    return fail(WB_ERR_UNSUPPORTED, "the layer caches and one episode's arrays exceed shared memory");
   WB_REQUIRE(n_agents >= 1, "n_agents must be at least 1");
   if (hp)
     for (int32_t a = 0; a < n_agents; a++)
@@ -196,10 +231,16 @@ int32_t wb_population_create(int32_t n_agents, const wb_hyperparams* hp, wb_popu
   wb_population* p = new (std::nothrow) wb_population();
   WB_REQUIRE(p, "out of host memory");
   p->n = n_agents;
+  p->nets = nets;
+  p->state = state_size;
+  p->action = action_size;
+  p->n_total = nets.actor.n_params + nets.critic.n_params;
+  p->stride = (p->n_total + 3 + 3) / 4 * 4;
+  p->n_dense = generic_layer_ends(nets.actor, nets.critic, p->layer_end);
   cudaGetDevice(&p->device);
   try {
     p->hp.resize(n_agents);
-    p->iterations.assign((size_t)n_agents * kDenseLayers, 0);
+    p->iterations.assign((size_t)n_agents * p->n_dense, 0);
     p->episodes.assign(n_agents, 0);
   } catch (const std::bad_alloc&) {
     delete p;
@@ -210,7 +251,7 @@ int32_t wb_population_create(int32_t n_agents, const wb_hyperparams* hp, wb_popu
     if (hp) p->hp[a] = hp[a]; else wb_hyperparams_default(&p->hp[a]);
     population_agent_consts(p->hp[a], &consts[a]);
   }
-  const size_t bytes = sizeof(float) * kAgentStride * (size_t)n_agents;
+  const size_t bytes = sizeof(float) * p->stride * (size_t)n_agents;
   cudaError_t e = cudaMalloc(&p->d_params, bytes);
   if (e == cudaSuccess) e = cudaMalloc(&p->d_m, bytes);
   if (e == cudaSuccess) e = cudaMalloc(&p->d_v, bytes);
@@ -227,6 +268,12 @@ int32_t wb_population_create(int32_t n_agents, const wb_hyperparams* hp, wb_popu
   }
   *out = p;
   return WB_OK;
+}
+
+int32_t wb_population_create(int32_t n_agents, const wb_hyperparams* hp, wb_population** out) {
+  const int32_t ak[6] = {WB_DENSE, WB_LEAKYRELU, WB_DENSE, WB_LEAKYRELU, WB_DENSE, WB_TANH}, as[6] = {kHid, 0, kHid, 0, kAct, 0};
+  const int32_t ck[3] = {WB_DENSE, WB_LEAKYRELU, WB_DENSE}, cs[3] = {kHid, 0, 1};
+  return wb_population_create_net(n_agents, kIn, kAct, ak, as, 6, ck, cs, 3, hp, out);
 }
 
 int32_t wb_population_destroy(wb_population* p) {
@@ -281,7 +328,15 @@ int32_t wb_population_get_adam(wb_population* p, int32_t agent, float* m_host, f
   WB_REQUIRE(p && m_host && v_host && steps_host, "null argument");
   if (int32_t rc = copy_agent(p, agent, p->d_m, nullptr, m_host)) return rc;
   if (int32_t rc = copy_agent(p, agent, p->d_v, nullptr, v_host)) return rc;
-  memcpy(steps_host, &p->iterations[(size_t)agent * kDenseLayers], sizeof(int32_t) * kDenseLayers);
+  memcpy(steps_host, &p->iterations[(size_t)agent * p->n_dense], sizeof(int32_t) * p->n_dense);
+  return WB_OK;
+}
+
+int32_t wb_population_num_params(const wb_population* p, int32_t which, int32_t* n_out) {
+  WB_REQUIRE(p && n_out, "null argument");
+  if (which == 0) *n_out = p->nets.actor.n_params;
+  else if (which == 1) *n_out = p->nets.critic.n_params;
+  else return fail(WB_ERR_INVALID, "which must be 0 (actor) or 1 (critic)");
   return WB_OK;
 }
 
@@ -295,19 +350,19 @@ int32_t wb_population_sample(wb_population* p, int32_t n, const float* states_ho
                              float* logp_host, float* mean_host) {
   WB_REQUIRE(p && states_host && uniforms_host && actions_host && logp_host, "null argument");
   WB_REQUIRE(n == p->n, "n must equal the population size (walker w acts with agent w)");
-  const size_t N = (size_t)n;
-  if (int32_t rc = grow_stage(p, sizeof(float) * N * (kIn + 2 * kAct + 3 * kAct))) return rc;
+  const size_t N = (size_t)n, IN = (size_t)p->state, ACT = (size_t)p->action;
+  if (int32_t rc = grow_stage(p, sizeof(float) * N * (IN + 2 * ACT + 3 * ACT))) return rc;
   float* d_states = p->d_stage;
-  float* d_uni = d_states + N * kIn;
-  float* d_act = d_uni + N * kAct * 2;
-  float* d_logp = d_act + N * kAct;
-  float* d_mean = d_logp + N * kAct;
-  WB_CUDA(cudaMemcpyAsync(d_states, states_host, sizeof(float) * N * kIn, cudaMemcpyHostToDevice, p->stream));
-  WB_CUDA(cudaMemcpyAsync(d_uni, uniforms_host, sizeof(float) * N * kAct * 2, cudaMemcpyHostToDevice, p->stream));
+  float* d_uni = d_states + N * IN;
+  float* d_act = d_uni + N * ACT * 2;
+  float* d_logp = d_act + N * ACT;
+  float* d_mean = d_logp + N * ACT;
+  WB_CUDA(cudaMemcpyAsync(d_states, states_host, sizeof(float) * N * IN, cudaMemcpyHostToDevice, p->stream));
+  WB_CUDA(cudaMemcpyAsync(d_uni, uniforms_host, sizeof(float) * N * ACT * 2, cudaMemcpyHostToDevice, p->stream));
   if (int32_t rc = act(p, n, kModeSample, d_states, d_uni, 0, 0, d_act, d_logp, d_mean, nullptr)) return rc;
-  WB_CUDA(cudaMemcpyAsync(actions_host, d_act, sizeof(float) * N * kAct, cudaMemcpyDeviceToHost, p->stream));
-  WB_CUDA(cudaMemcpyAsync(logp_host, d_logp, sizeof(float) * N * kAct, cudaMemcpyDeviceToHost, p->stream));
-  if (mean_host) WB_CUDA(cudaMemcpyAsync(mean_host, d_mean, sizeof(float) * N * kAct, cudaMemcpyDeviceToHost, p->stream));
+  WB_CUDA(cudaMemcpyAsync(actions_host, d_act, sizeof(float) * N * ACT, cudaMemcpyDeviceToHost, p->stream));
+  WB_CUDA(cudaMemcpyAsync(logp_host, d_logp, sizeof(float) * N * ACT, cudaMemcpyDeviceToHost, p->stream));
+  if (mean_host) WB_CUDA(cudaMemcpyAsync(mean_host, d_mean, sizeof(float) * N * ACT, cudaMemcpyDeviceToHost, p->stream));
   WB_CUDA(cudaStreamSynchronize(p->stream));
   return WB_OK;
 }
@@ -352,12 +407,13 @@ int32_t wb_population_train_trajectories(wb_population* p, int32_t n_traj, const
   WB_REQUIRE(n_index <= INT32_MAX, "too many mini-batch indices for one call");
   const size_t rows = (size_t)offsets_host[n_traj], R = rows > 0 ? rows : 1, N = (size_t)n_traj;
   WB_REQUIRE(rows <= (size_t)INT32_MAX, "too many rows");
-  const size_t floats = R * (kIn + 2 * kAct + 4) + 2 * N;
+  const size_t IN = (size_t)p->state, ACT = (size_t)p->action;
+  const size_t floats = R * (IN + 2 * ACT + 4) + 2 * N;
   if (int32_t rc = grow_stage(p, sizeof(float) * floats + sizeof(int32_t) * (N + (size_t)n_index) + 16)) return rc;
   float* d_states = p->d_stage;
-  float* d_actions = d_states + R * kIn;
-  float* d_logp = d_actions + R * kAct;
-  float* d_rewards = d_logp + R * kAct;
+  float* d_actions = d_states + R * IN;
+  float* d_logp = d_actions + R * ACT;
+  float* d_rewards = d_logp + R * ACT;
   float* d_values = d_rewards + R;
   float* d_returns = d_values + R;
   float* d_adv = d_returns + R;
@@ -365,9 +421,9 @@ int32_t wb_population_train_trajectories(wb_population* p, int32_t n_traj, const
   int32_t* d_skipped = reinterpret_cast<int32_t*>(d_losses + 2 * N);
   int32_t* d_index = d_skipped + N;
   if (rows) {
-    WB_CUDA(cudaMemcpyAsync(d_states, states_host, sizeof(float) * rows * kIn, cudaMemcpyHostToDevice, p->stream));
-    WB_CUDA(cudaMemcpyAsync(d_actions, actions_host, sizeof(float) * rows * kAct, cudaMemcpyHostToDevice, p->stream));
-    WB_CUDA(cudaMemcpyAsync(d_logp, logp_host, sizeof(float) * rows * kAct, cudaMemcpyHostToDevice, p->stream));
+    WB_CUDA(cudaMemcpyAsync(d_states, states_host, sizeof(float) * rows * IN, cudaMemcpyHostToDevice, p->stream));
+    WB_CUDA(cudaMemcpyAsync(d_actions, actions_host, sizeof(float) * rows * ACT, cudaMemcpyHostToDevice, p->stream));
+    WB_CUDA(cudaMemcpyAsync(d_logp, logp_host, sizeof(float) * rows * ACT, cudaMemcpyHostToDevice, p->stream));
     WB_CUDA(cudaMemcpyAsync(d_rewards, rewards_host, sizeof(float) * rows, cudaMemcpyHostToDevice, p->stream));
   }
   if (n_index) WB_CUDA(cudaMemcpyAsync(d_index, batch_index_host, sizeof(int32_t) * n_index, cudaMemcpyHostToDevice, p->stream));

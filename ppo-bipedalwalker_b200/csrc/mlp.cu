@@ -15,6 +15,7 @@
 // fused multiply-add; the cross-sample sum of dW is tiled (per CTA, then across CTAs) instead of the
 // reference's strictly sequential per-sample accumulation -- covered by the 1e-4 relative tolerance.
 #include "mlp.cuh"
+#include "ppo_device.cuh"
 
 #include <cfloat>
 
@@ -75,19 +76,6 @@ __device__ __forceinline__ void dense64_forward(const float* in, const float* W,
       const int o = to + 16 * j;
       out[(ts * 4 + k) * kPad + o] = leaky(acc[k][j] + b[o]);
     }
-}
-
-// Philox-4x32-10 (counter-based; extension -- the reference's System.Random is unseedable)
-__device__ __forceinline__ uint4 philox4x32(uint4 ctr, uint2 key) {
-#pragma unroll
-  for (int r = 0; r < 10; r++) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, ctr.x), lo0 = 0xD2511F53u * ctr.x;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, ctr.z), lo1 = 0xCD9E8D57u * ctr.z;
-    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-    key.x += 0x9E3779B9u;
-    key.y += 0xBB67AE85u;
-  }
-  return ctr;
 }
 
 // NormalDistribution.LogProbabilityDensity, NormalDistribution.cs:24-32 (-ln(std) and ln(sqrt(2pi)) precomputed on the host)
@@ -473,44 +461,6 @@ __global__ void adam_kernel(const AdamParams a) {
   adam_update(a, i, a.grads[i]);
 }
 
-// PPOAgent.MonteCarloReturn/MonteCarloAdvantages (:475-498), GeneralizedAdvantageEstimate (:414-444, whose nextGae is
-// never updated in the reference), Normalize (:461-472).  One trajectory: an inherently sequential fp32 recurrence.
-__device__ __forceinline__ void trajectory_returns(const float* __restrict__ rewards, const float* __restrict__ values, int n, float gamma,
-                                                   float lambda, int use_gae, int normalize, float norm_eps, float* __restrict__ returns,
-                                                   float* __restrict__ advantages) {
-  if (use_gae) {
-    const float next_gae = 0.0f;
-    float next_value = 0.0f;
-    for (int i = n - 1; i >= 0; i--) {
-      const float cur = values[i];
-      const float delta = __fsub_rn(__fadd_rn(rewards[i], __fmul_rn(gamma, next_value)), cur);
-      next_value = cur;
-      const float gae = __fadd_rn(delta, __fmul_rn(__fmul_rn(gamma, lambda), next_gae));
-      advantages[i] = gae;
-      returns[i] = __fadd_rn(gae, values[i]);
-    }
-  } else {
-    float g = 0.0f;
-    for (int i = n - 1; i >= 0; i--) {
-      g = __fadd_rn(rewards[i], __fmul_rn(g, gamma));
-      returns[i] = g;
-    }
-    for (int i = 0; i < n; i++) advantages[i] = __fsub_rn(returns[i], values[i]);
-  }
-  if (normalize && n > 0) {
-    double acc = 0.0;
-    for (int i = 0; i < n; i++) acc += (double)advantages[i];
-    const float mean = (float)(acc / (double)n);
-    double ss = 0.0;
-    for (int i = 0; i < n; i++) {
-      const double d = (double)__fsub_rn(advantages[i], mean);
-      ss += d * d;
-    }
-    const float sd = (float)sqrt(ss / (double)n);
-    const float div = __fadd_rn(sd, norm_eps);
-    for (int i = 0; i < n; i++) advantages[i] = __fdiv_rn(__fsub_rn(advantages[i], mean), div);
-  }
-}
 __global__ void returns_kernel(const float* rewards, const float* values, int n, float gamma, float lambda, int use_gae,
                                int normalize, float norm_eps, float* returns, float* advantages) {
   if (blockIdx.x != 0 || threadIdx.x != 0) return;
@@ -734,7 +684,7 @@ __global__ void __launch_bounds__(kActWarps * 32) population_act_kernel(const Po
 // the host's Adam correction table.  Independent networks, so the CTAs need no exchange (one SM per agent).  An item's rows live
 // in a time-major ring [R][C]: row i = ((t0 + i) mod R) * C + column.  Its rewards and values are gathered into shared memory for
 // trajectory_returns and the returns / advantages scattered back.  Mini-batch indices come from the caller or, with a null index
-// pointer, from draw_permutation (below).
+// pointer, from draw_permutation (ppo_device.cuh).
 struct __align__(16) PopSmem {
   MlpSmem m;
   int32_t rows[kTile];
@@ -742,26 +692,6 @@ struct __align__(16) PopSmem {
   uint32_t key[kPopMaxLen];
   int32_t perm[kPopMaxLen];
 };
-
-// PPOAgent.CreateBatches (PPOAgent.cs:501-540: sampling without replacement) drawn on the device: local row i of the episode gets
-// key(i) = Philox-4x32-10(counter (i, epoch, episode, agent), key (seed lo, seed hi)).x, where `episode` counts the agent's episodes
-// trained before this one; perm = the rows ordered by (key, row).  Each row's rank is counted over the <= 1 024 keys.
-__device__ __forceinline__ void draw_permutation(PopSmem& E, int L, int epoch, int episode, int agent, uint64_t seed, int tid) {
-  for (int i = tid; i < L; i += kMlpThreads)
-    E.key[i] = philox4x32(make_uint4((uint32_t)i, (uint32_t)epoch, (uint32_t)episode, (uint32_t)agent),
-                          make_uint2((uint32_t)seed, (uint32_t)(seed >> 32))).x;
-  __syncthreads();
-  for (int j = tid; j < L; j += kMlpThreads) {
-    const uint32_t kj = E.key[j];
-    int rank = 0;
-    for (int i = 0; i < L; i++) {
-      const uint32_t ki = E.key[i];
-      rank += (ki < kj || (ki == kj && i < j)) ? 1 : 0;
-    }
-    E.perm[rank] = j;
-  }
-  __syncthreads();
-}
 
 __global__ void __launch_bounds__(kMlpThreads, 1) population_episodes_kernel(const PopTrainParams P) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -830,7 +760,7 @@ __global__ void __launch_bounds__(kMlpThreads, 1) population_episodes_kernel(con
     for (int epoch = 0; epoch < P.epochs && per_epoch > 0; epoch++) {
       const int32_t* index = E.perm;
       if (P.batch_index) index = P.batch_index + item.index_off + (size_t)epoch * per_epoch * B;
-      else draw_permutation(E, L, epoch, item.episode, cta.agent, P.seed, tid);
+      else draw_permutation<kMlpThreads>(E.key, E.perm, L, epoch, item.episode, cta.agent, P.seed, tid);
       for (int b = 0; b < per_epoch; b++, step++, index += B) {
         float accW2[4][4];
 #pragma unroll
@@ -1021,6 +951,8 @@ void population_agent_consts(const wb_hyperparams& hp, PopAgent* o) {
   o->batch = hp.batch_size;
   o->use_gae = hp.use_gae;
   o->normalize = hp.normalize_advantages;
+  o->log_std = hp.log_std;
+  o->clip_eps = hp.epsilon;
 }
 
 cudaError_t launch_population_act(const PopActParams& a, cudaStream_t stream) {

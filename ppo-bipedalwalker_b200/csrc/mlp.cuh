@@ -121,7 +121,9 @@ struct PopAgent {
   float stdv, neg_log_std, log_sqrt_2pi, upper, lower, variance;  // GradConsts
   float alpha, beta1, beta2, adam_eps;
   float gamma, lambda, norm_eps, batch_size_f;
-  int32_t batch, use_gae, normalize, pad;
+  int32_t batch, use_gae, normalize;
+  float log_std, clip_eps;  // the raw values: the any-topology kernels derive sigma and the clip range on the device, as ppo_generic_kernel
+  int32_t pad[3];
 };
 void population_agent_consts(const wb_hyperparams& hp, PopAgent* out);
 struct PopActParams {
@@ -289,6 +291,37 @@ int generic_grid_for(int n, int ts, int sm_count);
 cudaError_t launch_mlp_generic(const GenParams& p, int grid, cudaStream_t stream);
 cudaError_t launch_reduce_partials_n(const float* partials, int nparts, float* grads, int n_floats, cudaStream_t stream);
 cudaError_t launch_adam_generic(const GenAdamParams& a, cudaStream_t stream);
+
+// the two networks of a wb_policy / wb_population, validated (wb_policy_create's limits and statuses; a failure records the message)
+struct Networks {
+  GenNet actor, critic;
+  int gen_ts;             // generic_tile_samples
+  bool default_topology;  // the reference's default networks: the specialised kernels apply
+};
+int32_t build_networks(int32_t state_size, int32_t action_size, const int32_t* actor_kinds, const int32_t* actor_sizes, int32_t actor_layers,
+                       const int32_t* critic_kinds, const int32_t* critic_sizes, int32_t critic_layers, Networks* out);
+// one past the last parameter of every dense layer (actor layers, then critic layers at + actor.n_params); returns their number
+int generic_layer_ends(const GenNet& actor, const GenNet& critic, int32_t* layer_end);
+
+// ---- populations of any topology (population_generic_act_kernel / population_generic_episodes_kernel, mlp_generic.cu)
+constexpr int kGenActWarps = 2;  // walkers (one warp each) per CTA of population_generic_act_kernel
+constexpr size_t kPopGenMaxSmem = 227 * 1024;  // shared memory a CTA may hold on sm_100
+struct PopGenActParams {
+  GenNet actor, critic;
+  int32_t stride;        // floats per agent row
+  int32_t chunk_floats;  // generic_act_chunk_floats
+  PopActParams a;        // states [n][state], uniforms [n][act][2], actions / logp / mean [n][act], value [n]
+};
+struct PopGenTrainParams {
+  GenNet actor, critic;
+  int32_t stride, ts, grad_floats, n_dense;
+  int32_t layer_end[kGenMaxDense];
+  PopTrainParams t;  // corr: [Adam steps][2 * n_dense]
+};
+int generic_act_chunk_floats(const GenNet& actor, const GenNet& critic);
+size_t generic_episodes_smem_bytes(const GenNet& actor, const GenNet& critic, int ts);
+cudaError_t launch_population_generic_act(const PopGenActParams& g, cudaStream_t stream);
+cudaError_t launch_population_generic_episodes(const PopGenTrainParams& g, int n_ctas, cudaStream_t stream);
 
 int tc_grid_for(int n, int sm_count);
 cudaError_t launch_mlp_tc(const MlpParams& p, int grid, cudaStream_t stream, const FusedTail* tail = nullptr);

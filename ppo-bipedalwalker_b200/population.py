@@ -4,8 +4,9 @@ In the reference every walker owns its agent -- new Walker() builds its own PPOA
 each of its own episodes as soon as the episode ends (Environment.cs:91,157-164 -> PPOAgent.Train(Trajectory), PPOAgent.cs:147-172).
 Running the reference N times gives N independent learners, which is how seed studies and hyper-parameter sweeps are run.
 
-  PPOPopulation   P agents of the default networks, each with its own weights, Adam state, step counters and Hyperparams.  Agent a
-                  is exactly PPOAgent(seed=seeds[a], hp=hp[a]) on kernel variant 1: same initial weights, same actions, same training.
+  PPOPopulation   P agents with the same two networks (the defaults, or any the DSL describes), each with its own weights, Adam
+                  state, step counters and Hyperparams.  Agent a is exactly PPOAgent(actor=, critic=, seed=seeds[a], hp=hp[a]) (kernel
+                  variant 1 for the default networks): same initial weights, same actions, same training.
   IndependentPPO  N walkers, N agents, the reference's episode semantics for every walker at once: no segments, no bootstrap; a
                   walker whose episode ended (Terminal, or steps > MaxTimesteps) trains its agent on the complete episode before it
                   acts again (Environment.Update -> TrainNetworks -> Reset).
@@ -18,11 +19,8 @@ import numpy as np
 
 from ._lib import ACT, OBS, Hyperparams, check, lib, ptr
 from .env import DT_FRAME, EnvBatch, default_hyperparams
-from .ppo import DEFAULT_ACTOR, DEFAULT_CRITIC, ParseLayers, dense_shapes, weights_lines, xavier_flat
+from .ppo import DEFAULT_ACTOR, DEFAULT_CRITIC, dense_shapes, resolve_networks, weights_lines, xavier_flat
 from .scene import IObject, TerrainEnvBatch
-
-N_PARAMS = 6149  # actor (5 252) | critic (897)
-N_ACTOR = 5252
 
 
 def default_seeds(seed: int, n_agents: int) -> list[int]:
@@ -31,13 +29,15 @@ def default_seeds(seed: int, n_agents: int) -> list[int]:
 
 
 class PPOPopulation:
-    """n_agents independent PPOAgent(12, 4) (PPOAgent.cs:23-37) on one device handle.
+    """n_agents independent PPOAgent(stateSize, actionSize) (PPOAgent.cs:23-37) on one device handle, all with the networks of the
+    DSL strings actor / critic (PPOAgent.__init__'s fallbacks apply).
 
     hp: None (the defaults), one Hyperparams shared by every agent, or a list of n_agents of them (a sweep:
     [Settings(...).to_hyperparams(), ...]).  seeds[a] seeds agent a's numpy Generator exactly as PPOAgent(seed=seeds[a]) does: its
     Xavier initialisation, its Box-Muller uniforms and its mini-batch permutations; default: default_seeds(seed, n_agents)."""
 
-    def __init__(self, n_agents: int, hp=None, seed: int = 0, seeds=None, stream: int | None = None):
+    def __init__(self, n_agents: int, hp=None, seed: int = 0, seeds=None, stream: int | None = None, actor: str = DEFAULT_ACTOR,
+                 critic: str = DEFAULT_CRITIC, stateSize: int = OBS, actionSize: int = ACT):
         if hp is None:
             hps = [default_hyperparams() for _ in range(n_agents)]
         elif isinstance(hp, Hyperparams):
@@ -47,21 +47,34 @@ class PPOPopulation:
             if len(hps) != n_agents:
                 raise ValueError(f"{len(hps)} Hyperparams for {n_agents} agents")
         self.n, self.hp = n_agents, hps
+        self.stateSize, self.actionSize = stateSize, actionSize
+        self.actor_structure, self.actor_layers, self.critic_structure, self.critic_layers = resolve_networks(actor, critic, actionSize)
+        lists = []
+        for layers in (self.actor_layers, self.critic_layers):
+            lists += [np.array([k for k, _ in layers], np.int32), np.array([s for _, s in layers], np.int32)]
         h = C.c_void_p()
-        check(lib().wb_population_create(n_agents, (Hyperparams * max(n_agents, 1))(*hps), C.byref(h)))
+        check(lib().wb_population_create_net(n_agents, stateSize, actionSize, ptr(lists[0]), ptr(lists[1]), len(self.actor_layers),
+                                             ptr(lists[2]), ptr(lists[3]), len(self.critic_layers), (Hyperparams * max(n_agents, 1))(*hps),
+                                             C.byref(h)))
         self._h = h
+        counts = []
+        for which in (0, 1):
+            n = C.c_int32(0)
+            check(lib().wb_population_num_params(h, which, C.byref(n)))
+            counts.append(n.value)
+        self.N_ACTOR, self.N_PARAMS = counts[0], counts[0] + counts[1]
+        self.n_dense = len(dense_shapes(stateSize, self.actor_layers)) + len(dense_shapes(stateSize, self.critic_layers))
         if stream is not None:
             self.set_stream(stream)
         self.seeds = default_seeds(seed, n_agents) if seeds is None else [int(s) for s in seeds]
         if len(self.seeds) != n_agents:
             raise ValueError(f"{len(self.seeds)} seeds for {n_agents} agents")
-        self.actor_layers, self.critic_layers = ParseLayers(DEFAULT_ACTOR), ParseLayers(DEFAULT_CRITIC)
         self.rngs = []
         for a in range(n_agents):  # PPOAgent.__init__: critic first, then actor, from the agent's own generator
             rng = np.random.default_rng(self.seeds[a])
-            critic = xavier_flat(OBS, self.critic_layers, rng)
-            actor = xavier_flat(OBS, self.actor_layers, rng)
-            self.set_weights(a, np.concatenate([actor, critic]))
+            critic_w = xavier_flat(stateSize, self.critic_layers, rng)
+            actor_w = xavier_flat(stateSize, self.actor_layers, rng)
+            self.set_weights(a, np.concatenate([actor_w, critic_w]))
             self.rngs.append(rng)
 
     def close(self):
@@ -84,45 +97,47 @@ class PPOPopulation:
 
     # -- per-agent state
     def get_weights(self, agent: int) -> np.ndarray:
-        """[6149] actor | critic of one agent (the flat layout of PPOAgent.actor / .critic get_flat, concatenated)."""
-        out = np.empty(N_PARAMS, np.float32)
+        """[N_PARAMS] actor | critic of one agent (the flat layout of PPOAgent.actor / .critic get_flat, concatenated)."""
+        out = np.empty(self.N_PARAMS, np.float32)
         check(lib().wb_population_get_weights(self._h, agent, ptr(out)))
         return out
 
     def set_weights(self, agent: int, flat):
         flat = np.ascontiguousarray(flat, np.float32)
-        assert flat.size == N_PARAMS
+        assert flat.size == self.N_PARAMS
         check(lib().wb_population_set_weights(self._h, agent, ptr(flat)))
 
     def get_grads(self, agent: int) -> np.ndarray:
-        out = np.empty(N_PARAMS, np.float32)
+        out = np.empty(self.N_PARAMS, np.float32)
         check(lib().wb_population_get_grads(self._h, agent, ptr(out)))
         return out
 
     def adam(self, agent: int):
-        """(m [6149], v [6149], step counters [5]: actor L1-L3, critic L1-L2) of one agent."""
-        m, v = np.empty(N_PARAMS, np.float32), np.empty(N_PARAMS, np.float32)
-        steps = np.zeros(5, np.int32)
+        """(m [N_PARAMS], v [N_PARAMS], step counters [n_dense]: actor layers, then critic layers) of one agent."""
+        m, v = np.empty(self.N_PARAMS, np.float32), np.empty(self.N_PARAMS, np.float32)
+        steps = np.zeros(self.n_dense, np.int32)
         check(lib().wb_population_get_adam(self._h, agent, ptr(m), ptr(v), ptr(steps)))
         return m, v, steps
 
     def Save(self, agent: int):
         """PPOAgent.Save (PPOAgent.cs:192-213) of one agent -> (critic lines, actor lines) of the two .weights files."""
         flat = self.get_weights(agent)
-        return (weights_lines(DEFAULT_CRITIC, dense_shapes(OBS, self.critic_layers), flat[N_ACTOR:]),
-                weights_lines(DEFAULT_ACTOR, dense_shapes(OBS, self.actor_layers), flat[:N_ACTOR]))
+        return (weights_lines(self.critic_structure, dense_shapes(self.stateSize, self.critic_layers), flat[self.N_ACTOR:]),
+                weights_lines(self.actor_structure, dense_shapes(self.stateSize, self.actor_layers), flat[:self.N_ACTOR]))
 
     # -- acting
     def SampleActions(self, states, uniforms=None):
         """PPOAgent.SampleActions (PPOAgent.cs:381-398) of every agent on its walker's state: states [P][12] -> (actions, logp, mean,
-        std), each [P][4].  uniforms [P][4][2] (injected), default: one draw of shape (1, 4, 2) from each agent's own generator."""
-        s = np.ascontiguousarray(states, np.float32).reshape(self.n, OBS)
+        std), each [P][actionSize].  uniforms [P][actionSize][2] (injected), default: one draw of shape (1, actionSize, 2) from each
+        agent's own generator."""
+        ACT_ = self.actionSize
+        s = np.ascontiguousarray(states, np.float32).reshape(self.n, self.stateSize)
         if uniforms is None:
-            uniforms = np.concatenate([rng.random((1, ACT, 2)) for rng in self.rngs])
-        u = np.ascontiguousarray(uniforms, np.float32).reshape(self.n, ACT, 2)
-        actions, logp, mean = (np.empty((self.n, ACT), np.float32) for _ in range(3))
+            uniforms = np.concatenate([rng.random((1, ACT_, 2)) for rng in self.rngs])
+        u = np.ascontiguousarray(uniforms, np.float32).reshape(self.n, ACT_, 2)
+        actions, logp, mean = (np.empty((self.n, ACT_), np.float32) for _ in range(3))
         check(lib().wb_population_sample(self._h, self.n, ptr(s), ptr(u), ptr(actions), ptr(logp), ptr(mean)))
-        std = np.array([[np.exp(np.float32(h.log_std))] * ACT for h in self.hp], np.float32)  # GetStandardDeviations, PPOAgent.cs:367-378
+        std = np.array([[np.exp(np.float32(h.log_std))] * ACT_ for h in self.hp], np.float32)  # GetStandardDeviations, PPOAgent.cs:367-378
         return actions, logp, mean, std
 
     # -- training
@@ -155,7 +170,7 @@ class PPOPopulation:
         def rows_of(attr, width):
             parts = [np.asarray(getattr(t, attr), np.float32).reshape(-1, width) for t in trajectories if len(t.States)]
             return np.ascontiguousarray(np.concatenate(parts) if parts else np.zeros((0, width), np.float32))
-        S, A, LP = rows_of("States", OBS), rows_of("Actions", ACT), rows_of("LogProbabilities", ACT)
+        S, A, LP = rows_of("States", self.stateSize), rows_of("Actions", self.actionSize), rows_of("LogProbabilities", self.actionSize)
         R = rows_of("Rewards", 1).reshape(rows)
         V, G, Adv = (np.empty(rows, np.float32) for _ in range(3))
         losses = np.zeros((len(pairs), 2), np.float32)
@@ -179,13 +194,16 @@ class IndependentPPO:
     indices drawn on the device (seed train_seed).  A ring column is only written by its own walker, and the walker has trained
     before it writes again.  episode_log() lists every finished episode: step, agent, length, reward sum and the two losses."""
 
-    def __init__(self, n_envs: int, floor="Metal", walker="Carpet", hp=None, seed: int = 0, epochs: int = 5, terrain=None, seeds=None):
+    def __init__(self, n_envs: int, floor="Metal", walker="Carpet", hp=None, seed: int = 0, epochs: int = 5, terrain=None, seeds=None,
+                 actor: str = DEFAULT_ACTOR, critic: str = DEFAULT_CRITIC, stateSize: int = OBS, actionSize: int = ACT):
+        if (stateSize, actionSize) != (OBS, ACT):
+            raise ValueError(f"the walker observes {OBS} values and takes {ACT} actions; got stateSize={stateSize}, actionSize={actionSize}")
         import torch
         self.torch = torch
         self.n, self.epochs, self.seed = n_envs, epochs, seed
         self.act_seed, self.train_seed = 2 * seed, 2 * seed + 1
         self.stream = torch.cuda.current_stream().cuda_stream
-        self.pop = PPOPopulation(n_envs, hp, seed=seed, seeds=seeds, stream=self.stream)
+        self.pop = PPOPopulation(n_envs, hp, seed=seed, seeds=seeds, stream=self.stream, actor=actor, critic=critic)
         env_hp = self.pop.hp[0]
         if any((h.iterations, h.max_timesteps) != (env_hp.iterations, env_hp.max_timesteps) for h in self.pop.hp):
             raise ValueError("the walkers step in lockstep: every agent's Hyperparams must share iterations and max_timesteps")

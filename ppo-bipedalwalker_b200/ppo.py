@@ -64,6 +64,24 @@ def xavier_flat(input_size: int, layers, rng: np.random.Generator) -> np.ndarray
     return np.concatenate(parts)
 
 
+def resolve_networks(actor: str, critic: str, actionSize: int):
+    """PPOAgent.CreateNetworks' fallbacks (PPOAgent.cs:41-93): a DSL string that does not parse, or whose last dense layer has the
+    wrong size (one value / actionSize means), is replaced by the default network.  -> (actor, actor layers, critic, critic layers)"""
+    try:
+        c_layers = ParseLayers(critic)
+    except ValueError:
+        critic, c_layers = DEFAULT_CRITIC, ParseLayers(DEFAULT_CRITIC)
+    try:
+        a_layers = ParseLayers(actor)
+    except ValueError:
+        actor, a_layers = DEFAULT_ACTOR, ParseLayers(DEFAULT_ACTOR)
+    if [s for k, s in c_layers if k == DENSE][-1:] != [1]:
+        critic, c_layers = DEFAULT_CRITIC, ParseLayers(DEFAULT_CRITIC)
+    if [s for k, s in a_layers if k == DENSE][-1:] != [actionSize]:
+        actor, a_layers = DEFAULT_ACTOR, ParseLayers(DEFAULT_ACTOR)
+    return actor, a_layers, critic, c_layers
+
+
 @dataclass
 class Trajectory:
     """Walker/PPO/Trajectory.cs (lists of per-step values for ONE episode)."""
@@ -186,19 +204,7 @@ class PPOAgent:
                  critic: str = DEFAULT_CRITIC, seed: int | None = None, stream: int | None = None):
         self.stateSize, self.actionSize = stateSize, actionSize
         self.hp = hp if hp is not None else default_hyperparams()
-        try:  # CreateNetworks falls back to the defaults on a bad DSL string (PPOAgent.cs:41-93)
-            c_layers = ParseLayers(critic)
-        except ValueError:
-            critic, c_layers = DEFAULT_CRITIC, ParseLayers(DEFAULT_CRITIC)
-        try:
-            a_layers = ParseLayers(actor)
-        except ValueError:
-            actor, a_layers = DEFAULT_ACTOR, ParseLayers(DEFAULT_ACTOR)
-        # the last dense layers must produce one value / actionSize means, else the defaults (PPOAgent.cs:78-92)
-        if [s for k, s in c_layers if k == DENSE][-1:] != [1]:
-            critic, c_layers = DEFAULT_CRITIC, ParseLayers(DEFAULT_CRITIC)
-        if [s for k, s in a_layers if k == DENSE][-1:] != [actionSize]:
-            actor, a_layers = DEFAULT_ACTOR, ParseLayers(DEFAULT_ACTOR)
+        actor, a_layers, critic, c_layers = resolve_networks(actor, critic, actionSize)
         ak = np.array([k for k, _ in a_layers], np.int32)
         asz = np.array([s for _, s in a_layers], np.int32)
         ck = np.array([k for k, _ in c_layers], np.int32)
