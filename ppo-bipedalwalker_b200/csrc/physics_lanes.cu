@@ -34,19 +34,8 @@
 #include "physics.cuh"
 #include "physics_math.cuh"
 
-// unroll factor of the vote-free SAT rounds (experiments: -DWB_SAT_UNROLL=1 keeps the loops rolled -> smaller code)
-#ifndef WB_SAT_UNROLL
-#define WB_SAT_UNROLL 6
-#endif
-// 1: the leg-split body sweep gives the Body a slot of its own (three slots per substep instead of two, see legs_sweep)
-#ifndef WB_BODY_SLOT
-#define WB_BODY_SLOT 0
-#endif
-
 namespace wb {
 namespace pl {
-constexpr int kSatUnroll = WB_SAT_UNROLL;
-
 constexpr unsigned kFull = 0xFFFFFFFFu;
 
 #ifdef WB_PHASE_PROFILE
@@ -58,7 +47,6 @@ __device__ __forceinline__ long long prof_clock() {
   asm volatile("mov.u64 %0, %%clock64;" : "=l"(t)::"memory");
   return t;
 }
-__device__ long long g_prof_sat_scratch;  // (unused; keeps the symbol table stable)
 // lanes kernel: clock64 cycles of each CTA (one warp) of the last launch: entry to the first substep, the substep loop,
 // observe + write-back (3 per CTA, CTAs beyond kLanesProfCtas are not recorded); read with wb_lanes_prof_read
 constexpr int kLanesProfCtas = 1 << 16;
@@ -98,7 +86,6 @@ struct Env {
   int sub;      // lane inside the env's L lanes
   int gsub;     // lane inside the current working group (the whole env for joints, one leg's half during the body sweep)
   int gshift;   // first lane of the current working group inside the warp
-  int col;      // (compacting kernel) the walker's column inside the CTA's shared-memory state: lets a noinline stage rebuild the pointers
   bool live;    // env < n
   int flags;    // Collided bits, Terminal, floor-first (identical on the L lanes)
   // material-derived constants (RigidBody ctor, RigidBody.cs:36-50; Impulses.cs:16-17)
@@ -417,83 +404,6 @@ __device__ __forceinline__ bool aabb_hit(float2 amin, float2 amax, float2 bmin, 
   return amin.x < bmax.x && amax.x > bmin.x && amin.y < bmax.y && amax.y > bmin.y;
 }
 
-// ---------------------------------------------------------------- the contact stage of a colliding pair as ONE function
-// Everything of resolve_pair (below) behind the SAT -- minimum over the group's lanes, orientation, significant faces, contact
-// points, MoveObjects, impulses -- with "B is the floor" as a RUN-TIME flag, for callers with two or more lanes per pair.  The
-// compacting kernel's pole drain and floor drain can call this one copy instead of inlining the ~700 instructions twice
-// (-DWB_SHARED_CONTACTS=1, experiment: 9.7 KB less hot code on a kernel that misses the instruction cache, hit rate 90 %).
-// Measured SLOWER (262144 walkers: 4.08 vs 3.99 ms): the call cannot take the two polygons in registers, and reloading them
-// costs more than the smaller footprint returns.  Same arithmetic per value: bit-identical results.
-#ifndef WB_SHARED_CONTACTS
-#define WB_SHARED_CONTACTS 0
-#endif
-}  // namespace pl
-namespace pc {
-template <int G, int kE> __device__ __forceinline__ void group_env_by_col(pl::Env<G, kE>& e, int col, bool live);  // (defined with the kernel)
-}
-namespace pl {
-// (the environment is rebuilt from the column index: a struct argument would carry generic 64-bit pointers, i.e. LD / ST instead of LDS / STS)
-template <class EV, int G>
-__device__ __noinline__ void contact_stage_shared(int col, bool live, bool colliding, int A, int B, bool floorb, float depth, int idx, float2 normal) {
-  static_assert(G > 1, "two or more lanes per pair");
-  EV e;
-  pc::group_env_by_col<G, EV::E>(e, col, live);
-  const FloorConst& fl = *e.fl;
-#pragma unroll
-  for (int m = 1; m < G; m <<= 1) {
-    const float od = __shfl_xor_sync(kFull, depth, m);
-    const int oi = __shfl_xor_sync(kFull, idx, m);
-    const float ox = __shfl_xor_sync(kFull, normal.x, m);
-    const float oy = __shfl_xor_sync(kFull, normal.y, m);
-    if (od < depth || (od == depth && oi < idx)) {
-      depth = od;
-      idx = oi;
-      normal = mk2(ox, oy);
-    }
-  }
-  BodyDyn X = load_dyn(e, A);
-  BodyDyn Y = load_dyn(e, floorb ? A : B);
-  if (floorb) Y = floor_dyn(e);
-  if (vdot(vsub(Y.c, X.c), normal) > 0.0f) normal = vmul(normal, -1.0f);
-  const bool odd = (e.gsub & 1) != 0;
-  const float2 nn = odd ? vneg(normal) : normal;
-  // my polygon: even lanes A, odd lanes B (or the floor, padded to a 6-gon with copies of its vertex 0)
-  const bool mine_floor = odd && floorb;
-  const float2* vb = mine_floor ? fl.v : &V2(e, (odd ? B : A) * 6);
-  const int stride = mine_floor ? 1 : EV::E;
-  const int n = mine_floor ? 4 : nverts(odd ? B : A);
-  float2 P[6];
-#pragma unroll
-  for (int i = 0; i < 6; i++) P[i] = vb[((mine_floor && i >= 4) ? 0 : i) * stride];
-  const int k = support_index6(P, nn);
-  const int kn = (k + 1 == n) ? 0 : k + 1;
-  const int kp = (k == 0) ? n - 1 : k - 1;
-  const Face mine = face_from(vb[k * stride], vb[kn * stride], vb[kp * stride], nn);
-  Face other;
-  other.a.x = __shfl_xor_sync(kFull, mine.a.x, 1);
-  other.a.y = __shfl_xor_sync(kFull, mine.a.y, 1);
-  other.b.x = __shfl_xor_sync(kFull, mine.b.x, 1);
-  other.b.y = __shfl_xor_sync(kFull, mine.b.y, 1);
-  other.max.x = __shfl_xor_sync(kFull, mine.max.x, 1);
-  other.max.y = __shfl_xor_sync(kFull, mine.max.y, 1);
-  const Face ref = odd ? other : mine;
-  const Face inc = odd ? mine : other;
-  float2 c0 = mk2(0.f, 0.f), c1 = mk2(0.f, 0.f);
-  const int ncp = contact_points(ref, inc, normal, c0, c1);
-  const float2 dA = floorb ? vmul(normal, depth) : vhalf(vmul(normal, depth));
-  const float2 dB = floorb ? mk2(0.f, 0.f) : vhalf(vmul(vneg(normal), depth));
-  lanes_sync<EV::L>();  // every lane has read the pre-move vertices, centroids and velocities
-  move_bodies<EV, G>(e, colliding, A, dA, !floorb, B, dB);
-  X.c = vadd(X.c, dA);
-  if (!floorb) Y.c = vadd(Y.c, dB);
-  resolve_impulses_split(X, Y, ncp, c0, c1, normal, floorb ? e.e_wf : e.e_ww, floorb ? e.mu_wf : e.mu_ww, odd);
-  if (ncp > 0 && colliding && e.gsub == 0) {
-    store_dyn(e, A, X);
-    if (!floorb) store_dyn(e, B, Y);  // the floor is never written (inverse mass/inertia 0)
-  }
-  lanes_sync<EV::L>();
-}
-
 // pair-trace record of a candidate whose SAT has not found a collision (yet)
 __device__ __forceinline__ wb_pair_trace pair_trace_no_sat(int other, bool aabb) {
   wb_pair_trace rec;
@@ -512,9 +422,9 @@ __device__ __forceinline__ wb_pair_trace pair_trace_no_sat(int other, bool aabb)
 // FLOORB = true : a walker body A against the static floor (scene constants)
 // `want`: this env takes part (candidate exists at this position of its list order).
 // `sep_axis` (may be null): receives the index (0..11, A's edges then B's) of the first separating axis this lane found
-// VOTE: 1 = one vote per SAT round with an early stop, 0 = straight-line rounds and one vote at the end, -1 = by layout (see kVote)
+// BY_LAYOUT: true = the SAT rounds vote or not by layout (see kVote), false = straight-line rounds and one vote at the end
 // KNOWN_HIT: the caller has already established that the bounding boxes overlap (stage 1 of the compacting kernel)
-template <class EV, int G, bool TRACE, bool FLOORB, int VOTE = -1, bool KNOWN_HIT = false, bool SHARED_CONTACTS = false>
+template <class EV, int G, bool TRACE, bool FLOORB, bool BY_LAYOUT = true, bool KNOWN_HIT = false>
 __device__ __forceinline__ void resolve_pair(EV& e, bool want, int A, int B, wb_pair_trace* tr, int* sep_axis = nullptr) {
   const FloorConst& fl = *e.fl;
   float2 PA[6], PB[6];
@@ -563,7 +473,7 @@ __device__ __forceinline__ void resolve_pair(EV& e, bool want, int A, int B, wb_
     // rare) the three rounds are fully unrolled WITHOUT votes: a straight-line block lets the rounds' long dependency chains
     // (edge -> 1/sqrt -> 12 dot products -> min/max tree) overlap; the separation flags meet in one vote after the last round.
     // Measured at 4096 walkers: G = 4 0.472 -> 0.452 ms per env-step; G = 8 (throughput bound) 0.474 -> 0.596, so it keeps the votes.
-    constexpr bool kVote = VOTE < 0 ? (G != 4) : (VOTE != 0);
+    constexpr bool kVote = BY_LAYOUT && G != 4;
     bool my_sep = false;
     auto accumulate = [&](bool use, float2 axis, int axis_idx, float omin, float omax, float tmin, float tmax) {
       const float2 dd = vsub(mk2(tmax, omax), mk2(omin, tmin));  // (tmax - omin, omax - tmin)
@@ -648,14 +558,14 @@ __device__ __forceinline__ void resolve_pair(EV& e, bool want, int A, int B, wb_
         for (int r = 0; r < 12; r += G)
           if (round_pole(r)) break;
       }
-    } else {
+    } else {  // (unrolled by 6, not fully: G = 1 gives the pole loop 12 trips; rolled rounds measured slower, DESIGN §4.1)
       if (FLOORB) {
-#pragma unroll kSatUnroll
+#pragma unroll 6
         for (int r = 0; r < 6; r += G) round_a_vs_floor(r);
-#pragma unroll kSatUnroll
+#pragma unroll 6
         for (int r = 0; r < 4; r += G) round_floor_vs_a(r);
       } else {
-#pragma unroll kSatUnroll
+#pragma unroll 6
         for (int r = 0; r < 12; r += G) round_pole(r);
       }
       sep = group_any<EV, G>(e, my_sep);
@@ -664,9 +574,9 @@ __device__ __forceinline__ void resolve_pair(EV& e, bool want, int A, int B, wb_
 #ifdef WB_PHASE_PROFILE
     rp_t1 = prof_clock();
 #endif
-    if constexpr (SHARED_CONTACTS && G > 1 && !TRACE) {
-      if (__any_sync(kFull, colliding)) contact_stage_shared<EV, G>(e.col, e.live, colliding, A, B, FLOORB, depth, idx, normal);
-    } else if (__any_sync(kFull, colliding)) {
+    // the contact stage stays inlined in every caller: one shared non-inlined copy for the compacting kernel's two drains
+    // measured slower, DESIGN §4.2
+    if (__any_sync(kFull, colliding)) {
       if (G > 1) {
 #pragma unroll
         for (int m = 1; m < G; m <<= 1) {
@@ -867,9 +777,8 @@ __device__ __forceinline__ void body_step(EV& e, bool on, int b, float dt, wb_pa
 //           RLL's candidates
 //   slot 1  LLU on the left half, RLU on the right half
 // Every body still meets its candidates in list order with the values the sequential sweep gives it, so the result is the
-// sequential one bit for bit.  -DWB_BODY_SLOT=1 builds the three-slot sweep instead (same-box A/B).  With G = 2 (4 lanes per
-// walker) the left half would move each of LLL and the Body on one lane in six rounds instead of three: measured slower
-// (contact_stress +2 %), so that layout keeps the three-slot sweep.
+// sequential one bit for bit.  With G = 2 (4 lanes per walker) the left half would move each of LLL and the Body on one lane
+// in six rounds instead of three: measured slower (contact_stress +2 %), so that layout keeps the three-slot sweep.
 template <class EV, int G, bool TRACE>
 __device__ __forceinline__ void legs_sweep(EV& e, bool left, float dt, wb_pair_trace* tr_base) {
   static_assert(G >= 4, "two or more lanes per body in slot 0");
@@ -899,7 +808,7 @@ __device__ __forceinline__ void legs_sweep(EV& e, bool left, float dt, wb_pair_t
       if (TRACE) {
         if (tr && e.live && left && e.gsub == 0 && !body_hit) *tr = pair_trace_no_sat(FLOOR, false);
       }
-      if (hits != 0u) resolve_pair<EV, G, TRACE, true, -1, true>(e, left && body_hit, left ? BODY : RLL, FLOOR, tr);
+      if (hits != 0u) resolve_pair<EV, G, TRACE, true, true, true>(e, left && body_hit, left ? BODY : RLL, FLOOR, tr);
     }
     resolve_candidates<EV, G, TRACE>(e, e.live, seg, tr_base);
   }
@@ -1147,9 +1056,9 @@ __global__ void __launch_bounds__(32, (L <= 4 || L == 16) ? 16 : 8) physics_lane
         const int leg = e.sub / G;
         e.gsub = e.sub % G;
         e.gshift = col * L + leg * G;
-        if constexpr (G >= 4 && !WB_BODY_SLOT) {
+        if constexpr (G >= 4) {
           legs_sweep<EV, G, TRACE>(e, leg == 0, dt, pt);
-        } else {  // three slots: (LLL | RLL), (LLU | RLU), (Body | idle)  (G <= 2, or -DWB_BODY_SLOT=1)
+        } else {  // three slots: (LLL | RLL), (LLU | RLU), (Body | idle)
 #pragma unroll 1
           for (int k = 0; k < 3; k++) {
             const bool on = e.live && (leg == 0 || k < 2);
@@ -1292,10 +1201,10 @@ static cudaError_t launch_l(const PhysicsParams& p, bool trace, cudaStream_t str
 //   stage 1  every thread, for ITS walker: the cheap, common part -- integrate the body; for a leg pair test the separating
 //            axis that separated this pair last time (temporal coherence; any order of the axis tests gives the reference's
 //            result: if one axis separates, SATCollision.IsColliding is false whatever the others say), then the AABBs; for
-//            a floor pair the AABBs (and the Collided latch); for a joint the gap.  Walkers that need the expensive part
-//            push an item (walker, body / joint) onto a queue in shared memory.
+//            a floor pair the AABBs (and the Collided latch).  Walkers that need the expensive part push an item (walker,
+//            body) onto a queue in shared memory.  (Joints run whole in the owning thread, see joint_in_thread.)
 //   stage 2  after a CTA barrier, the queued items are processed DENSELY: thread t takes item t (any thread can work on any
-//            walker: the state columns live in shared memory), runs the full resolve_pair / joint_step of the plain kernel
+//            walker: the state columns live in shared memory), runs the full resolve_pair of the plain kernel
 //            on that walker's columns and records the separating axis it found, if any, for the next substep (the hints
 //            also survive from launch to launch: PhysicsParams::axis_cache).
 // Left and right leg are swept in the same phase (they share no mutable state, see the leg split above), which halves the
@@ -1367,7 +1276,6 @@ struct Shared {
   FloorConst floor;
   unsigned char axis[4 * kE];   // last separating axis per ordered leg pair {LLL->LLU, LLU->LLL, RLL->RLU, RLU->RLL}
   unsigned short queue[3 * kE];  // a floor round holds at most three items per walker (two leg segments + the Body)
-  unsigned char jq[4 * kE];      // per-warp item lists of the compacted joint passes (128 slots per warp: lane | joint << 5)
   int count[2];  // ping-pong: the counter of the next round is cleared while the current one drains
   unsigned long long stage_bar;  // mbarrier of the bulk-copy staging
 #ifdef WB_PHASE_PROFILE
@@ -1458,43 +1366,9 @@ __device__ __noinline__ bool floor_pair_needs_work(int col, int A) {
   return aabb_hit(amin, amax, e.fl->bb_min, e.fl->bb_max);
 }
 
-// RigidBody.StepLinearVelocity / StepAngularVelocity / Skeleton.Move / Rotate of one body (the first half of body_step)
-template <class EV>
-__device__ __forceinline__ void integrate_body_inl(const EV& e, int b, float dt) {
-  float2 v = V2(e, kV2Vel + b);
-  v = vadd(v, vmul(mk2(0.0f, 980.0f), dt));
-  const float2 d = vmul(v, dt);
-  const float w = F1(e, kFOmega + b);
-  const float theta = fmul(w, dt);
-  float ang = fadd(F1(e, kFAngle + b), theta);
-  const float PI_F = 3.14159274f, TAU_F = 6.28318548f;
-  if (ang > PI_F) ang = fsub(ang, TAU_F);
-  else if (ang < -PI_F) ang = fadd(ang, TAU_F);
-  float m11, m12;
-  rotz(theta, m11, m12);
-  const float2 cen = vadd(V2(e, kV2Cen + b), d);
-#pragma unroll
-  for (int i = 0; i < 6; i++) {
-    float2 p = vadd(V2(e, b * 6 + i), d);
-    p = vsub(p, cen);
-    const float2 t = vrotate(p, m11, m12);
-    V2(e, b * 6 + i) = vadd(t, cen);
-  }
-  V2(e, kV2Cen + b) = cen;
-  V2(e, kV2Vel + b) = v;
-  F1(e, kFAngle + b) = ang;
-}
-template <int kE>
-__device__ __noinline__ void integrate_body(int col, int b, float dt) {
-  Env<1, kE> e;
-  env_for_column(e, shm<kE>(), col, true);
-  integrate_body_inl(e, b, dt);
-}
-// the same, and the bounding-box test against the floor on the NEW vertices while they are still in registers (what
-// floor_pair_needs_work would reload and recompute right afterwards for a floor-first walker); -DWB_FUSED_FLOOR_TEST=0: separate calls
-#ifndef WB_FUSED_FLOOR_TEST
-#define WB_FUSED_FLOOR_TEST 1
-#endif
+// RigidBody.StepLinearVelocity / StepAngularVelocity / Skeleton.Move / Rotate of one body (the first half of body_step), and
+// the bounding-box test against the floor on the NEW vertices while they are still in registers (what floor_pair_needs_work
+// would reload and recompute right afterwards for a floor-first walker)
 template <int kE>
 __device__ __noinline__ bool integrate_body_floor_test(int col, int b, float dt) {
   Env<1, kE> e;
@@ -1528,16 +1402,11 @@ __device__ __noinline__ bool integrate_body_floor_test(int col, int b, float dt)
   return aabb_hit(amin, amax, e.fl->bb_min, e.fl->bb_max);
 }
 
-
 // Joints: every thread runs Joint.Step for its OWN walker's four joints, in creation order, instead of three queue rounds.  A joint
 // needs correcting in ~20 % of the substeps and its chain is short (~120 instructions), so a warp executes all four chains at
 // 20 % lane density -- more issued instructions than the dense drain (+6 %), but three rounds (six barriers, three waits for
-// the slowest warp) fewer per substep: 262144 walkers 4.26 -> 4.05 ms per env-step (profiles/ab_experiments_r2.log).
-// -DWB_JOINTS_INTHREAD=0 restores the queue rounds; =2 merges joints 1 and 2 (disjoint bodies) into one function with two
-// independent instruction streams (measured slower: 4.23 ms).
-#ifndef WB_JOINTS_INTHREAD
-#define WB_JOINTS_INTHREAD 1
-#endif
+// the slowest warp) fewer per substep: 262144 walkers 4.26 -> 4.05 ms per env-step (profiles/ab_experiments_r2.log).  Two joints
+// merged into one function, static joint indices and warp-level joint passes all measured slower, DESIGN §4.2.
 template <int kE>
 __device__ __noinline__ void joint_in_thread(int col, int k) {
   Env<1, kE> e;
@@ -1545,136 +1414,14 @@ __device__ __noinline__ void joint_in_thread(int col, int k) {
   const int A = (0x4122 >> (4 * k)) & 0xF, B = (0x3041 >> (4 * k)) & 0xF;
   joint_step<Env<1, kE>, false>(e, A, k < 2 ? 1 : 2, B, k < 2 ? 4 : 3, nullptr);
 }
-// the same with the joint index known at compile time (static shared-memory offsets; -DWB_JOINTS_INTHREAD=4, experiment)
-template <int kE, int K>
-__device__ __noinline__ void joint_in_thread_static(int col) {
-  Env<1, kE> e;
-  env_for_column(e, shm<kE>(), col, true);
-  constexpr int A = (0x4122 >> (4 * K)) & 0xF, B = (0x3041 >> (4 * K)) & 0xF;
-  joint_step<Env<1, kE>, false>(e, A, K < 2 ? 1 : 2, B, K < 2 ? 4 : 3, nullptr);
-}
 
-// joints (Body, RLU) and (LLU, LLL) -- k = 1, 2 -- touch disjoint bodies: one early-out for both and two independent instruction
-// streams in one function (-DWB_JOINTS_INTHREAD=2)
-template <int kE>
-__device__ __noinline__ void joint_pair_in_thread(int col) {
-  using EV = Env<1, kE>;
-  EV e;
-  env_for_column(e, shm<kE>(), col, true);
-  struct J {
-    int A, ia, B, ib;
-    float2 pA, pB, ab;
-    float depth;
-    bool active;
-  } j[2];
-#pragma unroll
-  for (int q = 0; q < 2; q++) {
-    const int k = q + 1;
-    j[q].A = (0x4122 >> (4 * k)) & 0xF;
-    j[q].B = (0x3041 >> (4 * k)) & 0xF;
-    j[q].ia = k < 2 ? 1 : 2;
-    j[q].ib = k < 2 ? 4 : 3;
-    j[q].pA = V2(e, j[q].A * 6 + j[q].ia);
-    j[q].pB = V2(e, j[q].B * 6 + j[q].ib);
-    j[q].ab = vsub(j[q].pB, j[q].pA);
-    j[q].depth = fsqrt(fadd(fmul(j[q].ab.x, j[q].ab.x), fmul(j[q].ab.y, j[q].ab.y)));
-    j[q].active = !(j[q].depth < 0.1f);
-  }
-  if (!__any_sync(kFull, j[0].active || j[1].active)) return;
-  float2 n[2];
-#pragma unroll
-  for (int q = 0; q < 2; q++) n[q] = vnormalize_fast(j[q].ab);
-#pragma unroll
-  for (int q = 0; q < 2; q++) {  // Joint.Step, Joint.cs:31-41 (see joint_step above)
-    const float2 dA = vhalf(vmul(n[q], j[q].depth));
-    const float2 dB = vhalf(vmul(vneg(n[q]), j[q].depth));
-    BodyDyn X = load_dyn(e, j[q].B);
-    BodyDyn Y = load_dyn(e, j[q].A);
-    move_bodies<EV, 1>(e, j[q].active, j[q].A, dA, true, j[q].B, dB);
-    X.c = vadd(X.c, dB);
-    Y.c = vadd(Y.c, dA);
-    const float2 contact = vhalf(vadd(vadd(j[q].pA, dA), vadd(j[q].pB, dB)));
-    float2 rX, rY;
-    float imp;
-    calculate_impulse(X, Y, contact, fadd(1.0f, 1.0f), n[q], rX, rY, imp);
-    apply_impulses(X, Y, n[q], imp, rX, rY);
-    if (j[q].active) {
-      store_dyn(e, j[q].B, X);
-      store_dyn(e, j[q].A, Y);
-    }
-  }
-}
-
-// -DWB_JOINTS_INTHREAD=3: the four joints of a warp's 32 walkers as warp-level passes.  The reference steps the joints in creation
-// order, but two joints only depend on each other through a shared body AND only if the earlier one is active (an inactive joint
-// changes nothing): joint 1 (Body, RLU) and joint 2 (LLU, LLL) wait for joint 0 (Body, LLU), joint 3 (RLU, RLL) waits for joint 1.
-// Every pass the owning lane tests the joints of its walker whose predecessor is settled (inactive, or processed in an earlier
-// pass); the active ones of the whole warp -- on average 0.68 x 32 in the first pass -- are listed in shared memory and each
-// lane runs ONE of them (any lane can work on any walker of the warp: the state is in shared-memory columns).  Two or three
-// executions of the ~200-instruction correction per substep instead of four, bit-identical results.
-template <int kE>
-__device__ __noinline__ void joints_compacted(int col) {
-  using EV = Env<1, kE>;
-  Shared<kE>& S = shm<kE>();
-  EV own;
-  env_for_column(own, S, col, true);
-  const int lane = col & 31, col0 = col & ~31;
-  unsigned char* list = S.jq + 4 * col0;
-  unsigned todo = 0xFu;
-#pragma unroll 1
-  while (__any_sync(kFull, todo != 0u)) {
-    unsigned act = 0u;
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const int pred = k == 3 ? 1 : 0;
-      if (((todo >> k) & 1u) && (k == 0 || !((todo >> pred) & 1u))) {
-        const int A = (0x4122 >> (4 * k)) & 0xF, B = (0x3041 >> (4 * k)) & 0xF;
-        const float2 ab = vsub(V2(own, B * 6 + (k < 2 ? 4 : 3)), V2(own, A * 6 + (k < 2 ? 1 : 2)));
-        const float depth = fsqrt(fadd(fmul(ab.x, ab.x), fmul(ab.y, ab.y)));
-        if (!(depth < 0.1f)) act |= 1u << k;   // stays in todo until it has been processed
-        else todo &= ~(1u << k);               // inactive: settled, its successors may be tested in this very pass
-      }
-    }
-    int total = 0;
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const unsigned m = __ballot_sync(kFull, (act >> k) & 1u);
-      if ((act >> k) & 1u) list[total + __popc(m & ((1u << lane) - 1u))] = (unsigned char)(lane | (k << 5));
-      total += __popc(m);
-    }
-    __syncwarp();
-#pragma unroll 1
-    for (int base = 0; base < total; base += 32) {
-      const bool valid = base + lane < total;
-      const int item = valid ? list[base + lane] : 0;
-      const int k = item >> 5;
-      EV e;
-      env_for_column(e, S, col0 + (item & 31), valid);
-      const int A = (0x4122 >> (4 * k)) & 0xF, B = (0x3041 >> (4 * k)) & 0xF;
-      joint_step<EV, false>(e, A, k < 2 ? 1 : 2, B, k < 2 ? 4 : 3, nullptr);
-    }
-    __syncwarp();  // the corrections are visible to the owners' next tests; the list may be rewritten
-    todo &= ~act;
-  }
-}
-
-enum { kItemPole = 0, kItemFloor = 1, kItemJoint = 2 };
-// SAT rounds of the queued items: 16 items share a warp, so an early stop (all of them separated) practically never happens
-#ifndef WB_DRAIN_VOTE
-#define WB_DRAIN_VOTE 0
-#endif
-constexpr int kDrainVote = WB_DRAIN_VOTE;
+enum { kItemPole = 0, kItemFloor = 1 };
 
 // stage 2: the queued items, densely, kG lanes per item (the lanes split the SAT axes and the vertices of the moves exactly
 // like the L > 1 layouts of the plain kernel; with ~15-20 % of the walkers queued per round this keeps most warps of the CTA
-// busy and roughly halves the latency of the round).  Item = walker column | payload << 10.
+// busy and roughly halves the latency of the round).  Item = walker column | payload << 10.  Four lanes per floor item
+// measured slower, DESIGN §4.2.
 constexpr int kG = 2;
-// lanes per FLOOR item (-DWB_FLOOR_G=4, experiment): a floor round queues few items (~27 of 256 walkers), so wider groups still
-// fit one pass and shorten its SAT (10 axes: 5 rounds with two lanes, 3 with four)
-#ifndef WB_FLOOR_G
-#define WB_FLOOR_G 2
-#endif
-constexpr int kGFloor = WB_FLOOR_G;
 
 template <int G, int kE>
 __device__ __forceinline__ void group_env_for_column(Env<G, kE>& e, Shared<kE>& S, int col, bool live) {
@@ -1684,75 +1431,36 @@ __device__ __forceinline__ void group_env_for_column(Env<G, kE>& e, Shared<kE>& 
   e.sub = threadIdx.x % G;
   e.gsub = e.sub;
   e.gshift = ((threadIdx.x & 31) / G) * G;
-  e.col = col;
   e.live = live;
   e.flags = 0;
   set_materials(e, S.mtab[S.wmat[col]], S.mtab[S.fmat[col]]);
-}
-template <int G, int kE>
-__device__ __forceinline__ void group_env_by_col(pl::Env<G, kE>& e, int col, bool live) {
-  group_env_for_column<G, kE>(e, shm<kE>(), col, live);
 }
 
 template <int KIND, int kE>
 __device__ __noinline__ void drain(int parity) {
   Shared<kE>& S = shm<kE>();
-  constexpr int G = KIND == kItemFloor ? kGFloor : kG;
-  using EVG = Env<G, kE>;
+  using EVG = Env<kG, kE>;
   const int count = S.count[parity];
-  const int warp_base = (threadIdx.x >> 5) * (32 / G), lane = threadIdx.x & 31;
+  const int warp_base = (threadIdx.x >> 5) * (32 / kG), lane = threadIdx.x & 31;
 #pragma unroll 1
-  for (int base = warp_base; base < count; base += kE / G) {
-    const int slot = base + lane / G;
+  for (int base = warp_base; base < count; base += kE / kG) {
+    const int slot = base + lane / kG;
     const bool valid = slot < count;
     const int item = valid ? S.queue[slot] : 0;
     const int col = item & 1023, payload = item >> 10;
     EVG q;
-    group_env_for_column<G, kE>(q, S, col, valid);
+    group_env_for_column<kG, kE>(q, S, col, valid);
+    // straight-line SAT rounds (BY_LAYOUT = false): 16 items share a warp, so an early stop (all of them separated) practically
+    // never happens
     if (KIND == kItemPole) {
       int sep_axis = -1;
-      resolve_pair<EVG, G, false, false, kDrainVote, true, WB_SHARED_CONTACTS != 0>(q, valid, payload, partner_of(payload), nullptr, &sep_axis);
+      resolve_pair<EVG, kG, false, false, false, true>(q, valid, payload, partner_of(payload), nullptr, &sep_axis);
       // the lane that saw the lowest separating axis of the group records it (any separating axis is a valid cache entry)
       if (valid && sep_axis >= 0) S.axis[pair_slot(payload) * kE + col] = (unsigned char)sep_axis;
-    } else if (KIND == kItemFloor) {
-      resolve_pair<EVG, G, false, true, kDrainVote, true, WB_SHARED_CONTACTS != 0>(q, valid, payload, FLOOR, nullptr);
     } else {
-      const int k = payload;
-      const int A = (0x4122 >> (4 * k)) & 0xF, B = (0x3041 >> (4 * k)) & 0xF;
-      joint_step<EVG, false>(q, A, k < 2 ? 1 : 2, B, k < 2 ? 4 : 3, nullptr);
+      resolve_pair<EVG, kG, false, true, false, true>(q, valid, payload, FLOOR, nullptr);
     }
   }
-}
-
-// The upper legs' floor round (second leg phase) is sparse: an upper leg only reaches the floor when the walker has fallen, ~2.5
-// items per 256 walkers and substep, yet as a queue round it costs every warp of the CTA two barriers and the wait for one full
-// floor chain.  -DWB_F1_INWARP=1: the owning WARP resolves its own items instead (8 lanes per item, four items per pass; the
-// state columns are in shared memory, so any lane can work on any walker of the warp), no CTA barrier; warps without an item --
-// most of them -- skip the stage on a single vote.
-#ifndef WB_F1_INWARP
-#define WB_F1_INWARP 0
-#endif
-template <int kE>
-__device__ __noinline__ void warp_floor_items(bool f0, int b0, bool f1, int b1) {
-  const unsigned m0 = __ballot_sync(kFull, f0), m1 = __ballot_sync(kFull, f1);
-  if ((m0 | m1) == 0u) return;
-  __syncwarp();  // the owners' integration writes are visible to the lanes that take their walkers
-  Shared<kE>& S = shm<kE>();
-  constexpr int G = 8;
-  using EVG = Env<G, kE>;
-  const int lane = threadIdx.x & 31, col0 = threadIdx.x & ~31;
-  const int n0 = __popc(m0), total = n0 + __popc(m1);
-#pragma unroll 1
-  for (int base = 0; base < total; base += 32 / G) {
-    const int idx = base + lane / G;  // items: the b0 bodies in lane order, then the b1 bodies (all independent of each other)
-    const bool valid = idx < total;
-    const bool first = idx < n0;
-    const unsigned src = valid ? __fns(first ? m0 : m1, 0, (first ? idx : idx - n0) + 1) : 0u;
-    EVG q;
-    group_env_for_column<G, kE>(q, S, col0 + (int)src, valid);
-    resolve_pair<EVG, G, false, true, -1, true>(q, valid, first ? b0 : b1, FLOOR, nullptr);
-  }
-  __syncwarp();
 }
 
 template <int kE>
@@ -1856,12 +1564,6 @@ __global__ void __launch_bounds__(kE, kE == 192 ? 3 : (kE == 160 ? 3 : 512 / kE)
     const bool any_first = scope_any<kE>(floor_first);
     const bool any_last = scope_any<kE>(!floor_first);
 
-    auto joint_gap_active = [&](int k) {
-      const int A = (0x4122 >> (4 * k)) & 0xF, B = (0x3041 >> (4 * k)) & 0xF;
-      const float2 ab = vsub(V2(e, B * 6 + (k < 2 ? 4 : 3)), V2(e, A * 6 + (k < 2 ? 1 : 2)));
-      const float depth = fsqrt(fadd(fmul(ab.x, ab.x), fmul(ab.y, ab.y)));
-      return !(depth < 0.1f);
-    };
     // one queue round: (stage 1 already pushed) barrier, drain, barrier; the other counter is cleared in between
     int parity = 0;
     WB_PROF_DECL;
@@ -1908,29 +1610,7 @@ __global__ void __launch_bounds__(kE, kE == 192 ? 3 : (kE == 160 ? 3 : 512 / kE)
 
 #pragma unroll 1
     for (int it = 0; it < p.iterations; it++) {
-#if WB_JOINTS_INTHREAD == 4
-      joint_in_thread_static<kE, 0>(tid);
-      joint_in_thread_static<kE, 1>(tid);
-      joint_in_thread_static<kE, 2>(tid);
-      joint_in_thread_static<kE, 3>(tid);
-#elif WB_JOINTS_INTHREAD == 3
-      joints_compacted<kE>(tid);
-#elif WB_JOINTS_INTHREAD == 2
-      joint_in_thread<kE>(tid, 0);
-      joint_pair_in_thread<kE>(tid);
-      joint_in_thread<kE>(tid, 3);
-#elif WB_JOINTS_INTHREAD
       for (int k = 0; k < 4; k++) joint_in_thread<kE>(tid, k);
-#else
-      // ---- joints in creation order; (Body,RLU) and (LLU,LLL) touch disjoint bodies and share a round
-      push(S, parity, joint_gap_active(0), tid | (0 << 10));
-      round([&] { drain<kItemJoint, kE>(parity); });
-      push(S, parity, joint_gap_active(1), tid | (1 << 10));
-      push(S, parity, joint_gap_active(2), tid | (2 << 10));
-      round([&] { drain<kItemJoint, kE>(parity); });
-      push(S, parity, joint_gap_active(3), tid | (3 << 10));
-      round([&] { drain<kItemJoint, kE>(parity); });
-#endif
       // ---- body sweep: {LLL, RLL, Body}, then {LLU, RLU}; per leg segment [floor if floor-first] [leg partner] [floor if
       //      floor-last].  The Body only ever meets the floor (Walker.cs:204-209), so its step is independent of both legs during
       //      the sweep: it is integrated with the first pair and its floor item rides in that pair's first floor round instead
@@ -1940,39 +1620,21 @@ __global__ void __launch_bounds__(kE, kE == 192 ? 3 : (kE == 160 ? 3 : 512 / kE)
         const int b0 = ph == 0 ? LLL : LLU;
         const int b1 = ph == 0 ? RLL : RLU;
         bool body_pending = ph == 0;
-#if WB_FUSED_FLOOR_TEST
         const bool hit0 = integrate_body_floor_test<kE>(tid, b0, dt);
         const bool hit1 = integrate_body_floor_test<kE>(tid, b1, dt);
         const bool hitb = body_pending && integrate_body_floor_test<kE>(tid, BODY, dt);  // (ph is uniform: no divergent call)
-#else
-        integrate_body<kE>(tid, b0, dt);
-        integrate_body<kE>(tid, b1, dt);
-        if (body_pending) integrate_body<kE>(tid, BODY, dt);
-#endif
         if (any_first) {
-#if WB_FUSED_FLOOR_TEST
+          // (the upper legs' sparse floor round stays a queue round: resolving it in the owning warp measured slower, DESIGN §4.2)
           const bool f0 = floor_first && hit0, f1 = floor_first && hit1;
-#else
-          const bool f0 = floor_first && floor_pair_needs_work<kE>(tid, b0), f1 = floor_first && floor_pair_needs_work<kE>(tid, b1);
-#endif
           e.flags |= (f0 ? 1 << b0 : 0) | (f1 ? 1 << b1 : 0);
-          if (WB_F1_INWARP && ph == 1) {
-            warp_floor_items<kE>(f0, b0, f1, b1);
-          } else {
-            push(S, parity, f0, tid | (b0 << 10));
-            push(S, parity, f1, tid | (b1 << 10));
-            if (body_pending) {
-#if WB_FUSED_FLOOR_TEST
-              const bool fb = hitb;
-#else
-              const bool fb = floor_pair_needs_work<kE>(tid, BODY);
-#endif
-              if (fb) e.flags |= 1 << BODY;
-              push(S, parity, fb, tid | (BODY << 10));
-              body_pending = false;
-            }
-            round([&] { drain<kItemFloor, kE>(parity); });
+          push(S, parity, f0, tid | (b0 << 10));
+          push(S, parity, f1, tid | (b1 << 10));
+          if (body_pending) {
+            if (hitb) e.flags |= 1 << BODY;
+            push(S, parity, hitb, tid | (BODY << 10));
+            body_pending = false;
           }
+          round([&] { drain<kItemFloor, kE>(parity); });
         }
         push(S, parity, pole_pair_needs_work<kE>(tid, b0, partner_of(b0)), tid | (b0 << 10));
         push(S, parity, pole_pair_needs_work<kE>(tid, b1, partner_of(b1)), tid | (b1 << 10));
