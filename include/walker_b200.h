@@ -414,6 +414,21 @@ int32_t wb_population_get_grads(wb_population* pop, int32_t agent, float* flat_h
 /* agent a's Adam moments m / v [n_actor + n_critic] and the step counters [n_dense] of its dense layers (actor layers, then critic
  * layers; DenseLayer.cs:15-20) */
 int32_t wb_population_get_adam(wb_population* pop, int32_t agent, float* m_host, float* v_host, int32_t* steps_host);
+/* the mirror of wb_population_get_adam (and of wb_policy_set_adam): agent a's m / v [n_actor + n_critic] and step counters
+ * [n_dense] (DenseLayer.cs:15-20) */
+int32_t wb_population_set_adam(wb_population* pop, int32_t agent, const float* m_host, const float* v_host, const int32_t* steps_host);
+/* agent a's wb_hyperparams (Hyperparameters.cs:83-121; set mirrors wb_policy_set_hyperparams).  The next call that acts or trains
+ * with the agent uses them.  batch_size < 1: WB_ERR_INVALID, nothing changes. */
+int32_t wb_population_set_hyperparams(wb_population* pop, int32_t agent, const wb_hyperparams* hp);
+int32_t wb_population_get_hyperparams(const wb_population* pop, int32_t agent, wb_hyperparams* hp_out);
+/* Population-based training's exploit step, an extension with no reference counterpart (the reference's agents are independent):
+ * for i < n_pairs, agent dst_host[i] becomes a copy of agent src_host[i] -- its weights, Adam m / v and step counters, bit for
+ * bit -- with the hyper-parameters hp_host[i] (hp_host NULL: src's).  dst keeps its own gradient buffer (scratch of its last
+ * mini-batch) and its own count of trained episodes (which keys its device-drawn mini-batches).  Enqueue only: one launch on the
+ * population's stream, after whatever is already enqueued there.  Refused with WB_ERR_INVALID before anything changes:
+ * n_pairs < 1, an agent out of range, dst == src, a dst listed twice, an agent that is both a src and a dst, a batch_size < 1. */
+int32_t wb_population_copy_agents(wb_population* pop, int32_t n_pairs, const int32_t* dst_host, const int32_t* src_host,
+                                  const wb_hyperparams* hp_host);
 /* PPOAgent.SampleActions (PPOAgent.cs:381-398) for n == P walkers, walker w with agent w, with the two System.Random uniforms of
  * each Box-Muller draw injected (NormalDistribution.cs:12-32): states [n][state], uniforms [n][act][2] -> actions, logp [n][act],
  * mean [n][act] or NULL.  Row w equals wb_policy_sample of agent w. */

@@ -9,7 +9,7 @@ from .env import (DT_FRAME, MATERIALS, Carpet, EnvBatch, Environment, Ice, IMate
 from . import dist  # noqa: F401
 from .ppo import *  # noqa: F401,F403
 from .loop import VectorPPO  # noqa: F401
-from .population import IndependentPPO, PPOPopulation, default_seeds  # noqa: F401
+from .population import PBT, IndependentPPO, PPOPopulation, default_seeds  # noqa: F401
 from .scene import (CreateCreature, CreateFloor, CreateRoughFloor, Hexagon, Hull, IObject, Joint, Pole, Scene, Square,  # noqa: F401
                     TerrainEnvBatch, Triangle)
 from .settings import DeserializeJson, SerializeJson, Settings  # noqa: F401

@@ -162,6 +162,10 @@ def lib() -> C.CDLL:
         "wb_population_get_weights": (C.c_int32, [vp, C.c_int32, vp]),
         "wb_population_get_grads": (C.c_int32, [vp, C.c_int32, vp]),
         "wb_population_get_adam": (C.c_int32, [vp, C.c_int32, vp, vp, vp]),
+        "wb_population_set_adam": (C.c_int32, [vp, C.c_int32, vp, vp, vp]),
+        "wb_population_set_hyperparams": (C.c_int32, [vp, C.c_int32, hpp]),
+        "wb_population_get_hyperparams": (C.c_int32, [vp, C.c_int32, hpp]),
+        "wb_population_copy_agents": (C.c_int32, [vp, C.c_int32, vp, vp, hpp]),
         "wb_population_sample": (C.c_int32, [vp, C.c_int32, vp, vp, vp, vp, vp]),
         "wb_population_act_dev": (C.c_int32, [vp, C.c_int32, vp, C.c_uint64, C.c_uint64, vp, vp, vp, vp]),
         "wb_population_train_trajectories": (C.c_int32, [vp, C.c_int32, vp, vp, C.c_int32] + [vp] * 10),

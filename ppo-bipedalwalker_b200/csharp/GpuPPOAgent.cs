@@ -416,5 +416,27 @@ public sealed class GpuPopulation : IDisposable
         }
     }
 
+    // population-based training (an extension: the reference's agents are independent).  Agent dst[i] becomes a copy of agent
+    // src[i] -- weights, Adam state and step counters -- with the hyper-parameters hp[i] (null: src's).  One kernel launch.
+    public void CopyAgents(int[] dst, int[] src, WbHyperparams[] hp = null)
+    {
+        if (dst.Length == 0 || dst.Length != src.Length || (hp != null && hp.Length != dst.Length))
+            throw new ArgumentException("dst, src and hp must have the same, positive length");
+        if (hp == null)
+        {
+            hp = new WbHyperparams[src.Length];
+            for (int i = 0; i < src.Length; i++)
+                Wb.Ok(Wb.wb_population_get_hyperparams(_population, src[i], ref hp[i]), "wb_population_get_hyperparams");
+        }
+        Wb.Ok(Wb.wb_population_copy_agents(_population, dst.Length, dst, src, ref hp[0]), "wb_population_copy_agents");
+    }
+
+    public void SetHyperparams(int agent, WbHyperparams hp) =>
+        Wb.Ok(Wb.wb_population_set_hyperparams(_population, agent, ref hp), "wb_population_set_hyperparams");
+
+    // one agent's Adam moments [actor | critic parameters] and per-dense-layer step counters (DenseLayer.cs:15-20)
+    public void SetAdam(int agent, float[] m, float[] v, int[] steps) =>
+        Wb.Ok(Wb.wb_population_set_adam(_population, agent, m, v, steps), "wb_population_set_adam");
+
     public void Dispose() => Wb.wb_population_destroy(_population);
 }

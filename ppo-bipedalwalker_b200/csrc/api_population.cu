@@ -33,7 +33,7 @@ struct wb_population {
   // staging of the host entries (grown on demand)
   float* d_stage = nullptr;
   size_t stage_bytes = 0;
-  // item table + Adam correction table of a train call: one pinned upload
+  // the table of a train call (items + Adam corrections) or a copy call (pairs + constants): one pinned upload
   char* h_tab = nullptr;
   char* d_tab = nullptr;
   size_t tab_bytes = 0;
@@ -51,6 +51,23 @@ static int32_t grow_stage(wb_population* p, size_t bytes) {
 }
 
 static size_t align16(size_t b) { return (b + 15) / 16 * 16; }
+
+// the pinned table of one call and its device copy, at least `bytes` long, once the previous call's upload has left the pinned copy
+static int32_t stage_table(wb_population* p, size_t bytes) {
+  if (!p->tab_copied) WB_CUDA(cudaEventCreateWithFlags(&p->tab_copied, cudaEventDisableTiming));
+  WB_CUDA(cudaEventSynchronize(p->tab_copied));
+  if (bytes > p->tab_bytes) {
+    if (p->h_tab) cudaFreeHost(p->h_tab);
+    cudaFree(p->d_tab);
+    p->h_tab = nullptr;
+    p->d_tab = nullptr;
+    p->tab_bytes = 0;
+    WB_CUDA(cudaHostAlloc(&p->h_tab, bytes, cudaHostAllocDefault));
+    WB_CUDA(cudaMalloc(&p->d_tab, bytes));
+    p->tab_bytes = bytes;
+  }
+  return WB_OK;
+}
 
 // one train call, validated and enqueued: items [n_items][4] = (agent, column, t0, length) in list order
 static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* items, int32_t ring_rows, int32_t columns, int32_t epochs,
@@ -91,18 +108,7 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
   const size_t item_bytes = align16(sizeof(PopItem) * n_items);
   const int nd = p->n_dense;
   const size_t tab_bytes = cta_bytes + item_bytes + sizeof(float) * 2 * nd * (size_t)steps;
-  if (!p->tab_copied) WB_CUDA(cudaEventCreateWithFlags(&p->tab_copied, cudaEventDisableTiming));
-  WB_CUDA(cudaEventSynchronize(p->tab_copied));  // (the previous call's upload has read the pinned copy)
-  if (tab_bytes > p->tab_bytes) {
-    if (p->h_tab) cudaFreeHost(p->h_tab);
-    cudaFree(p->d_tab);
-    p->h_tab = nullptr;
-    p->d_tab = nullptr;
-    p->tab_bytes = 0;
-    WB_CUDA(cudaHostAlloc(&p->h_tab, tab_bytes, cudaHostAllocDefault));
-    WB_CUDA(cudaMalloc(&p->d_tab, tab_bytes));
-    p->tab_bytes = tab_bytes;
-  }
+  if (int32_t rc = stage_table(p, tab_bytes)) return rc;
   // nothing fails below this line: the step counters and episode counters advance only for a call that is enqueued
   memcpy(p->h_tab, ctas.data(), sizeof(PopCta) * ctas.size());
   PopItem* tab_items = reinterpret_cast<PopItem*>(p->h_tab + cta_bytes);
@@ -329,6 +335,84 @@ int32_t wb_population_get_adam(wb_population* p, int32_t agent, float* m_host, f
   if (int32_t rc = copy_agent(p, agent, p->d_m, nullptr, m_host)) return rc;
   if (int32_t rc = copy_agent(p, agent, p->d_v, nullptr, v_host)) return rc;
   memcpy(steps_host, &p->iterations[(size_t)agent * p->n_dense], sizeof(int32_t) * p->n_dense);
+  return WB_OK;
+}
+
+int32_t wb_population_set_adam(wb_population* p, int32_t agent, const float* m_host, const float* v_host, const int32_t* steps_host) {
+  WB_REQUIRE(p && m_host && v_host && steps_host, "null argument");
+  if (int32_t rc = copy_agent(p, agent, p->d_m, m_host, nullptr)) return rc;
+  if (int32_t rc = copy_agent(p, agent, p->d_v, v_host, nullptr)) return rc;
+  memcpy(&p->iterations[(size_t)agent * p->n_dense], steps_host, sizeof(int32_t) * p->n_dense);
+  return WB_OK;
+}
+
+int32_t wb_population_set_hyperparams(wb_population* p, int32_t agent, const wb_hyperparams* hp) {
+  WB_REQUIRE(p && hp, "null argument");
+  WB_REQUIRE(agent >= 0 && agent < p->n, "agent outside the population");
+  WB_REQUIRE(hp->batch_size >= 1, "batch_size must be positive");
+  PopAgent c;
+  population_agent_consts(*hp, &c);
+  WB_CUDA(cudaMemcpyAsync(p->d_agents + agent, &c, sizeof(PopAgent), cudaMemcpyHostToDevice, p->stream));
+  WB_CUDA(cudaStreamSynchronize(p->stream));
+  p->hp[agent] = *hp;
+  return WB_OK;
+}
+
+int32_t wb_population_get_hyperparams(const wb_population* p, int32_t agent, wb_hyperparams* hp_out) {
+  WB_REQUIRE(p && hp_out, "null argument");
+  WB_REQUIRE(agent >= 0 && agent < p->n, "agent outside the population");
+  *hp_out = p->hp[agent];
+  return WB_OK;
+}
+
+int32_t wb_population_copy_agents(wb_population* p, int32_t n_pairs, const int32_t* dst_host, const int32_t* src_host,
+                                  const wb_hyperparams* hp_host) {
+  WB_REQUIRE(p && dst_host && src_host, "null argument");
+  WB_REQUIRE(n_pairs >= 1, "n_pairs must be at least 1");
+  // every dst distinct and never a src: the pairs are independent copies, in any order
+  enum : uint8_t { kNone, kDst, kSrc };
+  std::vector<uint8_t> role(p->n, kNone);
+  for (int32_t i = 0; i < n_pairs; i++) {
+    const int32_t d = dst_host[i], s = src_host[i];
+    if (d < 0 || d >= p->n) return fail(WB_ERR_INVALID, "pair %d: dst %d outside 0..%d", i, d, p->n - 1);
+    if (s < 0 || s >= p->n) return fail(WB_ERR_INVALID, "pair %d: src %d outside 0..%d", i, s, p->n - 1);
+    if (d == s) return fail(WB_ERR_INVALID, "pair %d: agent %d copies itself", i, d);
+    if (role[d] == kDst) return fail(WB_ERR_INVALID, "pair %d: dst %d is listed twice", i, d);
+    role[d] = kDst;
+    if (hp_host && hp_host[i].batch_size < 1) return fail(WB_ERR_INVALID, "pair %d: batch_size must be positive", i);
+  }
+  for (int32_t i = 0; i < n_pairs; i++)
+    if (role[src_host[i]] == kDst) return fail(WB_ERR_INVALID, "pair %d: agent %d is both a src and a dst", i, src_host[i]);
+  const size_t pair_bytes = align16(sizeof(int32_t) * 2 * n_pairs);
+  if (int32_t rc = stage_table(p, pair_bytes + sizeof(PopAgent) * n_pairs)) return rc;
+  int32_t* tab_pairs = reinterpret_cast<int32_t*>(p->h_tab);
+  PopAgent* tab_consts = reinterpret_cast<PopAgent*>(p->h_tab + pair_bytes);
+  std::vector<wb_hyperparams> hp(n_pairs);
+  for (int32_t i = 0; i < n_pairs; i++) {
+    tab_pairs[2 * i] = dst_host[i];
+    tab_pairs[2 * i + 1] = src_host[i];
+    hp[i] = hp_host ? hp_host[i] : p->hp[src_host[i]];
+    population_agent_consts(hp[i], &tab_consts[i]);
+  }
+  WB_CUDA(cudaMemcpyAsync(p->d_tab, p->h_tab, pair_bytes + sizeof(PopAgent) * n_pairs, cudaMemcpyHostToDevice, p->stream));
+  WB_CUDA(cudaEventRecord(p->tab_copied, p->stream));
+  PopCopyParams c{};
+  c.params = p->d_params;
+  c.m = p->d_m;
+  c.v = p->d_v;
+  c.agents = p->d_agents;
+  c.pairs = reinterpret_cast<const int32_t*>(p->d_tab);
+  c.consts = reinterpret_cast<const PopAgent*>(p->d_tab + pair_bytes);
+  c.n_pairs = n_pairs;
+  c.stride = p->stride;
+  WB_CUDA(launch_population_copy(c, p->stream));
+  p->launches++;
+  // the host half: dst's hyper-parameters and Adam step counters (the bias corrections); its episode counter stays its own
+  const int nd = p->n_dense;
+  for (int32_t i = 0; i < n_pairs; i++) {
+    p->hp[dst_host[i]] = hp[i];
+    memcpy(&p->iterations[(size_t)dst_host[i] * nd], &p->iterations[(size_t)src_host[i] * nd], sizeof(int32_t) * nd);
+  }
   return WB_OK;
 }
 

@@ -814,6 +814,29 @@ __global__ void __launch_bounds__(kMlpThreads, 1) population_episodes_kernel(con
   }
 }
 
+// Population-based training's exploit step: for every pair (dst, src), src's rows of the weights and both Adam moments become
+// dst's, and dst gets its new per-agent constants.  A pure HBM copy (3 x stride x 4 bytes read and written per pair), so the
+// grid is (chunks of kCopyThreads x kCopyIlp float4 per row x pairs, 3 arrays): one row spreads over several CTAs, and every
+// thread issues all its 16-byte loads before its first store.  The gradient row is scratch of the last mini-batch: not copied.
+__global__ void __launch_bounds__(kCopyThreads) population_copy_kernel(const PopCopyParams c) {
+  constexpr int kChunk = kCopyThreads * kCopyIlp;
+  const int row4 = c.stride / 4;
+  const int chunks = (row4 + kChunk - 1) / kChunk;
+  const int pair = blockIdx.x / chunks, first = (blockIdx.x - pair * chunks) * kChunk + threadIdx.x;
+  const int dst = c.pairs[2 * pair], src = c.pairs[2 * pair + 1];
+  float* base = blockIdx.y == 0 ? c.params : blockIdx.y == 1 ? c.m : c.v;
+  const float4* from = reinterpret_cast<const float4*>(base + (size_t)src * c.stride);
+  float4* to = reinterpret_cast<float4*>(base + (size_t)dst * c.stride);
+  if (blockIdx.y == 0 && first == 0) c.agents[dst] = c.consts[pair];
+  float4 r[kCopyIlp];
+#pragma unroll
+  for (int k = 0; k < kCopyIlp; k++)
+    if (first + k * kCopyThreads < row4) r[k] = from[first + k * kCopyThreads];
+#pragma unroll
+  for (int k = 0; k < kCopyIlp; k++)
+    if (first + k * kCopyThreads < row4) to[first + k * kCopyThreads] = r[k];
+}
+
 // The same recurrences over a time-major rollout buffer [T][N] of N lockstep environments (the reference trains on one
 // episode of one environment, PPOAgent.cs:147; here every environment contributes the fragments of its episodes that fall
 // inside the T-step segment).  One thread per environment, reverse scan; a step with done != 0 is the LAST step of its
@@ -979,6 +1002,12 @@ cudaError_t launch_population_episodes(const PopTrainParams& t, int n_ctas, cuda
     if (dev >= 0 && dev < 64) configured[dev] = true;
   }
   population_episodes_kernel<<<n_ctas, kMlpThreads, sizeof(PopSmem), stream>>>(t);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_population_copy(const PopCopyParams& c, cudaStream_t stream) {
+  const int chunks = (c.stride / 4 + kCopyThreads * kCopyIlp - 1) / (kCopyThreads * kCopyIlp);
+  population_copy_kernel<<<dim3((unsigned)(c.n_pairs * chunks), 3), kCopyThreads, 0, stream>>>(c);
   return cudaGetLastError();
 }
 

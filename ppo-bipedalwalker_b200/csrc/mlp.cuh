@@ -174,6 +174,20 @@ struct PopTrainParams {
   uint64_t seed;
 };
 cudaError_t launch_population_episodes(const PopTrainParams& t, int n_ctas, cudaStream_t stream);
+// population-based training: pair i copies agent src's rows of params / m / v (stride floats each, any topology) to agent dst and
+// writes dst's PopAgent.  Every dst differs from every src and from every other dst, so the copies are independent.
+constexpr int kCopyThreads = 256;
+constexpr int kCopyIlp = 4;  // independent 16-byte loads in flight per thread before its stores
+struct PopCopyParams {
+  float* params;           // [P][stride]
+  float* m;
+  float* v;
+  PopAgent* agents;        // [P]
+  const int32_t* pairs;    // [n_pairs][2] = (dst, src)
+  const PopAgent* consts;  // [n_pairs] dst's new constants
+  int32_t n_pairs, stride; // stride: a multiple of 4 floats
+};
+cudaError_t launch_population_copy(const PopCopyParams& c, cudaStream_t stream);
 
 int mlp_grid_for(int n, int sm_count);
 cudaError_t launch_mlp(const MlpParams& p, int grid, cudaStream_t stream);

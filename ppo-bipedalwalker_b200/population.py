@@ -10,6 +10,8 @@ Running the reference N times gives N independent learners, which is how seed st
   IndependentPPO  N walkers, N agents, the reference's episode semantics for every walker at once: no segments, no bootstrap; a
                   walker whose episode ended (Terminal, or steps > MaxTimesteps) trains its agent on the complete episode before it
                   acts again (Environment.Update -> TrainNetworks -> Reset).
+  PBT             population-based training for IndependentPPO: lagging agents copy a leader's weights and Adam state and
+                  perturb its hyper-parameters (an extension; the reference's agents are independent).
 """
 from __future__ import annotations
 
@@ -119,6 +121,34 @@ class PPOPopulation:
         check(lib().wb_population_get_adam(self._h, agent, ptr(m), ptr(v), ptr(steps)))
         return m, v, steps
 
+    def set_adam(self, agent: int, m, v, steps):
+        """The mirror of adam(): m / v [N_PARAMS], step counters [n_dense]."""
+        m, v = np.ascontiguousarray(m, np.float32), np.ascontiguousarray(v, np.float32)
+        steps = np.ascontiguousarray(steps, np.int32)
+        assert m.size == v.size == self.N_PARAMS and steps.size == self.n_dense
+        check(lib().wb_population_set_adam(self._h, agent, ptr(m), ptr(v), ptr(steps)))
+
+    def set_hyperparams(self, agent: int, hp: Hyperparams):
+        check(lib().wb_population_set_hyperparams(self._h, agent, C.byref(hp)))
+        self.hp[agent] = Hyperparams.from_buffer_copy(hp)
+
+    def copy_agents(self, pairs, hp=None):
+        """PBT's exploit step in one launch, enqueued on the population's stream: for each (dst, src) of pairs, dst's weights, Adam
+        m / v and step counters become src's, bit for bit, and its hyper-parameters hp[i] (hp None: src's).  dst keeps its own
+        generator rngs[dst], its count of trained episodes (which keys its device-drawn mini-batches) and its gradient buffer.  A
+        dst listed twice, dst == src or an agent that is both a src and a dst is refused."""
+        pairs = np.ascontiguousarray(np.asarray(pairs, np.int64).reshape(-1, 2), np.int32)
+        dst, src = np.ascontiguousarray(pairs[:, 0]), np.ascontiguousarray(pairs[:, 1])
+        hps = None
+        if hp is not None:
+            if len(hp) != len(pairs):
+                raise ValueError(f"{len(hp)} Hyperparams for {len(pairs)} pairs")
+            hps = (Hyperparams * len(pairs))(*hp)
+        check(lib().wb_population_copy_agents(self._h, len(pairs), ptr(dst), ptr(src), hps))
+        new = [Hyperparams.from_buffer_copy(hps[i] if hps is not None else self.hp[s]) for i, s in enumerate(src)]
+        for d, h in zip(dst, new):
+            self.hp[d] = h
+
     def Save(self, agent: int):
         """PPOAgent.Save (PPOAgent.cs:192-213) of one agent -> (critic lines, actor lines) of the two .weights files."""
         flat = self.get_weights(agent)
@@ -183,6 +213,89 @@ class PPOPopulation:
         return [(float(c), float(a)) for c, a in losses]
 
 
+PERTURBABLE = ("alpha", "beta1", "beta2", "adam_epsilon", "gamma", "lambda_", "epsilon", "log_std")  # wb_hyperparams field order
+DEFAULT_PERTURB = {"alpha": (1e-5, 1e-2), "epsilon": (0.05, 0.5), "log_std": (-3.0, 0.0)}
+
+
+class PBT:
+    """Population-based training schedule for IndependentPPO (host only: it decides the copies, IndependentPPO issues them).
+
+    History and score.  Each agent keeps the reward sums of the episodes it finished since its last copy, or since the start.
+    Its score is the float64 mean of the last `window` of them; an agent with fewer than `window` episodes is unranked.
+
+    Snapshot.  After the training of every env-step t with (t + 1) % interval == 0, a snapshot of the ranked agents is taken:
+    score descending, ties broken by the lower agent index first.  With m ranked agents, k = floor(fraction * m); the top set is
+    the first k, the bottom set the last k (0 <= fraction <= 0.5, so the two are disjoint).  It replaces the previous snapshot.
+
+    Copy.  An agent in the current snapshot's bottom set copies once per snapshot: at the end of the first env-step after the
+    snapshot's step in which its own episode ends, after that step's training (its walker has just reset, so none of its old
+    policy's actions are in flight).  A bottom agent whose episode has not ended when the next snapshot is taken does not copy.
+    The copies of one step are taken in ascending dst order; dst's src is top[g.integers(k)], g = np.random.default_rng(seed),
+    and dst then clears its history.
+
+    Explore.  dst takes src's hyper-parameters; then, for each field of `perturb` (a dict field -> (lo, hi); Hyperparams field
+    names, applied in wb_hyperparams field order), the value v becomes clip(float32(float64(v) * f), lo, hi) as a float32, with
+    f = 0.8 if g.random() < 0.5 else 1.2.  Per dst the draws are: the src, then one per perturbed field.  Only the float fields
+    alpha, beta1, beta2, adam_epsilon, gamma, lambda_, epsilon and log_std may be perturbed; default DEFAULT_PERTURB.
+
+    Within env-step t: (1) the reward sums of the episodes that ended in t join their agents' histories, (2) the copies of t are
+    decided, (3) if (t + 1) % interval == 0 the new snapshot is taken."""
+
+    def __init__(self, interval: int, fraction: float = 0.2, window: int = 5, perturb=None, seed: int = 0):
+        if int(interval) < 1:
+            raise ValueError(f"interval must be at least 1, got {interval}")
+        if not 0.0 <= float(fraction) <= 0.5:
+            raise ValueError(f"fraction must be in [0, 0.5], got {fraction}")
+        if int(window) < 1:
+            raise ValueError(f"window must be at least 1, got {window}")
+        perturb = DEFAULT_PERTURB if perturb is None else dict(perturb)
+        for name, (lo, hi) in perturb.items():
+            if name not in PERTURBABLE:
+                raise ValueError(f"{name!r} cannot be perturbed (one of {', '.join(PERTURBABLE)})")
+            if not lo <= hi:
+                raise ValueError(f"{name}: lo {lo} > hi {hi}")
+        self.interval, self.fraction, self.window = int(interval), float(fraction), int(window)
+        self.perturb = {name: (float(perturb[name][0]), float(perturb[name][1])) for name in PERTURBABLE if name in perturb}
+        self.rng = np.random.default_rng(seed)
+        # per agent: its last `window` reward sums, oldest first (a shift register), and how many it has had since its last copy
+        self.history, self.count = None, None
+        self.top, self.bottom = [], None  # the current snapshot; bottom[a]: a has not copied yet
+
+    def scores(self) -> dict:
+        """{agent: score} of the ranked agents."""
+        ranked = np.flatnonzero(self.count >= self.window) if self.count is not None else np.zeros(0, np.int64)
+        return dict(zip(ranked.tolist(), self.history[ranked].mean(axis=1).tolist()))
+
+    def step(self, t: int, agents, rewards, hp) -> list:
+        """Env-step t ended the episodes of `agents` (each at most once) with the reward sums `rewards`; hp: every agent's current
+        Hyperparams.  Returns the copies of this step: [(dst, src, dst's new Hyperparams)] in ascending dst order."""
+        if self.history is None:
+            self.history, self.count = np.zeros((len(hp), self.window)), np.zeros(len(hp), np.int64)
+            self.bottom = np.zeros(len(hp), bool)
+        ended = np.asarray(agents, np.int64).reshape(-1)
+        self.history[ended, :-1] = self.history[ended, 1:]
+        self.history[ended, -1] = np.asarray(rewards, np.float32).reshape(-1)
+        self.count[ended] += 1
+        copies = []
+        for dst in np.sort(ended[self.bottom[ended]]).tolist():
+            src = self.top[int(self.rng.integers(len(self.top)))]
+            h = Hyperparams.from_buffer_copy(hp[src])
+            for name, (lo, hi) in self.perturb.items():
+                f = 0.8 if self.rng.random() < 0.5 else 1.2
+                setattr(h, name, float(np.float32(min(max(np.float32(np.float64(getattr(h, name)) * f), lo), hi))))
+            copies.append((dst, src, h))
+            self.count[dst] = 0
+            self.bottom[dst] = False
+        if (t + 1) % self.interval == 0:
+            ranked = np.flatnonzero(self.count >= self.window)
+            order = ranked[np.lexsort((ranked, -self.history[ranked].mean(axis=1)))]
+            k = int(np.floor(self.fraction * len(order)))
+            self.top = order[:k].tolist()
+            self.bottom[:] = False
+            self.bottom[order[len(order) - k:] if k else []] = True
+        return copies
+
+
 class IndependentPPO:
     """N walkers, N independent agents (walker w acts with and trains agent w), resident on the GPU.
 
@@ -192,10 +305,14 @@ class IndependentPPO:
     ring and resets finished walkers, and ONE synchronisation reads the N done bytes through a pinned buffer.  If any walker
     finished, ONE wb_population_train_dev launch trains each of those walkers' agents on its complete episode, with mini-batch
     indices drawn on the device (seed train_seed).  A ring column is only written by its own walker, and the walker has trained
-    before it writes again.  episode_log() lists every finished episode: step, agent, length, reward sum and the two losses."""
+    before it writes again.  episode_log() lists every finished episode: step, agent, length, reward sum and the two losses.
+
+    pbt: a PBT schedule, or None.  With one, the synchronisation also reads the N running reward sums, and after the training
+    launch the step issues the schedule's copies as ONE wb_population_copy_agents launch; exploit_log() lists them."""
 
     def __init__(self, n_envs: int, floor="Metal", walker="Carpet", hp=None, seed: int = 0, epochs: int = 5, terrain=None, seeds=None,
-                 actor: str = DEFAULT_ACTOR, critic: str = DEFAULT_CRITIC, stateSize: int = OBS, actionSize: int = ACT):
+                 actor: str = DEFAULT_ACTOR, critic: str = DEFAULT_CRITIC, stateSize: int = OBS, actionSize: int = ACT,
+                 pbt: PBT | None = None):
         if (stateSize, actionSize) != (OBS, ACT):
             raise ValueError(f"the walker observes {OBS} values and takes {ACT} actions; got stateSize={stateSize}, actionSize={actionSize}")
         import torch
@@ -232,6 +349,10 @@ class IndependentPPO:
         self.done_host = torch.zeros(n, dtype=torch.uint8).pin_memory()
         self.idx_host = torch.zeros(n, dtype=torch.int64).pin_memory()
         self.ep_reward = torch.zeros(n, **f32)
+        self.pbt = pbt
+        if pbt is not None:
+            self.reward_host = torch.zeros(n, dtype=torch.float32).pin_memory()
+        self._exploit = []
         self.obs = torch.from_numpy(self.env.get_obs()).to(dev)  # Environment.InitialState
         self.start = np.zeros(n, np.int64)  # env-step at which each walker's running episode began
         self.t = 0
@@ -258,6 +379,8 @@ class IndependentPPO:
         if ev:
             ev[2].record()
         self.done_host.copy_(self.done, non_blocking=True)
+        if self.pbt is not None:
+            self.reward_host.copy_(self.ep_reward, non_blocking=True)
         torch.cuda.current_stream().synchronize()
         done = self.done_host.numpy().copy()
         if ev:
@@ -276,6 +399,12 @@ class IndependentPPO:
             self._log.append((self.t, w, lengths, self.ep_reward.index_select(0, idx), losses))
             self.ep_reward.index_fill_(0, idx, 0.0)
             self.start[w] = self.t + 1
+        if self.pbt is not None:
+            w = np.flatnonzero(done)
+            copies = self.pbt.step(self.t, w, self.reward_host.numpy()[w], self.pop.hp)
+            if copies:
+                self.pop.copy_agents([(d, s) for d, s, _ in copies], [h for _, _, h in copies])
+                self._exploit += [(self.t, d, s, h) for d, s, h in copies]
         if ev:
             ev[4].record()
             self.timing.append(ev)
@@ -302,4 +431,14 @@ class IndependentPPO:
         return out
 
 
-__all__ = ["PPOPopulation", "IndependentPPO", "default_seeds"]
+    def exploit_log(self) -> np.ndarray:
+        """Every copy of the PBT schedule in order: step (the env-step it ended), dst, src and dst's new hyper-parameters (the
+        Hyperparams fields)."""
+        fields = [(name, np.int32 if ctype is C.c_int32 else np.float32) for name, ctype in Hyperparams._fields_]
+        out = np.zeros(len(self._exploit), [("step", np.int64), ("dst", np.int32), ("src", np.int32)] + fields)
+        for i, (t, d, s, h) in enumerate(self._exploit):
+            out[i] = (t, d, s) + tuple(getattr(h, name) for name, _ in fields)
+        return out
+
+
+__all__ = ["PPOPopulation", "IndependentPPO", "PBT", "default_seeds"]
