@@ -43,11 +43,8 @@ struct wb_policy {
   void* opened[kExchMaxWorld] = {};  // IPC mappings to close
   int comm_rank = -1, comm_world = 0;
   uint32_t comm_epoch = 0;
-  // wb_ppo_train_trajectories: device offsets + Adam correction table (uploaded from a pinned host copy), scratch rows
-  char* h_episode_tab = nullptr;
-  char* d_episode_tab = nullptr;
-  size_t episode_tab_bytes = 0;
-  cudaEvent_t episode_tab_copied = nullptr;  // the previous upload has left the pinned copy
+  // wb_ppo_train_trajectories: the table of a population of one (CTA, agent constants, items, Adam corrections), scratch rows
+  PinnedTable tab;
   float* d_episode_scratch = nullptr;
   size_t episode_scratch_floats = 0;
 };
@@ -192,9 +189,6 @@ int32_t wb_policy_destroy(wb_policy* p) {
   cudaFree(p->d_comm_dead);
   cudaFree(p->d_partials);
   cudaFree(p->d_stage);
-  if (p->h_episode_tab) cudaFreeHost(p->h_episode_tab);
-  cudaFree(p->d_episode_tab);
-  if (p->episode_tab_copied) cudaEventDestroy(p->episode_tab_copied);
   cudaFree(p->d_episode_scratch);
   delete p;
   return WB_OK;
@@ -868,62 +862,51 @@ int32_t wb_ppo_train_trajectories_dev(wb_policy* p, int32_t n_traj, const int32_
     return WB_OK;
   }
 
-  // default networks: ONE launch.  Table = device offsets [n_traj + 1] then the Adam bias corrections [steps][10] (next_corrections,
-  // the function every other Adam entry uses, so wb_policy_get_adam reports what the per-mini-batch path reports)
-  const size_t off_bytes = ((sizeof(int32_t) * (n_traj + 1)) + 15) / 16 * 16;
-  const size_t tab_bytes = off_bytes + sizeof(float) * 10 * (size_t)steps;
-  if (!p->episode_tab_copied) WB_CUDA(cudaEventCreateWithFlags(&p->episode_tab_copied, cudaEventDisableTiming));
-  WB_CUDA(cudaEventSynchronize(p->episode_tab_copied));  // (the previous call's upload has read the pinned copy)
-  if (tab_bytes > p->episode_tab_bytes) {
-    if (p->h_episode_tab) cudaFreeHost(p->h_episode_tab);
-    cudaFree(p->d_episode_tab);
-    p->h_episode_tab = nullptr;
-    p->d_episode_tab = nullptr;
-    p->episode_tab_bytes = 0;
-    WB_CUDA(cudaHostAlloc(&p->h_episode_tab, tab_bytes, cudaHostAllocDefault));
-    WB_CUDA(cudaMalloc(&p->d_episode_tab, tab_bytes));
-    p->episode_tab_bytes = tab_bytes;
+  // default networks: ONE launch of population_episodes_kernel over a population of one.  The packed list is a ring of one column:
+  // item e = (column 0, t0 = offsets[e], T_e), and non-decreasing offsets give t0 + T_e <= rows <= ring_rows, so no item wraps
+  // (the kernel runs an item longer than kPopMaxLen in place on that condition).  Table = the CTA, the agent's constants, the
+  // items and the Adam bias corrections [steps][10] (next_corrections, the function every other Adam entry uses, so
+  // wb_policy_get_adam reports what the per-mini-batch path reports)
+  const size_t cta_bytes = align16(sizeof(PopCta)), agent_bytes = align16(sizeof(PopAgent)), item_bytes = align16(sizeof(PopItem) * n_traj);
+  const size_t tab_bytes = cta_bytes + agent_bytes + item_bytes + sizeof(float) * 10 * (size_t)steps;
+  if (int32_t rc = p->tab.reserve(tab_bytes)) return rc;
+  *reinterpret_cast<PopCta*>(p->tab.host) = PopCta{0, 0, n_traj, 0};
+  population_agent_consts(p->hp, reinterpret_cast<PopAgent*>(p->tab.host + cta_bytes));
+  PopItem* items = reinterpret_cast<PopItem*>(p->tab.host + cta_bytes + agent_bytes);
+  int64_t index_off = 0, corr_off = 0;
+  for (int32_t e = 0; e < n_traj; e++) {
+    const int32_t T = offsets_host[e + 1] - offsets_host[e];
+    const int64_t nb = (int64_t)epochs * (T / B);
+    items[e] = PopItem{e, 0, T > 0 ? offsets_host[e] : 0, T, (int32_t)index_off, (int32_t)corr_off, 0, 0};
+    index_off += nb * B;
+    corr_off += nb;
   }
-  memcpy(p->h_episode_tab, offsets_host, sizeof(int32_t) * (n_traj + 1));
-  float* corr = reinterpret_cast<float*>(p->h_episode_tab + off_bytes);
+  float* corr = reinterpret_cast<float*>(p->tab.host + cta_bytes + agent_bytes + item_bytes);
   for (int64_t st = 0; st < steps; st++) next_corrections(p, corr + 10 * st, corr + 10 * st + 5);
-  WB_CUDA(cudaMemcpyAsync(p->d_episode_tab, p->h_episode_tab, tab_bytes, cudaMemcpyHostToDevice, p->stream));
-  WB_CUDA(cudaEventRecord(p->episode_tab_copied, p->stream));
-  EpisodeParams e{};
-  e.rewards = rewards_dev;
-  e.values = values_dev;
-  e.returns = returns_dev;
-  e.advantages = advantages_dev;
-  e.offsets = reinterpret_cast<const int32_t*>(p->d_episode_tab);
-  e.batch_index = batch_index_dev;
-  e.corr = reinterpret_cast<const float*>(p->d_episode_tab + off_bytes);
-  e.grads = p->d_grads;
-  e.losses = losses_dev;
-  e.skipped = skipped_dev;
-  e.adam.params = p->d_params;
-  e.adam.grads = p->d_grads;
-  e.adam.m = p->d_m;
-  e.adam.v = p->d_v;
-  e.adam.alpha = p->hp.alpha;
-  e.adam.beta1 = p->hp.beta1;
-  e.adam.beta2 = p->hp.beta2;
-  e.adam.eps = p->hp.adam_epsilon;
-  e.n_traj = n_traj;
-  e.epochs = epochs;
-  e.batch = B;
-  e.use_gae = p->hp.use_gae;
-  e.normalize = p->hp.normalize_advantages;
-  e.gamma = p->hp.gamma;
-  e.lambda = p->hp.lambda;
-  e.norm_eps = p->hp.epsilon;
-  MlpParams m;
-  fill_mlp_common(p, m, (int)rows, kModeGrad);
-  m.states = states_dev;
-  m.actions = actions_dev;
-  m.old_logp = old_logp_dev;
-  m.advantages = advantages_dev;
-  m.returns = returns_dev;
-  WB_CUDA(launch_episodes(e, m, p->stream));
+  if (int32_t rc = p->tab.upload(tab_bytes, p->stream)) return rc;
+  PopTrainParams t{};
+  t.states = states_dev;
+  t.actions = actions_dev;
+  t.old_logp = old_logp_dev;
+  t.rewards = rewards_dev;
+  t.values = values_dev;
+  t.returns = returns_dev;
+  t.advantages = advantages_dev;
+  t.batch_index = batch_index_dev;
+  t.ctas = reinterpret_cast<const PopCta*>(p->tab.dev);
+  t.agents = reinterpret_cast<const PopAgent*>(p->tab.dev + cta_bytes);
+  t.items = reinterpret_cast<const PopItem*>(p->tab.dev + cta_bytes + agent_bytes);
+  t.corr = reinterpret_cast<const float*>(p->tab.dev + cta_bytes + agent_bytes + item_bytes);
+  t.params = p->d_params;
+  t.m = p->d_m;
+  t.v = p->d_v;
+  t.grads = p->d_grads;
+  t.losses = losses_dev;
+  t.skipped = skipped_dev;
+  t.ring_rows = rows > 0 ? (int32_t)rows : 1;
+  t.columns = 1;
+  t.epochs = epochs;
+  WB_CUDA(launch_population_episodes(t, 1, p->stream));
   p->launches++;
   return WB_OK;
 }

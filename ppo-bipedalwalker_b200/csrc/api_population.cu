@@ -33,11 +33,7 @@ struct wb_population {
   // staging of the host entries (grown on demand)
   float* d_stage = nullptr;
   size_t stage_bytes = 0;
-  // the table of a train call (items + Adam corrections) or a copy call (pairs + constants): one pinned upload
-  char* h_tab = nullptr;
-  char* d_tab = nullptr;
-  size_t tab_bytes = 0;
-  cudaEvent_t tab_copied = nullptr;  // the previous upload has left the pinned copy
+  PinnedTable tab;                  // the table of a train call (items + Adam corrections) or a copy call (pairs + constants)
 };
 
 static int32_t grow_stage(wb_population* p, size_t bytes) {
@@ -47,25 +43,6 @@ static int32_t grow_stage(wb_population* p, size_t bytes) {
   p->stage_bytes = 0;
   WB_CUDA(cudaMalloc(&p->d_stage, bytes));
   p->stage_bytes = bytes;
-  return WB_OK;
-}
-
-static size_t align16(size_t b) { return (b + 15) / 16 * 16; }
-
-// the pinned table of one call and its device copy, at least `bytes` long, once the previous call's upload has left the pinned copy
-static int32_t stage_table(wb_population* p, size_t bytes) {
-  if (!p->tab_copied) WB_CUDA(cudaEventCreateWithFlags(&p->tab_copied, cudaEventDisableTiming));
-  WB_CUDA(cudaEventSynchronize(p->tab_copied));
-  if (bytes > p->tab_bytes) {
-    if (p->h_tab) cudaFreeHost(p->h_tab);
-    cudaFree(p->d_tab);
-    p->h_tab = nullptr;
-    p->d_tab = nullptr;
-    p->tab_bytes = 0;
-    WB_CUDA(cudaHostAlloc(&p->h_tab, bytes, cudaHostAllocDefault));
-    WB_CUDA(cudaMalloc(&p->d_tab, bytes));
-    p->tab_bytes = bytes;
-  }
   return WB_OK;
 }
 
@@ -108,11 +85,11 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
   const size_t item_bytes = align16(sizeof(PopItem) * n_items);
   const int nd = p->n_dense;
   const size_t tab_bytes = cta_bytes + item_bytes + sizeof(float) * 2 * nd * (size_t)steps;
-  if (int32_t rc = stage_table(p, tab_bytes)) return rc;
+  if (int32_t rc = p->tab.reserve(tab_bytes)) return rc;
   // nothing fails below this line: the step counters and episode counters advance only for a call that is enqueued
-  memcpy(p->h_tab, ctas.data(), sizeof(PopCta) * ctas.size());
-  PopItem* tab_items = reinterpret_cast<PopItem*>(p->h_tab + cta_bytes);
-  float* corr = reinterpret_cast<float*>(p->h_tab + cta_bytes + item_bytes);
+  memcpy(p->tab.host, ctas.data(), sizeof(PopCta) * ctas.size());
+  PopItem* tab_items = reinterpret_cast<PopItem*>(p->tab.host + cta_bytes);
+  float* corr = reinterpret_cast<float*>(p->tab.host + cta_bytes + item_bytes);
   std::vector<int32_t> fill(ctas.size(), 0);
   int64_t index_off = 0, corr_off = 0;
   for (int32_t i = 0; i < n_items; i++) {
@@ -134,8 +111,7 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
     index_off += nb * B;
     corr_off += nb;
   }
-  WB_CUDA(cudaMemcpyAsync(p->d_tab, p->h_tab, tab_bytes, cudaMemcpyHostToDevice, p->stream));
-  WB_CUDA(cudaEventRecord(p->tab_copied, p->stream));
+  if (int32_t rc = p->tab.upload(tab_bytes, p->stream)) return rc;
   PopTrainParams t{};
   t.states = states;
   t.actions = actions;
@@ -145,9 +121,9 @@ static int32_t enqueue_train(wb_population* p, int32_t n_items, const int32_t* i
   t.returns = returns;
   t.advantages = advantages;
   t.batch_index = batch_index;
-  t.ctas = reinterpret_cast<const PopCta*>(p->d_tab);
-  t.items = reinterpret_cast<const PopItem*>(p->d_tab + cta_bytes);
-  t.corr = reinterpret_cast<const float*>(p->d_tab + cta_bytes + item_bytes);
+  t.ctas = reinterpret_cast<const PopCta*>(p->tab.dev);
+  t.items = reinterpret_cast<const PopItem*>(p->tab.dev + cta_bytes);
+  t.corr = reinterpret_cast<const float*>(p->tab.dev + cta_bytes + item_bytes);
   t.agents = p->d_agents;
   t.params = p->d_params;
   t.m = p->d_m;
@@ -290,9 +266,6 @@ int32_t wb_population_destroy(wb_population* p) {
   cudaFree(p->d_grads);
   cudaFree(p->d_agents);
   cudaFree(p->d_stage);
-  if (p->h_tab) cudaFreeHost(p->h_tab);
-  cudaFree(p->d_tab);
-  if (p->tab_copied) cudaEventDestroy(p->tab_copied);
   delete p;
   return WB_OK;
 }
@@ -384,9 +357,10 @@ int32_t wb_population_copy_agents(wb_population* p, int32_t n_pairs, const int32
   for (int32_t i = 0; i < n_pairs; i++)
     if (role[src_host[i]] == kDst) return fail(WB_ERR_INVALID, "pair %d: agent %d is both a src and a dst", i, src_host[i]);
   const size_t pair_bytes = align16(sizeof(int32_t) * 2 * n_pairs);
-  if (int32_t rc = stage_table(p, pair_bytes + sizeof(PopAgent) * n_pairs)) return rc;
-  int32_t* tab_pairs = reinterpret_cast<int32_t*>(p->h_tab);
-  PopAgent* tab_consts = reinterpret_cast<PopAgent*>(p->h_tab + pair_bytes);
+  const size_t tab_bytes = pair_bytes + sizeof(PopAgent) * n_pairs;
+  if (int32_t rc = p->tab.reserve(tab_bytes)) return rc;
+  int32_t* tab_pairs = reinterpret_cast<int32_t*>(p->tab.host);
+  PopAgent* tab_consts = reinterpret_cast<PopAgent*>(p->tab.host + pair_bytes);
   std::vector<wb_hyperparams> hp(n_pairs);
   for (int32_t i = 0; i < n_pairs; i++) {
     tab_pairs[2 * i] = dst_host[i];
@@ -394,15 +368,14 @@ int32_t wb_population_copy_agents(wb_population* p, int32_t n_pairs, const int32
     hp[i] = hp_host ? hp_host[i] : p->hp[src_host[i]];
     population_agent_consts(hp[i], &tab_consts[i]);
   }
-  WB_CUDA(cudaMemcpyAsync(p->d_tab, p->h_tab, pair_bytes + sizeof(PopAgent) * n_pairs, cudaMemcpyHostToDevice, p->stream));
-  WB_CUDA(cudaEventRecord(p->tab_copied, p->stream));
+  if (int32_t rc = p->tab.upload(tab_bytes, p->stream)) return rc;
   PopCopyParams c{};
   c.params = p->d_params;
   c.m = p->d_m;
   c.v = p->d_v;
   c.agents = p->d_agents;
-  c.pairs = reinterpret_cast<const int32_t*>(p->d_tab);
-  c.consts = reinterpret_cast<const PopAgent*>(p->d_tab + pair_bytes);
+  c.pairs = reinterpret_cast<const int32_t*>(p->tab.dev);
+  c.consts = reinterpret_cast<const PopAgent*>(p->tab.dev + pair_bytes);
   c.n_pairs = n_pairs;
   c.stride = p->stride;
   WB_CUDA(launch_population_copy(c, p->stream));

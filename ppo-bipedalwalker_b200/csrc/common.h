@@ -45,4 +45,46 @@ inline void* device_alias_of_pinned(const void* p, size_t bytes) {
     if (!(cond)) return wb::fail(WB_ERR_INVALID, "%s", msg); \
   } while (0)
 
+inline size_t align16(size_t b) { return (b + 15) / 16 * 16; }
+
+// The table of one call (items, Adam corrections, copy pairs ...): filled in pinned host memory and uploaded to its device copy
+// with one copy.  The pinned copy is reused by the next call, so that call first waits until this upload has read it.
+struct PinnedTable {
+  char* host = nullptr;
+  char* dev = nullptr;
+  size_t bytes = 0;
+  cudaEvent_t copied = nullptr;  // the previous upload has left the pinned copy
+
+  PinnedTable() = default;
+  PinnedTable(const PinnedTable&) = delete;
+  PinnedTable& operator=(const PinnedTable&) = delete;
+  ~PinnedTable() {
+    if (host) cudaFreeHost(host);
+    cudaFree(dev);
+    if (copied) cudaEventDestroy(copied);
+  }
+  // host / dev at least `want` bytes long, once the previous upload has left the pinned copy
+  int32_t reserve(size_t want) {
+    if (!copied) WB_CUDA(cudaEventCreateWithFlags(&copied, cudaEventDisableTiming));
+    WB_CUDA(cudaEventSynchronize(copied));
+    if (want > bytes) {
+      if (host) cudaFreeHost(host);
+      cudaFree(dev);
+      host = nullptr;
+      dev = nullptr;
+      bytes = 0;
+      WB_CUDA(cudaHostAlloc(&host, want, cudaHostAllocDefault));
+      WB_CUDA(cudaMalloc(&dev, want));
+      bytes = want;
+    }
+    return WB_OK;
+  }
+  // the first `used` bytes of the pinned copy -> dev, enqueued on `stream`
+  int32_t upload(size_t used, cudaStream_t stream) {
+    WB_CUDA(cudaMemcpyAsync(dev, host, used, cudaMemcpyHostToDevice, stream));
+    WB_CUDA(cudaEventRecord(copied, stream));
+    return WB_OK;
+  }
+};
+
 }  // namespace wb

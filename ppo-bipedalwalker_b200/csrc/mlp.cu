@@ -115,7 +115,7 @@ __device__ __forceinline__ void sample_action(float mu, float stdv, float neg_lo
   lp = log_prob(mu, stdv, a, neg_log_std, log_sqrt_2pi);
 }
 
-// ---- the 64-sample tile pipeline of PPOAgent.Train(Batch), shared by ppo_fused_kernel and ppo_episodes_kernel (one CTA of
+// ---- the 64-sample tile pipeline of PPOAgent.Train(Batch), shared by ppo_fused_kernel and population_episodes_kernel (one CTA of
 // kMlpThreads threads over MlpSmem; the callers stage the tile's states in S.X and own the weight-gradient accumulators and loss
 // sums, which stay in registers across every tile the CTA processes)
 
@@ -467,97 +467,6 @@ __global__ void returns_kernel(const float* rewards, const float* values, int n,
   trajectory_returns(rewards, values, n, gamma, lambda, use_gae, normalize, norm_eps, returns, advantages);
 }
 
-// PPOAgent.Train(Trajectory) (PPOAgent.cs:147-172) for a list of trajectories, in list order, as ONE persistent CTA: the Adam
-// steps form a serial chain (each mini-batch is trained with the weights the previous one left), so one SM without host round
-// trips is the shape of the work.  Per trajectory: critic forward over its rows (tile_forward, as the forward mode of
-// ppo_fused_kernel), returns / advantages (trajectory_returns, as returns_kernel), then epochs x floor(T / B) mini-batches:
-// the indexed rows are gathered into the tile, ceil(B / 64) tiles accumulate in registers (the tile pipeline of
-// ppo_fused_kernel), the gradient goes to the gradient buffer, and DenseLayer.Adam runs over every parameter with that step's
-// bias corrections from the host's table before the shared-memory weights are refreshed.
-struct __align__(16) EpisodeSmem {
-  MlpSmem m;
-  int32_t rows[kTile];  // pool row of every sample of the current mini-batch tile
-};
-
-__global__ void __launch_bounds__(kMlpThreads, 1) ppo_episodes_kernel(const EpisodeParams e, const MlpParams p, const GradConsts gc) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  EpisodeSmem& E = *reinterpret_cast<EpisodeSmem*>(smem_raw);
-  MlpSmem& S = E.m;
-  const int tid = threadIdx.x;
-  const int B = e.batch;
-  stage_weights(S, p, tid);
-  int step = 0;
-  const int32_t* index = e.batch_index;
-  for (int t = 0; t < e.n_traj; t++) {
-    const int r0 = e.offsets[t], T = e.offsets[t + 1] - r0;
-    // ---- CalculateValues (PPOAgent.cs:175-189): the critic over the trajectory's rows with the current weights
-    for (int s0 = 0; s0 < T; s0 += kTile) {
-      const int nvalid = min(kTile, T - s0);
-      __syncthreads();
-      for (int i = tid; i < kTile * kIn; i += kMlpThreads) S.X[i] = (i < nvalid * kIn) ? p.states[(size_t)(r0 + s0) * kIn + i] : 0.0f;
-      __syncthreads();
-      tile_forward(S, tid);
-      if (tid < nvalid) e.values[r0 + s0 + tid] = S.V[tid];
-    }
-    __syncthreads();
-    if (tid == 0 && T > 0)
-      trajectory_returns(e.rewards + r0, e.values + r0, T, e.gamma, e.lambda, e.use_gae, e.normalize, e.norm_eps, e.returns + r0,
-                         e.advantages + r0);
-    __syncthreads();
-    // ---- epochs x floor(T / B) mini-batches, each Train(Batch) + NeuralNetwork.Optimise
-    const int nb = e.epochs * (T / B);
-    float skipped_total = 0.0f;
-    for (int b = 0; b < nb; b++, step++, index += B) {
-      float accW2[4][4];
-#pragma unroll
-      for (int j = 0; j < 4; j++)
-#pragma unroll
-        for (int l = 0; l < 4; l++) accW2[j][l] = 0.0f;
-      float accW1[3] = {0.f, 0.f, 0.f}, accWc1[3] = {0.f, 0.f, 0.f};
-      float accW3 = 0.0f, accS = 0.0f, accT = 0.0f;
-      float lossV = 0.0f, lossA = 0.0f, skipped = 0.0f;
-      for (int b0 = 0; b0 < B; b0 += kTile) {
-        const int nvalid = min(kTile, B - b0);
-        __syncthreads();
-        if (tid < kTile) E.rows[tid] = r0 + (tid < nvalid ? index[b0 + tid] : 0);
-        __syncthreads();
-        for (int i = tid; i < kTile * kIn; i += kMlpThreads) {
-          const int s = i / kIn;
-          S.X[i] = (s < nvalid) ? p.states[(size_t)E.rows[s] * kIn + (i - s * kIn)] : 0.0f;
-        }
-        __syncthreads();
-        tile_forward(S, tid);
-        tile_surrogate(S, p, gc, nvalid, [&](int s) { return E.rows[s]; }, lossV, lossA, skipped, tid);
-        tile_backward(S, accW2, accW1, accWc1, accW3, accS, accT, tid);
-      }
-      __syncthreads();
-      write_grad(S, accW2, accW1, accWc1, accW3, accS, accT, lossV, lossA, skipped, e.grads, tid);
-      // the per-mini-batch path reduces ONE partial (0 + partial + 0 ...): the same values, with -0 stored as +0
-      AdamParams a = e.adam;
-#pragma unroll
-      for (int l = 0; l < 5; l++) {
-        a.corr1[l] = e.corr[step * 10 + l];
-        a.corr2[l] = e.corr[step * 10 + 5 + l];
-      }
-      for (int i = tid; i < kTotalParams + 3; i += kMlpThreads) {
-        const float g = __fadd_rn(e.grads[i], 0.0f);
-        e.grads[i] = g;
-        if (i < kTotalParams) adam_update(a, i, g);
-      }
-      __syncthreads();
-      if (tid == 0) skipped_total += e.grads[kGradSkipped];
-      stage_weights(S, p, tid);  // (ordered before the next use by the next tile's first barrier)
-    }
-    if (tid == 0) {
-      if (e.losses) {
-        e.losses[2 * t] = nb > 0 ? e.grads[kGradLossV] : 0.0f;
-        e.losses[2 * t + 1] = nb > 0 ? e.grads[kGradLossA] : 0.0f;
-      }
-      if (e.skipped) e.skipped[t] = (int32_t)skipped_total;
-    }
-  }
-}
-
 // ---- populations: P independent agents of the default networks, agent a at a * kAgentStride of the parameter / Adam / gradient
 // arrays (new Walker() builds its own PPOAgent(12, 4), Walker.cs:25-34; N walkers of the reference are N independent learners)
 
@@ -679,12 +588,26 @@ __global__ void __launch_bounds__(kActWarps * 32) population_act_kernel(const Po
   }
 }
 
-// population_episodes_kernel: ppo_episodes_kernel over many agents -- one CTA per agent with work in the call, training that agent's
-// items (finished episodes) in list order with the agent's own parameters, Adam moments, gradient buffer, constants and slice of
-// the host's Adam correction table.  Independent networks, so the CTAs need no exchange (one SM per agent).  An item's rows live
-// in a time-major ring [R][C]: row i = ((t0 + i) mod R) * C + column.  Its rewards and values are gathered into shared memory for
-// trajectory_returns and the returns / advantages scattered back.  Mini-batch indices come from the caller or, with a null index
-// pointer, from draw_permutation (ppo_device.cuh).
+// population_episodes_kernel: PPOAgent.Train(Trajectory) (PPOAgent.cs:147-172) for many agents -- one CTA per agent with work in
+// the call, training that agent's items (finished episodes) in list order with the agent's own parameters, Adam moments, gradient
+// buffer, constants and slice of the host's Adam correction table.  An agent's Adam steps form a serial chain (each mini-batch is
+// trained with the weights the previous one left), so one SM without host round trips is the shape of its work; the networks are
+// independent, so the CTAs need no exchange.  A single policy (wb_ppo_train_trajectories) is a population of one.  Per item: the
+// critic over its rows (tile_forward), returns / advantages (trajectory_returns), then epochs x floor(L / B) mini-batches: the
+// indexed rows are gathered into the tile, ceil(B / 64) tiles accumulate in registers (the tile pipeline of ppo_fused_kernel),
+// the gradient goes to the agent's gradient buffer, and DenseLayer.Adam runs over every parameter with that step's bias
+// corrections before the shared-memory weights are refreshed.  An item's rows live in a time-major ring [R][C]: row i =
+// ((t0 + i) mod R) * C + column.  Its rewards and values are gathered into shared memory for trajectory_returns and the returns /
+// advantages scattered back; an item longer than kPopMaxLen runs trajectory_returns in place in global memory instead.
+// Mini-batch indices come from the caller or, with a null index pointer, from draw_permutation (ppo_device.cuh).
+
+// trajectory_returns on rows in global memory, out of line: the inlined call on the shared-memory copies keeps its shared-memory
+// loads and stores, and the recurrence stays one piece of source
+__device__ __noinline__ void trajectory_returns_in_place(const float* rewards, float* values, int n, float gamma, float lambda, int use_gae,
+                                                         int normalize, float norm_eps, float* returns, float* advantages) {
+  trajectory_returns(rewards, values, n, gamma, lambda, use_gae, normalize, norm_eps, returns, advantages);
+}
+
 struct __align__(16) PopSmem {
   MlpSmem m;
   int32_t rows[kTile];
@@ -729,6 +652,9 @@ __global__ void __launch_bounds__(kMlpThreads, 1) population_episodes_kernel(con
       const int t = item.t0 + i;
       return (t >= R ? t - R : t) * C + item.column;
     };
+    // An item longer than the shared arrays only comes from a single policy's packed list: one column that never wraps
+    // (columns == 1, t0 + L <= ring_rows), so row_of(i) == row_of(0) + i and its rows are worked on where they are.
+    const bool in_place = L > kPopMaxLen;
     // ---- CalculateValues (PPOAgent.cs:175-189)
     for (int s0 = 0; s0 < L; s0 += kTile) {
       const int nvalid = min(kTile, L - s0);
@@ -739,19 +665,30 @@ __global__ void __launch_bounds__(kMlpThreads, 1) population_episodes_kernel(con
       }
       __syncthreads();
       tile_forward(S, tid);
-      if (tid < nvalid) E.val[s0 + tid] = S.V[tid];
+      if (tid < nvalid) {
+        if (in_place) P.values[row_of(s0 + tid)] = S.V[tid];
+        else E.val[s0 + tid] = S.V[tid];
+      }
     }
-    for (int i = tid; i < L; i += kMlpThreads) E.rew[i] = P.rewards[row_of(i)];
+    if (!in_place)
+      for (int i = tid; i < L; i += kMlpThreads) E.rew[i] = P.rewards[row_of(i)];
     __syncthreads();
-    if (tid == 0 && L > 0)
-      trajectory_returns(E.rew, E.val, L, ag.gamma, ag.lambda, ag.use_gae, ag.normalize, ag.norm_eps, E.ret, E.adv);
-    __syncthreads();
-    for (int i = tid; i < L; i += kMlpThreads) {
-      const int r = row_of(i);
-      P.values[r] = E.val[i];
-      P.returns[r] = E.ret[i];
-      P.advantages[r] = E.adv[i];
+    if (tid == 0 && L > 0) {
+      const int r0 = row_of(0);
+      if (in_place)
+        trajectory_returns_in_place(P.rewards + r0, P.values + r0, L, ag.gamma, ag.lambda, ag.use_gae, ag.normalize, ag.norm_eps,
+                                    P.returns + r0, P.advantages + r0);
+      else
+        trajectory_returns(E.rew, E.val, L, ag.gamma, ag.lambda, ag.use_gae, ag.normalize, ag.norm_eps, E.ret, E.adv);
     }
+    __syncthreads();
+    if (!in_place)
+      for (int i = tid; i < L; i += kMlpThreads) {
+        const int r = row_of(i);
+        P.values[r] = E.val[i];
+        P.returns[r] = E.ret[i];
+        P.advantages[r] = E.adv[i];
+      }
     __syncthreads();  // (the surrogate reads the returns / advantages back from global memory)
     // ---- epochs x floor(L / B) mini-batches, each Train(Batch) + NeuralNetwork.Optimise
     const int per_epoch = L / B;
@@ -794,7 +731,7 @@ __global__ void __launch_bounds__(kMlpThreads, 1) population_episodes_kernel(con
           a.corr2[l] = corr[5 + l];
         }
         for (int i = tid; i < kTotalParams + 3; i += kMlpThreads) {
-          const float g = __fadd_rn(grads[i], 0.0f);  // (as ppo_episodes_kernel: what the one-partial reduction stores)
+          const float g = __fadd_rn(grads[i], 0.0f);  // (what the one-partial reduction of the per-mini-batch path stores: -0 as +0)
           grads[i] = g;
           if (i < kTotalParams) adam_update(a, i, g);
         }
@@ -1167,19 +1104,6 @@ cudaError_t launch_reduce_partials(const float* partials, int nparts, float* gra
 
 cudaError_t launch_adam(const AdamParams& p, cudaStream_t stream) {
   adam_kernel<<<(kTotalParams + 127) / 128, 128, 0, stream>>>(p);
-  return cudaGetLastError();
-}
-
-cudaError_t launch_episodes(const EpisodeParams& e, const MlpParams& p, cudaStream_t stream) {
-  static bool configured[64] = {};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64 || !configured[dev]) {
-    cudaError_t err = cudaFuncSetAttribute(ppo_episodes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(EpisodeSmem));
-    if (err != cudaSuccess) return err;
-    if (dev >= 0 && dev < 64) configured[dev] = true;
-  }
-  ppo_episodes_kernel<<<1, kMlpThreads, sizeof(EpisodeSmem), stream>>>(e, p, grad_consts(p.log_std, p.epsilon));
   return cudaGetLastError();
 }
 

@@ -86,25 +86,6 @@ __device__ __forceinline__ void adam_update(const AdamParams& a, int i, float g)
 }
 #endif
 
-// PPOAgent.Train(Trajectory) over a list of trajectories in one launch (ppo_episodes_kernel, default networks).  The row arrays
-// (states / actions / old_logp of the MlpParams, rewards, values, returns, advantages) hold the trajectories back to back.
-struct EpisodeParams {
-  const float* rewards;
-  float* values;
-  float* returns;
-  float* advantages;
-  const int32_t* offsets;      // [n_traj + 1] (device copy of the host's offsets)
-  const int32_t* batch_index;  // per mini-batch B local row numbers, in call order
-  const float* corr;           // [Adam steps][10]: corr1 of the 5 dense layers, then corr2
-  float* grads;                // the gradient buffer (last mini-batch's gradient, loss sums, skipped)
-  float* losses;               // [n_traj][2] or null
-  int32_t* skipped;            // [n_traj] or null
-  AdamParams adam;             // params / m / v and the hyper-parameters (the corrections come from the table)
-  int32_t n_traj, epochs, batch;
-  int32_t use_gae, normalize;
-  float gamma, lambda, norm_eps;
-};
-cudaError_t launch_episodes(const EpisodeParams& e, const MlpParams& p, cudaStream_t stream);
 cudaError_t launch_gather_rows(const int32_t* index, int B, int row_base, int sdim, int adim, const float* states, const float* actions,
                                const float* logp, const float* adv, const float* ret, float* o_states, float* o_actions, float* o_logp,
                                float* o_adv, float* o_ret, cudaStream_t stream);
@@ -114,7 +95,9 @@ cudaError_t launch_episode_losses(const float* grads_tail, float* losses, int32_
 // ---- populations: P independent agents of the default networks (population_act_kernel / population_episodes_kernel, mlp.cu)
 // Every agent's parameters, Adam moments and gradient buffer sit at agent * kAgentStride floats (16-byte aligned rows).
 constexpr int kAgentStride = kGradFloats;  // 6152 >= kTotalParams + 3
-constexpr int kPopMaxLen = 1024;           // longest episode a population trains (the reference caps one at MaxTimesteps + 1 = 1 001)
+// longest episode a population trains (the reference caps one at MaxTimesteps + 1 = 1 001); a single policy's list of trajectories
+// (wb_ppo_train_trajectories: a population of one) may hold longer ones, whose returns are computed in place
+constexpr int kPopMaxLen = 1024;
 constexpr int kActWarps = 4;               // walkers (one warp each) per CTA of population_act_kernel
 // per-agent constants, built on the host from the agent's wb_hyperparams (population_agent_consts)
 struct PopAgent {

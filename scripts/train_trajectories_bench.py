@@ -1,6 +1,7 @@
 """PPOAgent.Train(Trajectory) per finished episode: the per-mini-batch path (PPOAgent.Train: wb_policy_forward +
 wb_returns_advantages + one wb_ppo_train per mini-batch, each a synchronous host call) against one wb_ppo_train_trajectories call
-for the whole list (PPOAgent.TrainTrajectories: one launch of ppo_episodes_kernel on the default networks).
+for the whole list (PPOAgent.TrainTrajectories: on the default networks, one launch of population_episodes_kernel over a
+population of one).
 
   python scripts/train_trajectories_bench.py [--repeats 5] [--out profiles/train_trajectories_bench.json]
 

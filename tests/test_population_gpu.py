@@ -181,7 +181,10 @@ def test_host_training_equals_ppoagent_per_agent(gpu):
         sub = [(i, fresh(t)) for i, (b, t) in enumerate(pairs) if b == a]
         if not sub:
             continue
-        ref_losses = ref.TrainTrajectories([t for _, t in sub])
+        # B = 64: PPOAgent.Train per trajectory (the per-mini-batch kernels), independent of the episode kernel and bit-identical to
+        # it at that size; B = 100 has no other form with the episode kernel's summation order
+        ts = [t for _, t in sub]
+        ref_losses = [ref.Train(t) for t in ts] if ref.hp.batch_size == 64 else ref.TrainTrajectories(ts)
         assert_same(pop_state(pop, a), agent_state(ref), a)
         assert np.array_equal(bits([losses[i] for i, _ in sub]), bits(ref_losses)), a
         for i, t in sub:

@@ -8,7 +8,8 @@ import pytest
 
 pytestmark = pytest.mark.gpu
 
-LENGTHS = [37, 130, 0, 1001, 64, 200, 63]  # below B, not a multiple of 64, empty, the max_timesteps cap, exactly B
+# below B, not a multiple of 64, empty, the max_timesteps cap, exactly B, longer than the kernel's shared-memory returns (1 024 rows)
+LENGTHS = [37, 130, 0, 1001, 64, 200, 63, 1500]
 
 
 def rollout(gpu, lengths, seed=0, sdim=12):
